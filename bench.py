@@ -2,6 +2,7 @@
 """bench.py -- LR frames/s of EAVSR+ x4 on synthetic 270x480 clips (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload model|hotpath] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass over one synthetic 30-frame 270x480 LR clip per GPU:
   * workload "model"   : full EAVSR+ x4 forward (eavsr_b200.model.EAVSRP: SPyNet + encoder + 4
@@ -16,12 +17,17 @@ The JSON line carries `roofline` for the dominant hot-path kernel (tcgen05 DCNv2
 live with CUDA events, `cpu_baseline` (the oracle port timed on the host cores on a bounded
 sample) and `e2e` (host buffers in, host buffers out, copies inside the timed region).
 `--impl reference` times the CPU oracle port of the same workload (the reference's own
-`--gpu_ids -1` path cannot travel to the GPU box: /root/reference and mmcv are not there).
+`--gpu_ids -1` path needs the reference's source tree and mmcv, which this project does not ship).
+`--dump-outputs DIR` (e.g. `bench_outputs`) writes what the last timed step returned as DIR/<name>.npy (see
+`dump_outputs`), so that two builds of the project can be compared output for output on the same seeded inputs.
+Compare with a tolerance: the channel-attention sums are accumulated with floating-point atomics, so two runs
+of the same build agree to rounding, not bit for bit.
 """
 from __future__ import annotations
 
 import argparse
 import json
+import math
 import os
 import subprocess
 import sys
@@ -101,6 +107,9 @@ class HotpathWorkload:
     (SURVEY.md 3.2: 4 branches x (2T-3) MultiAdSTN calls = 5 warps + 1 DCN each; T-2 flow
     compositions per branch; 6-level SPyNet border warps for both directions)."""
     name = "eavsrp_x4_alignment_hotpath_30x272x480_bf16"
+    # step() returns the last DCNv2 output of the clip, so --dump-outputs covers only that one call: the warps and
+    # flow compositions of the step, and the other 227 DCNv2 calls, leave nothing that is compared
+    output_name = "dcn_out"
 
     def __init__(self, device, dtype=torch.bfloat16, t=T_FRAMES, h=PAD_H, w=LR_W, dg=8):
         import eavsr_b200 as E
@@ -170,6 +179,7 @@ class ModelWorkload:
     1080x1920 (SURVEY.md F4).  The forward is captured once into a CUDA graph (the reference issues
     ~20k launches per clip from one Python thread) and replayed per step."""
     name = "eavsrp_x4_full_clip_30x270x480_bf16"
+    output_name = "sr"              # step() returns the SR clips, (clips, 30, 3, 1080, 1920)
 
     def __init__(self, device, t=T_FRAMES, h=LR_H, w=LR_W, dtype=torch.bfloat16, graph=True, rank=0, world=1,
                  distinct=8, clips_per_step=1, streams=1, net=None):
@@ -317,6 +327,7 @@ class TrainWorkload:
     batch_size 8, patch_size 64), data-parallel over the ranks with NCCL DistributedDataParallel: the gradient
     all-reduce (12.28 M fp32 = 49.1 MB) is the collective.  bf16 = autocast with fp32 master weights."""
     name = "eavsrp_x4_train_step_8x15x64x64_bf16"
+    output_name = "loss"            # step() returns the step's L1 loss
 
     def __init__(self, device, rank=0, world=1, batch=8, t=15, size=64, dtype=torch.bfloat16, distinct=4, pwc=False,
                  graph=False):
@@ -411,6 +422,50 @@ def make_workload(name, device, rank=0, world=1, args=None):
         return ModelWorkload(device, t=T_FRAMES, h=LR_H, w=LR_W, rank=rank, world=world, distinct=distinct,
                              clips_per_step=args.clips_per_step if args else 1, streams=args.streams if args else 1)
     raise SystemExit(f"unknown workload {name}")
+
+
+DUMP_WHOLE = 8 << 20     # elements: an output up to this size is written whole (32 MiB in float32)
+DUMP_SAMPLE = 4 << 20    # elements drawn from a larger one: 16 MiB of float32 values + 32 MiB of float64 indices
+DUMP_LIMIT = 64 << 20    # bytes written in all
+
+
+def dump_outputs(out_dir, name, out, seed=0):
+    """Write `out`, what one step returned (a tensor, or a list of tensors that are the parts of one batch), as
+    out_dir/<name>.npy in float32.  An output of more than DUMP_WHOLE elements is replaced by DUMP_SAMPLE of its
+    elements, one drawn from each of DUMP_SAMPLE equal runs of its flat (row-major) index, at offsets that depend
+    only on its size and `seed`; the increasing indices go to out_dir/<name>_index.npy as float64 (exact below
+    2**53).  The sample is gathered from the output in place: no copy of the whole output is made.
+    Returns {file name: bytes}."""
+    import numpy as np
+    parts = [p.detach() for p in out] if isinstance(out, (list, tuple)) else [out.detach()]
+    shape = tuple(parts[0].shape)
+    if len(parts) > 1:
+        shape = (sum(p.shape[0] for p in parts),) + shape[1:]
+    numel = math.prod(shape)
+    arrays = {}
+    if numel <= DUMP_WHOLE:
+        arrays[name] = (parts[0] if len(parts) == 1 else torch.cat(parts)).float().cpu().numpy()
+    else:
+        g = torch.Generator().manual_seed(seed)
+        k = torch.arange(DUMP_SAMPLE, dtype=torch.int64)
+        lo, hi = k * numel // DUMP_SAMPLE, (k + 1) * numel // DUMP_SAMPLE
+        idx = lo + (torch.rand(DUMP_SAMPLE, generator=g, dtype=torch.float64) * (hi - lo)).long()
+        coords = torch.unravel_index(idx, shape)
+        vals = torch.empty(DUMP_SAMPLE, dtype=torch.float32)
+        first = 0
+        for p in parts:                          # the parts are consecutive runs of dim 0
+            sel = (coords[0] >= first) & (coords[0] < first + p.shape[0])
+            at = (coords[0][sel] - first,) + tuple(c[sel] for c in coords[1:])
+            vals[sel] = p[tuple(c.to(p.device) for c in at)].float().cpu()
+            first += p.shape[0]
+        arrays[name] = vals.numpy()
+        arrays[name + "_index"] = idx.double().numpy()
+    if sum(a.nbytes for a in arrays.values()) > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {name} exceeds {DUMP_LIMIT} bytes")
+    os.makedirs(out_dir, exist_ok=True)
+    for key, a in arrays.items():
+        np.save(os.path.join(out_dir, key + ".npy"), a)
+    return {key + ".npy": a.nbytes for key, a in arrays.items()}
 
 
 # ------------------------------------------------------------------------------------------------
@@ -576,31 +631,33 @@ def cpu_hotpath_frames_per_s(budget_s=20.0):
 
 def run_reference_arm(args):
     """`--impl reference`: the reference's own CPU path for the same workload (oracle port: the reference is
-    Python + mmcv + cupy and /root/reference does not travel) on all host threads.  One step = the complete x4
-    forward of a 6-frame clip at the stated 272x480 geometry (~70 s on 16 cores); as many of the requested
-    steps as fit ~4 minutes are run and `steps` reports the number actually timed."""
+    Python + mmcv + cupy, which this project does not ship) on all host threads, exactly `--steps` timed steps.
+    model: a step = the complete x4 forward of a 6-frame clip at the stated 272x480 geometry (~70 s on 16 cores),
+    after one untimed 3x64x64 clip that pays the lazy initialisations.  hotpath: a step = the 4 * (2T - 3) = 228
+    MultiAdSTN-equivalents (5 warps + 1 DCNv2) of one 30-frame clip, after one untimed MultiAdSTN-equivalent."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     torch.set_num_threads(os.cpu_count() or 1)
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    steps = args.steps
     if args.workload == "model":
         from oracle import eavsrp_cpu as R
         sd = R._seeded_state_dict()
-        t_s, hs, ws, est = R.plan_sample(120.0, PAD_H, LR_W, sd, frames=(6, 4, 3))
-        steps = max(1, min(args.steps, int(180.0 // max(est, 1.0))))
-        secs = [R.time_clip_forward(t_s, hs, ws, sd, seed=1234 + i) for i in range(steps)]
+        t_s = 6
+        R.time_clip_forward(3, 64, 64, sd)
+        secs = [R.time_clip_forward(t_s, PAD_H, LR_W, sd, seed=1234 + i) for i in range(steps)]
         el = sum(secs) / len(secs)
-        fps = t_s / el * (hs * ws) / (PAD_H * LR_W)
-        geo = f"{hs}x{ws}" + ("" if (hs, ws) == (PAD_H, LR_W) else f" (extrapolated by LR pixels to {PAD_H}x{LR_W})")
-        sample = (f"{steps} step(s) of {args.steps} requested; a step = full x4 forward of a {t_s}-frame {geo} clip "
-                  f"({el:.1f} s) on {torch.get_num_threads()} threads, fp32, ATen grid_sample + torchvision CPU DCNv2; "
-                  f"no warm-up steps beyond a 3x64x96 probe clip; frames/s of the short clip (the 30-frame clip of the "
-                  f"metric does 1.9 alignments per frame against {(2 * t_s - 3) / t_s:.1f} here: favours the CPU)")
+        fps = t_s / el
+        sample = (f"{steps} step(s); a step = full x4 forward of a {t_s}-frame {PAD_H}x{LR_W} clip ({el:.1f} s) on "
+                  f"{torch.get_num_threads()} threads, fp32, ATen grid_sample + torchvision CPU DCNv2; no warm-up steps "
+                  f"beyond a 3x64x64 clip; frames/s of the short clip (the 30-frame clip of the metric does 1.9 "
+                  f"alignments per frame against {(2 * t_s - 3) / t_s:.1f} here: favours the CPU)")
         name, ms = ModelWorkload.name, el * 1e3
     else:
-        fps, sample = cpu_hotpath_frames_per_s(20.0 * max(1, min(args.steps, 6)))
-        name, ms, steps = HotpathWorkload.name, None, args.steps
+        from oracle import cpu_reference as R
+        fps, sample = R.time_hotpath_sample(PAD_H, LR_W, T_FRAMES, clips=steps)
+        name, ms = HotpathWorkload.name, T_FRAMES / fps * 1e3
     line = {"impl": "reference", "metric": METRIC, "value": fps, "unit": "frames/s", "n_gpus": args.gpus,
             "steps": steps, "steps_requested": args.steps, "warmup": 0, "ms_per_step": ms, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -643,12 +700,18 @@ def main():
                     help="--workload train: run the epoch >= npost branch too (PWC-Net cost volume + backwarp)")
     ap.add_argument("--streams", type=int, default=1,
                     help="run the clips of a step as this many concurrent forwards (CUDA streams) instead of one batch")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them returned as DIR/<name>.npy (rank 0)")
     ap.add_argument("--clips-per-step", type=int, default=8,
                     help="clips in flight per GPU and step (BASELINE config 4 gives every GPU 8 clips): clips-per-step / "
                          "streams are batched into one forward, the forwards run on `streams` CUDA streams; default: the 8 "
                          "clips of config 4 as ONE batch (+12 %% over one clip at a time, which is reported next to it as "
                          "`single_clip`: the per-layer barrier / set-up of the chained convolutions is amortised over 8 images)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; --impl reference does not run it")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -704,7 +767,7 @@ def main():
         torch.cuda.profiler.start()          # no-op unless run under `ncu --profile-from-start off`
         e0.record()
         for _ in range(args.steps):
-            wl.step()
+            out = wl.step()
         e1.record()
         barrier()
         torch.cuda.profiler.stop()
@@ -718,6 +781,9 @@ def main():
             tt = torch.tensor([ms], device=device)
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
             ms = tt.item()
+        if args.dump_outputs and rank == 0:      # before the runs below overwrite the step's output buffers
+            written = dump_outputs(args.dump_outputs, wl.output_name, out)
+            print(f"bench.py: wrote {written} to {args.dump_outputs}", file=sys.stderr)
 
         # end to end: pinned host clip in, host result out, through the public API
         e2e = None

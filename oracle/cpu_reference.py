@@ -35,10 +35,11 @@ def ref_dcn(x, offset, mask, weight, bias, stride=1, padding=1, dilation=1):
                                          dilation=dilation, mask=mask)
 
 
-def time_hotpath_sample(h, w, t, budget_s=15.0, dg=8):
+def time_hotpath_sample(h, w, t, budget_s=15.0, dg=8, clips=None):
     """Time whole MultiAdSTN-equivalents (quarter/half/3x full-res 64-ch warps + one DCNv2,
-    models/networks.py:605-630) on the host until `budget_s` is spent; scale to the 4*(2t-3)
-    calls of a t-frame clip.  Returns (LR frames/s, description of the sample)."""
+    models/networks.py:605-630) on the host until `budget_s` is spent, or, with `clips`, exactly the
+    4*(2t-3) calls of that many t-frame clips; scale to the calls of one clip.
+    Returns (LR frames/s, description of the sample)."""
     g = torch.Generator().manual_seed(0)
     f1 = torch.randn(1, 64, h, w, generator=g)
     f2 = torch.randn(1, 64, h // 2, w // 2, generator=g)
@@ -59,6 +60,7 @@ def time_hotpath_sample(h, w, t, budget_s=15.0, dg=8):
         feat = ref_flow_warp(f1, fl1)
         return ref_dcn(feat, off, msk, wgt, bias)
 
+    units_per_clip = 4 * (2 * t - 3)
     with torch.no_grad():
         unit()                                    # warm-up (thread pool, allocator)
         n, t0 = 0, time.time()
@@ -66,10 +68,9 @@ def time_hotpath_sample(h, w, t, budget_s=15.0, dg=8):
             unit()
             n += 1
             el = time.time() - t0
-            if el >= budget_s or n >= 64:
+            if n >= clips * units_per_clip if clips else (el >= budget_s or n >= 64):
                 break
     per_unit = el / n
-    units_per_clip = 4 * (2 * t - 3)
     fps = t / (per_unit * units_per_clip)
     return fps, (f"{n} MultiAdSTN-equivalents (5 warps + 1 DCNv2 dg={dg}, fp32, {h}x{w}) in {el:.1f} s, "
                  f"scaled to {units_per_clip} per {t}-frame clip; torchvision CPU DCN + ATen grid_sample, "

@@ -1,6 +1,7 @@
 """The drop-in route: with eavsr_b200.install the UNMODIFIED reference imports and builds its
-EAVSRP with our ModulatedDeformConv2d / flow_warp / correlation.  Needs /root/reference (build
-container only); the forward itself needs a GPU (there is no CPU fallback), which is asserted."""
+EAVSRP with our ModulatedDeformConv2d / flow_warp / correlation.  Needs a checkout of the reference
+(HITRainer/EAVSR), named by EAVSR_REFERENCE; the forward itself needs a GPU (there is no CPU fallback),
+which is asserted."""
 import os
 import subprocess
 import sys
@@ -8,10 +9,11 @@ import textwrap
 
 import pytest
 
-REF = os.environ.get("EAVSR_REFERENCE", "/root/reference")
+REF = os.environ.get("EAVSR_REFERENCE", "")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")), reason="reference tree not present")
+pytestmark = pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "models")),
+                                reason="EAVSR_REFERENCE does not name a checkout of the reference")
 
 
 def test_reference_builds_on_our_ops():
