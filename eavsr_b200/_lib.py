@@ -6,8 +6,10 @@ call fails, the error is raised -- loudly -- to the caller.
 from __future__ import annotations
 
 import ctypes
+import functools
 import os
-from ctypes import c_char_p, c_float, c_int, c_int64, c_size_t, c_uint, c_uint64, c_void_p, POINTER
+import re
+from ctypes import c_char_p, c_float, c_int, c_int64, c_longlong, c_size_t, c_uint, c_uint64, c_void_p, POINTER
 from pathlib import Path
 
 _LIB_PATH = Path(__file__).resolve().parent / "libeavsr_b200.so"
@@ -29,8 +31,6 @@ CONV_SUMS_PREZEROED = 1
 CORR_TF32 = 2
 
 Strides = c_int64 * 4
-_P64 = POINTER(c_int64)
-_PF = c_void_p  # float* passed as raw device address
 
 
 class EavsrError(RuntimeError):
@@ -50,62 +50,46 @@ class ConvLayer(ctypes.Structure):
                 ("negative_slope", c_float)]
 
 
-_SIGNATURES = {
-    "eavsr_version": (c_int, []),
-    "eavsr_last_error": (c_char_p, []),
-    "eavsr_launch_count": (c_uint64, []),
-    "eavsr_flow_warp_forward": (c_int, [c_void_p, _P64, _PF, c_int, c_void_p, _P64, c_int, c_int, c_int, c_int,
-                                        c_int, c_int, c_void_p]),
-    "eavsr_flow_warp_backward": (c_int, [c_void_p, _P64, c_void_p, _P64, _PF, c_int, _PF, _P64, _PF, c_int, c_int,
-                                         c_int, c_int, c_int, c_int, c_void_p]),
-    "eavsr_flow_warp2_forward": (c_int, [c_void_p, _P64, c_void_p, _P64, _PF, c_int, c_void_p, _P64, c_void_p, _P64] +
-                                 [c_int] * 6 + [c_void_p]),
-    "eavsr_flow_warp_pyramid_forward": (c_int, [c_void_p, _P64, c_void_p, _P64, POINTER(FlowTerm), c_int, c_void_p, _P64,
-                                                c_void_p, _P64, _PF] + [c_int] * 6 + [c_void_p]),
-    "eavsr_spynet_level_input_forward": (c_int, [_PF, _PF, _PF, _PF] + [c_int] * 5 + [c_void_p]),
-    "eavsr_backwarp_forward": (c_int, [c_void_p, _P64, _PF, c_void_p, _P64, c_void_p] + [c_int] * 5 + [c_void_p]),
-    "eavsr_backwarp_backward": (c_int, [c_void_p, _P64, c_void_p, _P64, _PF, _PF, _P64, _PF] + [c_int] * 5 +
-                                [c_void_p]),
-    "eavsr_dcn_forward_workspace": (c_size_t, [c_int] * 7),
-    "eavsr_dcn_forward_uses_tensor_cores": (c_int, [_P64, _P64] + [c_int] * 12 + [c_uint]),
-    "eavsr_dcn_forward": (c_int, [c_void_p, _P64, _PF, _PF, c_void_p, c_void_p, c_void_p, _P64] + [c_int] * 16 +
-                          [c_void_p, c_size_t, c_uint, c_void_p]),
-    "eavsr_dcn_backward": (c_int, [c_void_p, _P64, c_void_p, _P64, _PF, _PF, c_void_p, _PF, _P64, _PF, _PF, _PF,
-                                   _PF] + [c_int] * 16 + [c_void_p, c_size_t, c_uint, c_void_p]),
-    "eavsr_dcn_backward_workspace": (c_size_t, [c_int] * 7),
-    "eavsr_dcn_affine_forward": (c_int, [c_void_p, _P64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, _P64] +
-                                 [c_int] * 5 + [c_void_p, c_size_t, c_uint, c_void_p]),
-    "eavsr_correlation_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
-                                          c_void_p]),
-    "eavsr_correlation_forward_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_uint,
-                                             c_void_p]),
-    "eavsr_correlation_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
-                                           c_int, c_int, c_void_p]),
-    "eavsr_adapt_mix_forward": (c_int, [c_void_p] * 7 + [c_int] * 4 + [c_float, c_int, c_void_p]),
-    "eavsr_affine_offsets_forward": (c_int, [c_void_p, _P64, c_void_p, _P64, c_void_p, _P64, c_void_p, c_void_p,
-                                             c_void_p, _PF, _PF] + [c_int] * 5 + [c_void_p]),
-    "eavsr_ca_residual_forward": (c_int, [c_void_p] * 9 + [c_int] * 6 + [c_void_p]),
-    "eavsr_bias_act_forward": (c_int, [c_void_p, c_void_p, c_int, ctypes.c_longlong, c_float, c_int, c_void_p]),
-    "eavsr_grouped_conv3x3_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
-                                              c_int, c_void_p]),
-    "eavsr_grouped_conv3x3_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
-                                               c_int, c_int, c_int, c_int, c_void_p]),
-    "eavsr_channel_sum_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, ctypes.c_longlong, c_int, c_void_p]),
-    "eavsr_channel_dot_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.c_longlong, c_int, c_void_p]),
-    "eavsr_nhwc_cat_forward": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, ctypes.c_longlong, c_int,
-                                       c_void_p]),
-    "eavsr_bias_act_shuffle_forward": (c_int, [c_void_p, c_void_p, c_void_p] + [c_int] * 4 + [c_float, c_int, c_void_p]),
-    "eavsr_ca_scale_forward": (c_int, [c_void_p, c_void_p, _PF] + [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
-    "eavsr_conv3x3_packed_weight_bytes": (c_size_t, []),
-    "eavsr_conv3x3_pack_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
-    "eavsr_conv3x3_ca_forward": (c_int, [c_void_p, c_void_p, _PF] + [c_void_p] * 8 + [_PF] + [c_int] * 3 +
-                                 [c_float, c_int, c_uint, c_void_p]),
-    "eavsr_conv3x3_chain_forward": (c_int, [POINTER(ConvLayer), c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
-    "eavsr_conv3x3_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, _PF] + [c_int] * 5 +
-                              [c_float, c_int, c_uint, c_void_p]),
-}
+_HEADER = Path(__file__).resolve().parents[1] / "include" / "eavsr_b200.h"
+# ctypes type of each spelling the header uses; any other pointer is passed as a raw address (c_void_p)
+_CTYPES = {"const char*": c_char_p, "const int64_t[4]": POINTER(c_int64), "const EavsrFlowTerm*": POINTER(FlowTerm),
+           "const EavsrConvLayer*": POINTER(ConvLayer), "int": c_int, "unsigned": c_uint, "size_t": c_size_t,
+           "long long": c_longlong, "float": c_float, "uint64_t": c_uint64}
 
-EXPORTED_SYMBOLS = tuple(_SIGNATURES)
+
+def _ctype(spelling: str, name: str):
+    if spelling in _CTYPES:
+        return _CTYPES[spelling]
+    if spelling.endswith("*"):
+        return c_void_p
+    raise EavsrError(f"{_HEADER}: {name} uses `{spelling}`, which has no ctypes type in eavsr_b200._lib")
+
+
+def _arg_type(decl: str, name: str):
+    """ctypes type of one declared parameter: "const int64_t x_strides[4]" -> POINTER(c_int64)."""
+    m = re.fullmatch(r"(.*?\S)\s*\b\w+(\[4\])?", " ".join(decl.split()))
+    if m is None:
+        raise EavsrError(f"{_HEADER}: cannot read parameter `{decl.strip()}` of {name}")
+    return _ctype(m[1] + (m[2] or ""), name)
+
+
+@functools.cache
+def _signatures() -> dict:
+    """{name: (restype, argtypes)} of every eavsr_* prototype in include/eavsr_b200.h."""
+    if not _HEADER.exists():
+        raise EavsrError(f"{_HEADER} not found: the ctypes signatures are read from the C header")
+    text = re.sub(r"/\*.*?\*/", "", _HEADER.read_text(), flags=re.S)
+    sigs = {}
+    for ret, name, params in re.findall(r"^(\w[\w ]*?\**)\s*\b(eavsr_\w+)\(([^)]*)\);", text, flags=re.M):
+        args = [] if params.strip() == "void" else [_arg_type(p, name) for p in params.split(",")]
+        sigs[name] = (_ctype(ret, name), args)
+    return sigs
+
+
+def __getattr__(attr):
+    if attr == "EXPORTED_SYMBOLS":      # every entry point the header declares (and load() binds)
+        return tuple(_signatures())
+    raise AttributeError(f"module {__name__!r} has no attribute {attr!r}")
 
 
 def lib_path() -> Path:
@@ -121,8 +105,9 @@ def load():
             raise EavsrError(
                 f"{path} not found: build it with `python -m eavsr_b200.build` "
                 "(eavsr_b200 has no CPU or PyTorch fallback)")
+        sigs = _signatures()
         lib = ctypes.CDLL(str(path))
-        for name, (res, args) in _SIGNATURES.items():
+        for name, (res, args) in sigs.items():
             fn = getattr(lib, name)
             fn.restype = res
             fn.argtypes = args

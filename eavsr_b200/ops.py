@@ -64,7 +64,9 @@ def _dtype_code(name: str, t: torch.Tensor) -> int:
         raise TypeError(f"eavsr_b200.{name}: dtype {t.dtype} not supported (float32 / bfloat16)") from None
 
 
-def _strides(t: torch.Tensor):
+def _strides(t: Optional[torch.Tensor]):
+    if t is None:
+        return None
     s = list(t.stride())
     if t.dim() == 4 and t.shape[0] == 1:
         # the stride of a size-1 batch dimension is arbitrary in PyTorch (views such as `x.view(t, 1, ...).unbind(0)`
@@ -73,12 +75,31 @@ def _strides(t: torch.Tensor):
     return L.Strides(*s)
 
 
-def _stream(t: torch.Tensor) -> int:
-    return torch.cuda.current_stream(t.device).cuda_stream
+# `isinstance(a, torch.Tensor)` costs ~0.1 us for a non-tensor, and most arguments are sizes: test those by type first
+_PLAIN_ARGS = frozenset((int, float, type(None), L.Strides))
 
 
-def _ptr(t: Optional[torch.Tensor]):
-    return None if t is None else t.data_ptr()
+def _launch(entry: str, *args) -> None:
+    """Call ``eavsr_<entry>(*args, stream)`` on the current stream of the first tensor argument's device, inside
+    that device's guard.  Tensors are passed as their ``data_ptr()``; ``args`` keeps them alive until the call has
+    been issued, so a converted temporary cannot be freed and its memory reused by a later argument."""
+    cargs = [a if type(a) in _PLAIN_ARGS else a.data_ptr() if isinstance(a, torch.Tensor) else a for a in args]
+    dev = next(a for a in args if isinstance(a, torch.Tensor)).device
+    fn = getattr(L.load(), "eavsr_" + entry)
+    with torch.cuda.device(dev):
+        # the handle of torch.cuda.current_stream(dev), without building a Stream object on every launch
+        rc = fn(*cargs, torch._C._cuda_getCurrentRawStream(dev.index))
+    L.check(rc, entry)
+
+
+def _param(t: Optional[torch.Tensor], dtype) -> Optional[torch.Tensor]:
+    """Detached contiguous ``dtype`` view / copy of a parameter (None stays None)."""
+    return None if t is None else t.detach().to(dtype).contiguous()
+
+
+def _grad(g: Optional[torch.Tensor], dtype) -> Optional[torch.Tensor]:
+    """An fp32 gradient buffer cast to the dtype of its input (None stays None)."""
+    return None if g is None else g.to(dtype)
 
 
 def _is_channels_last(t: torch.Tensor) -> bool:
@@ -109,19 +130,15 @@ def _dense(t: torch.Tensor) -> torch.Tensor:
 class _FlowWarpFn(Function):
     @staticmethod
     def forward(ctx, x, flow, layout: int, pad: int):
-        lib = L.load()
-        with torch.cuda.device(x.device):
-            if (x.shape[1] * x.element_size()) % 16 == 0:
-                xd = x.contiguous(memory_format=torch.channels_last)  # vectorised NHWC path
-            else:
-                xd = _dense(x)                                        # 2/3-channel maps: strided path
-            flow32 = flow.detach().to(torch.float32).contiguous()
-            out = _empty_like_layout(xd)
-            n, c, h, w = xd.shape
-            L.check(lib.eavsr_flow_warp_forward(xd.data_ptr(), _strides(xd), flow32.data_ptr(), layout,
-                                                out.data_ptr(), _strides(out), n, c, h, w,
-                                                _dtype_code("flow_warp", xd), pad, _stream(xd)),
-                    "flow_warp_forward")
+        if (x.shape[1] * x.element_size()) % 16 == 0:
+            xd = x.contiguous(memory_format=torch.channels_last)  # vectorised NHWC path
+        else:
+            xd = _dense(x)                                        # 2/3-channel maps: strided path
+        flow32 = _param(flow, torch.float32)
+        out = _empty_like_layout(xd)
+        n, c, h, w = xd.shape
+        _launch("flow_warp_forward", xd, _strides(xd), flow32, layout, out, _strides(out), n, c, h, w,
+                _dtype_code("flow_warp", xd), pad)
         ctx.save_for_backward(xd, flow32)
         ctx.layout, ctx.pad, ctx.flow_dtype = layout, pad, flow.dtype
         return out
@@ -130,25 +147,14 @@ class _FlowWarpFn(Function):
     @once_differentiable
     def backward(ctx, gout):
         xd, flow32 = ctx.saved_tensors
-        lib = L.load()
-        need_x, need_f = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
-        gx32 = gflow = None
-        with torch.cuda.device(xd.device):
-            fmt = torch.channels_last if _is_channels_last(xd) else torch.contiguous_format
-            g = gout.to(xd.dtype).contiguous(memory_format=fmt)
-            if need_x:
-                gx32 = _empty_like_layout(xd, dtype=torch.float32)
-            if need_f:
-                gflow = torch.empty_like(flow32)
-            n, c, h, w = xd.shape
-            L.check(lib.eavsr_flow_warp_backward(g.data_ptr(), _strides(g), xd.data_ptr(), _strides(xd),
-                                                 flow32.data_ptr(), ctx.layout, _ptr(gx32),
-                                                 _strides(gx32) if gx32 is not None else None, _ptr(gflow),
-                                                 n, c, h, w, _dtype_code("flow_warp", xd), ctx.pad, _stream(xd)),
-                    "flow_warp_backward")
-        gx = gx32.to(xd.dtype) if gx32 is not None else None
-        gf = gflow.to(ctx.flow_dtype) if gflow is not None else None
-        return gx, gf, None, None
+        fmt = torch.channels_last if _is_channels_last(xd) else torch.contiguous_format
+        g = gout.to(xd.dtype).contiguous(memory_format=fmt)
+        gx32 = _empty_like_layout(xd, dtype=torch.float32) if ctx.needs_input_grad[0] else None
+        gflow = torch.empty_like(flow32) if ctx.needs_input_grad[1] else None
+        n, c, h, w = xd.shape
+        _launch("flow_warp_backward", g, _strides(g), xd, _strides(xd), flow32, ctx.layout, gx32, _strides(gx32), gflow,
+                n, c, h, w, _dtype_code("flow_warp", xd), ctx.pad)
+        return _grad(gx32, xd.dtype), _grad(gflow, ctx.flow_dtype), None, None
 
 
 def _flow_warp(name, x, flow, layout, interpolation, padding_mode, align_corners):
@@ -195,15 +201,11 @@ def flow_warp2(x1, x2, flow, padding_mode='zeros'):
           and padding_mode in ('zeros', 'border'))
     if not ok:
         return flow_warp(x1, flow, padding_mode=padding_mode), flow_warp(x2, flow, padding_mode=padding_mode)
-    lib = L.load()
     n, c, h, w = x1.shape
-    with torch.cuda.device(x1.device):
-        f32 = flow.detach().to(torch.float32).contiguous()
-        o1, o2 = torch.empty_like(x1), torch.empty_like(x2)
-        L.check(lib.eavsr_flow_warp2_forward(x1.data_ptr(), _strides(x1), x2.data_ptr(), _strides(x2), f32.data_ptr(),
-                                             L.FLOW_N2HW, o1.data_ptr(), _strides(o1), o2.data_ptr(), _strides(o2),
-                                             n, c, h, w, L.BF16, L.PAD_ZEROS if padding_mode == 'zeros' else L.PAD_BORDER,
-                                             _stream(x1)), "flow_warp2_forward")
+    o1, o2 = torch.empty_like(x1), torch.empty_like(x2)
+    _launch("flow_warp2_forward", x1, _strides(x1), x2, _strides(x2), _param(flow, torch.float32), L.FLOW_N2HW,
+            o1, _strides(o1), o2, _strides(o2), n, c, h, w, L.BF16,
+            L.PAD_ZEROS if padding_mode == 'zeros' else L.PAD_BORDER)
     return o1, o2
 
 
@@ -224,27 +226,22 @@ def flow_warp_pyramid(x, terms, x2=None, want_flow=False, keep=()):
     ``terms``: [(flow (n,2,hi,wi), scale), ...] (<= 4); ``x2``: a second map warped with the same flow (:621-623);
     ``want_flow``: also return the summed flow; ``keep``: indices of terms whose ``scale * resize(flow)`` is returned
     too.  Returns (out, [out2], [flow], [kept terms...]).  Inference only: check `flow_warp_pyramid_eligible`."""
-    lib = L.load()
     n, c, h, w = x.shape
-    with torch.cuda.device(x.device):
-        out = torch.empty_like(x)
-        out2 = torch.empty_like(x2) if x2 is not None else None
-        fl = torch.empty((n, 2, h, w), dtype=torch.float32, device=x.device) if want_flow else None
-        arr = (L.FlowTerm * len(terms))()
-        hold, kept = [], []
-        for i, (a, (f, sc)) in enumerate(zip(arr, terms)):
-            f32 = f.detach().to(torch.float32).contiguous()
-            hold.append(f32)
-            a.flow, a.h, a.w, a.scale = f32.data_ptr(), f32.shape[2], f32.shape[3], float(sc)
-            if i in keep:
-                t = torch.empty((n, 2, h, w), dtype=torch.float32, device=x.device)
-                kept.append(t)
-                a.scaled_out = t.data_ptr()
-        L.check(lib.eavsr_flow_warp_pyramid_forward(
-            x.data_ptr(), _strides(x), _ptr(x2), _strides(x2) if x2 is not None else None, arr, len(terms),
-            out.data_ptr(), _strides(out), _ptr(out2), _strides(out2) if out2 is not None else None, _ptr(fl),
-            n, c, h, w, _dtype_code("flow_warp_pyramid", x), L.PAD_ZEROS, _stream(x)), "flow_warp_pyramid_forward")
-        del hold
+    out = torch.empty_like(x)
+    out2 = torch.empty_like(x2) if x2 is not None else None
+    fl = torch.empty((n, 2, h, w), dtype=torch.float32, device=x.device) if want_flow else None
+    arr = (L.FlowTerm * len(terms))()
+    hold, kept = [], []             # `arr` holds raw addresses: the tensors behind them must outlive the launch
+    for i, (a, (f, sc)) in enumerate(zip(arr, terms)):
+        f32 = _param(f, torch.float32)
+        hold.append(f32)
+        a.flow, a.h, a.w, a.scale = f32.data_ptr(), f32.shape[2], f32.shape[3], float(sc)
+        if i in keep:
+            t = torch.empty((n, 2, h, w), dtype=torch.float32, device=x.device)
+            kept.append(t)
+            a.scaled_out = t.data_ptr()
+    _launch("flow_warp_pyramid_forward", x, _strides(x), x2, _strides(x2), arr, len(terms), out, _strides(out),
+            out2, _strides(out2), fl, n, c, h, w, _dtype_code("flow_warp_pyramid", x), L.PAD_ZEROS)
     res = [out]
     if out2 is not None:
         res.append(out2)
@@ -259,18 +256,13 @@ def spynet_level_input(ref, supp, flow_prev=None):
     level, ``flow_prev=None``): the input of one SPyNet level (models/eavsrp_model.py:468-486) in one launch
     (SURVEY.md section 8 row f4).  NCHW fp32, inference only.  Returns (n, 8, h, w); channels 6:8 are ``up``."""
     _require_cuda("spynet_level_input", ref, supp, flow_prev)
-    lib = L.load()
     n, c, h, w = ref.shape
     if c != 3 or supp.shape != ref.shape or ref.dtype != torch.float32 or supp.dtype != torch.float32:
         raise ValueError(f"spynet_level_input: expected two (n,3,h,w) fp32 images, got {tuple(ref.shape)} / {tuple(supp.shape)}")
-    with torch.cuda.device(ref.device):
-        r, s_ = ref.contiguous(), supp.contiguous()
-        fp = flow_prev.detach().to(torch.float32).contiguous() if flow_prev is not None else None
-        out = torch.empty((n, 8, h, w), dtype=torch.float32, device=ref.device)
-        L.check(lib.eavsr_spynet_level_input_forward(r.data_ptr(), s_.data_ptr(), _ptr(fp), out.data_ptr(), n, h, w,
-                                                     fp.shape[2] if fp is not None else 0,
-                                                     fp.shape[3] if fp is not None else 0, _stream(ref)),
-                "spynet_level_input_forward")
+    fp = _param(flow_prev, torch.float32)
+    out = torch.empty((n, 8, h, w), dtype=torch.float32, device=ref.device)
+    _launch("spynet_level_input_forward", ref.contiguous(), supp.contiguous(), fp, out, n, h, w,
+            fp.shape[2] if fp is not None else 0, fp.shape[3] if fp is not None else 0)
     return out
 
 
@@ -280,16 +272,13 @@ def spynet_level_input(ref, supp, flow_prev=None):
 class _BackwarpFn(Function):
     @staticmethod
     def forward(ctx, x, flow):
-        lib = L.load()
-        with torch.cuda.device(x.device):
-            xd = _dense(x)
-            flow32 = flow.detach().to(torch.float32).contiguous()
-            n, c, h, w = xd.shape
-            out = _empty_like_layout(xd)
-            mask = torch.empty((n, 1, h, w), dtype=xd.dtype, device=xd.device)
-            L.check(lib.eavsr_backwarp_forward(xd.data_ptr(), _strides(xd), flow32.data_ptr(), out.data_ptr(),
-                                               _strides(out), mask.data_ptr(), n, c, h, w,
-                                               _dtype_code("backwarp", xd), _stream(xd)), "backwarp_forward")
+        xd = _dense(x)
+        flow32 = _param(flow, torch.float32)
+        n, c, h, w = xd.shape
+        out = _empty_like_layout(xd)
+        mask = torch.empty((n, 1, h, w), dtype=xd.dtype, device=xd.device)
+        _launch("backwarp_forward", xd, _strides(xd), flow32, out, _strides(out), mask, n, c, h, w,
+                _dtype_code("backwarp", xd))
         ctx.save_for_backward(xd, flow32)
         ctx.flow_dtype = flow.dtype
         ctx.mark_non_differentiable(mask)
@@ -299,22 +288,13 @@ class _BackwarpFn(Function):
     @once_differentiable
     def backward(ctx, gout, _gmask):
         xd, flow32 = ctx.saved_tensors
-        lib = L.load()
-        need_x, need_f = ctx.needs_input_grad
-        gx32 = gflow = None
-        with torch.cuda.device(xd.device):
-            g = _dense(gout.to(xd.dtype))
-            if need_x:
-                gx32 = _empty_like_layout(xd, dtype=torch.float32)
-            if need_f:
-                gflow = torch.empty_like(flow32)
-            n, c, h, w = xd.shape
-            L.check(lib.eavsr_backwarp_backward(g.data_ptr(), _strides(g), xd.data_ptr(), _strides(xd),
-                                                flow32.data_ptr(), _ptr(gx32),
-                                                _strides(gx32) if gx32 is not None else None, _ptr(gflow), n, c, h, w,
-                                                _dtype_code("backwarp", xd), _stream(xd)), "backwarp_backward")
-        return (gx32.to(xd.dtype) if gx32 is not None else None,
-                gflow.to(ctx.flow_dtype) if gflow is not None else None)
+        g = _dense(gout.to(xd.dtype))
+        gx32 = _empty_like_layout(xd, dtype=torch.float32) if ctx.needs_input_grad[0] else None
+        gflow = torch.empty_like(flow32) if ctx.needs_input_grad[1] else None
+        n, c, h, w = xd.shape
+        _launch("backwarp_backward", g, _strides(g), xd, _strides(xd), flow32, gx32, _strides(gx32), gflow, n, c, h, w,
+                _dtype_code("backwarp", xd))
+        return _grad(gx32, xd.dtype), _grad(gflow, ctx.flow_dtype)
 
 
 def _backwarp(name, tenInput, tenFlow):
@@ -378,7 +358,7 @@ def _dcn_workspace(weight, dtype, ws_bytes, static):
     nothing = lambda: None      # noqa: E731
     if not static or (torch.is_grad_enabled() and weight.requires_grad):
         return torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=weight.device), False, nothing
-    key = (id(weight), torch.cuda.current_stream(weight.device).cuda_stream)
+    key = (id(weight), torch.cuda.current_stream(weight.device))
     with _DCN_WS_LOCK:
         hit = _DCN_WS_CACHE.get(key)
     if hit is not None:
@@ -438,28 +418,22 @@ class _ModulatedDeformConv2dFn(Function):
         if tuple(mask.shape) != (n, deform_groups * K, ho, wo):
             raise ValueError(f"modulated_deform_conv2d: mask shape {tuple(mask.shape)}, expected "
                              f"{(n, deform_groups * K, ho, wo)}")
-        with torch.cuda.device(input.device):
-            code = _dtype_code("modulated_deform_conv2d", input)
-            xd = _dcn_prepare_x(input, weight, groups)
-            off32 = offset.detach().to(torch.float32).contiguous()
-            msk32 = mask.detach().to(torch.float32).contiguous()
-            wd = weight.detach().to(input.dtype).contiguous()
-            bd = bias.detach().to(input.dtype).contiguous() if bias is not None else None
-            out = _empty_like_layout(xd, channels=cout, hw=(ho, wo))
-            ws_bytes = lib.eavsr_dcn_forward_workspace(cin, cout, kh, kw, groups, deform_groups, code)
-            ws, packed, commit = _dcn_workspace(weight, input.dtype, ws_bytes, bool(flags & _DCN_STATIC_WEIGHT))
-            flags &= ~_DCN_STATIC_WEIGHT
-            if packed:
-                flags |= DCN_WS_PACKED
-            L.check(lib.eavsr_dcn_forward(xd.data_ptr(), _strides(xd), off32.data_ptr(), msk32.data_ptr(),
-                                          wd.data_ptr(), _ptr(bd), out.data_ptr(), _strides(out), n, cin, h, w,
-                                          cout, kh, kw, sh, sw, ph, pw, dh, dw, groups, deform_groups, code,
-                                          ws.data_ptr(), ws.numel(), flags, _stream(xd)),
-                    "dcn_forward")
-            if ws_bytes and lib.eavsr_dcn_forward_uses_tensor_cores(
-                    _strides(xd), _strides(out), cin, cout, kh, kw, sh, sw, ph, pw, dh, dw, groups, deform_groups,
-                    flags):
-                commit()        # only a tensor-core launch has packed the workspace
+        code = _dtype_code("modulated_deform_conv2d", input)
+        xd = _dcn_prepare_x(input, weight, groups)
+        off32 = _param(offset, torch.float32)
+        msk32 = _param(mask, torch.float32)
+        wd = _param(weight, input.dtype)
+        out = _empty_like_layout(xd, channels=cout, hw=(ho, wo))
+        ws_bytes = lib.eavsr_dcn_forward_workspace(cin, cout, kh, kw, groups, deform_groups, code)
+        ws, packed, commit = _dcn_workspace(weight, input.dtype, ws_bytes, bool(flags & _DCN_STATIC_WEIGHT))
+        flags &= ~_DCN_STATIC_WEIGHT
+        if packed:
+            flags |= DCN_WS_PACKED
+        _launch("dcn_forward", xd, _strides(xd), off32, msk32, wd, _param(bias, input.dtype), out, _strides(out),
+                n, cin, h, w, cout, kh, kw, sh, sw, ph, pw, dh, dw, groups, deform_groups, code, ws, ws.numel(), flags)
+        if ws_bytes and lib.eavsr_dcn_forward_uses_tensor_cores(
+                _strides(xd), _strides(out), cin, cout, kh, kw, sh, sw, ph, pw, dh, dw, groups, deform_groups, flags):
+            commit()        # only a tensor-core launch has packed the workspace
         ctx.save_for_backward(xd, off32, msk32, wd)
         ctx.geom = (sh, sw, ph, pw, dh, dw, groups, deform_groups)
         ctx.bwd_flags = flags & (L.DCN_FORCE_GENERIC | L.DCN_BWD_GENERIC_DATA | L.DCN_BWD_GENERIC_WEIGHT)
@@ -471,35 +445,25 @@ class _ModulatedDeformConv2dFn(Function):
     @once_differentiable
     def backward(ctx, gout):
         xd, off32, msk32, wd = ctx.saved_tensors
-        lib = L.load()
         sh, sw, ph, pw, dh, dw, groups, dg = ctx.geom
         need = ctx.needs_input_grad
         n, cin, h, w = xd.shape
         cout, _, kh, kw = wd.shape
-        with torch.cuda.device(xd.device):
-            fmt = torch.channels_last if _is_channels_last(xd) else torch.contiguous_format
-            g = gout.to(xd.dtype).contiguous(memory_format=fmt)
-            gx32 = _empty_like_layout(xd, dtype=torch.float32) if need[0] else None
-            goff = torch.empty_like(off32) if need[1] else None
-            gmsk = torch.empty_like(msk32) if need[2] else None
-            gw32 = torch.empty(wd.shape, dtype=torch.float32, device=xd.device) if need[3] else None
-            gb32 = torch.empty(cout, dtype=torch.float32, device=xd.device) if (need[4] and ctx.has_bias) else None
-            code = _dtype_code("modulated_deform_conv2d", xd)
-            ws_bytes = lib.eavsr_dcn_backward_workspace(cin, cout, kh, kw, groups, dg, code)
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=xd.device) if ws_bytes else None
-            L.check(lib.eavsr_dcn_backward(g.data_ptr(), _strides(g), xd.data_ptr(), _strides(xd),
-                                           off32.data_ptr(), msk32.data_ptr(), wd.data_ptr(), _ptr(gx32),
-                                           _strides(gx32) if gx32 is not None else None, _ptr(goff), _ptr(gmsk),
-                                           _ptr(gw32), _ptr(gb32), n, cin, h, w, cout, kh, kw, sh, sw, ph, pw,
-                                           dh, dw, groups, dg, code, _ptr(ws), ws_bytes, ctx.bwd_flags,
-                                           _stream(xd)),
-                    "dcn_backward")
+        fmt = torch.channels_last if _is_channels_last(xd) else torch.contiguous_format
+        g = gout.to(xd.dtype).contiguous(memory_format=fmt)
+        gx32 = _empty_like_layout(xd, dtype=torch.float32) if need[0] else None
+        goff = torch.empty_like(off32) if need[1] else None
+        gmsk = torch.empty_like(msk32) if need[2] else None
+        gw32 = torch.empty(wd.shape, dtype=torch.float32, device=xd.device) if need[3] else None
+        gb32 = torch.empty(cout, dtype=torch.float32, device=xd.device) if (need[4] and ctx.has_bias) else None
+        code = _dtype_code("modulated_deform_conv2d", xd)
+        ws_bytes = L.load().eavsr_dcn_backward_workspace(cin, cout, kh, kw, groups, dg, code)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=xd.device) if ws_bytes else None
+        _launch("dcn_backward", g, _strides(g), xd, _strides(xd), off32, msk32, wd, gx32, _strides(gx32), goff, gmsk,
+                gw32, gb32, n, cin, h, w, cout, kh, kw, sh, sw, ph, pw, dh, dw, groups, dg, code, ws, ws_bytes,
+                ctx.bwd_flags)
         od, md, wdt, bdt = ctx.in_dtypes
-        return (gx32.to(xd.dtype) if gx32 is not None else None,
-                goff.to(od) if goff is not None else None,
-                gmsk.to(md) if gmsk is not None else None,
-                gw32.to(wdt) if gw32 is not None else None,
-                gb32.to(bdt) if gb32 is not None else None,
+        return (_grad(gx32, xd.dtype), _grad(goff, od), _grad(gmsk, md), _grad(gw32, wdt), _grad(gb32, bdt),
                 None, None, None, None, None, None)
 
 
@@ -572,15 +536,11 @@ class _FunctionCorrelation(Function):
             raise NotImplementedError()          # pwc/correlation/correlation.py:324-325
         if first.shape != second.shape or first.dim() != 4:
             raise ValueError(f"correlation: shapes {tuple(first.shape)} / {tuple(second.shape)}")
-        lib = L.load()
         n, c, h, w = first.shape
-        with torch.cuda.device(first.device):
-            code = _dtype_code("FunctionCorrelation", first)
-            second = second.to(first.dtype)
-            out = first.new_empty((n, 81, h, w))
-            L.check(lib.eavsr_correlation_forward_ex(first.data_ptr(), second.data_ptr(), out.data_ptr(), n, c, h, w,
-                                                     code, L.CORR_TF32 if CORRELATION_TF32 else 0,
-                                                     _stream(first)), "correlation_forward")
+        code = _dtype_code("FunctionCorrelation", first)
+        second = second.to(first.dtype)
+        out = first.new_empty((n, 81, h, w))
+        _launch("correlation_forward_ex", first, second, out, n, c, h, w, code, L.CORR_TF32 if CORRELATION_TF32 else 0)
         ctx.save_for_backward(first, second)
         return out
 
@@ -588,16 +548,12 @@ class _FunctionCorrelation(Function):
     @once_differentiable
     def backward(ctx, gout):
         first, second = ctx.saved_tensors
-        lib = L.load()
         n, c, h, w = first.shape
-        with torch.cuda.device(first.device):
-            g = gout.to(first.dtype).contiguous()
-            g1 = torch.empty_like(first) if ctx.needs_input_grad[0] else None
-            g2 = torch.empty_like(second) if ctx.needs_input_grad[1] else None
-            if g1 is not None or g2 is not None:
-                L.check(lib.eavsr_correlation_backward(first.data_ptr(), second.data_ptr(), g.data_ptr(), _ptr(g1),
-                                                       _ptr(g2), n, c, h, w, _dtype_code("FunctionCorrelation", first),
-                                                       _stream(first)), "correlation_backward")
+        g1 = torch.empty_like(first) if ctx.needs_input_grad[0] else None
+        g2 = torch.empty_like(second) if ctx.needs_input_grad[1] else None
+        if g1 is not None or g2 is not None:
+            _launch("correlation_backward", first, second, gout.to(first.dtype).contiguous(), g1, g2, n, c, h, w,
+                    _dtype_code("FunctionCorrelation", first))
         return g1, g2
 
 
@@ -616,16 +572,6 @@ class ModuleCorrelation(nn.Module):
 # fused inference-only producers / consumers around the hot path (no autograd: the callers in
 # eavsr_b200.model use the PyTorch modules whenever a gradient is required)
 # ------------------------------------------------------------------------------------------
-def _b(bias, like):
-    return None if bias is None else bias.detach().to(like.dtype).contiguous()
-
-
-def _as(t, dtype):
-    """Detached contiguous `dtype` view / copy of a parameter.  Keep the result in a local until the launch
-    has been issued (see adapt_mix)."""
-    return t.detach().to(dtype).contiguous()
-
-
 def fused_inference_ok(*tensors) -> bool:
     """True when the fused (non-differentiable) kernels may be used: autograd is off (``torch.no_grad()`` /
     ``inference_mode``) and every tensor is a CUDA fp32 / bf16 tensor."""
@@ -643,20 +589,12 @@ def adapt_mix(a, b, w1, b1, w2, b2, negative_slope: float = 0.2):
     """``concat2(concat(cat[a, b]))`` of the reference's AdaptBlocks (models/networks.py:289-290,299):
     depthwise 3x3 + LeakyReLU + grouped (2->1) 3x3 + LeakyReLU in one pass.  a, b: (n,64,h,w)."""
     _require_cuda("adapt_mix", a, b, w1, b1, w2, b2)
-    lib = L.load()
     n, c, h, w = a.shape
-    with torch.cuda.device(a.device):
-        ad = a.contiguous(memory_format=torch.channels_last)
-        bd = b.to(a.dtype).contiguous(memory_format=torch.channels_last)
-        out = torch.empty_like(ad)
-        # converted parameters are bound to locals that outlive the launch: `.data_ptr()` of a temporary
-        # would be handed back to the caching allocator before the next conversion in the argument list
-        w1d, b1d, w2d, b2d = (_as(t, a.dtype) for t in (w1, b1, w2, b2))
-        L.check(lib.eavsr_adapt_mix_forward(ad.data_ptr(), bd.data_ptr(), w1d.data_ptr(), b1d.data_ptr(),
-                                            w2d.data_ptr(), b2d.data_ptr(), out.data_ptr(), n, c, h, w,
-                                            float(negative_slope), _dtype_code("adapt_mix", ad), _stream(ad)),
-                "adapt_mix")
-        del w1d, b1d, w2d, b2d
+    ad = a.contiguous(memory_format=torch.channels_last)
+    out = torch.empty_like(ad)
+    _launch("adapt_mix_forward", ad, b.to(a.dtype).contiguous(memory_format=torch.channels_last),
+            *(_param(t, a.dtype) for t in (w1, b1, w2, b2)), out, n, c, h, w, float(negative_slope),
+            _dtype_code("adapt_mix", ad))
     return out
 
 
@@ -666,24 +604,18 @@ def affine_offsets_mask(transform, translation, mask_logits, deform_groups: int,
     (models/networks.py:302-313) -> fp32 NCHW (offset (n,18D,h,w), mask (n,9D,h,w) or None).
     The optional biases are added to T / t / logits first (bias-free producing convolutions)."""
     _require_cuda("affine_offsets_mask", transform, translation, mask_logits)
-    lib = L.load()
     n, _, h, w = transform.shape
     D = deform_groups
-    with torch.cuda.device(transform.device):
-        translation = translation.to(transform.dtype)
-        offset = torch.empty((n, 18 * D, h, w), dtype=torch.float32, device=transform.device)
-        mask = None
-        if mask_logits is not None:
-            mask_logits = mask_logits.to(transform.dtype)
-            mask = torch.empty((n, 9 * D, h, w), dtype=torch.float32, device=transform.device)
-        bT, bt, bm = _b(transform_bias, transform), _b(translation_bias, transform), _b(mask_bias, transform)
-        L.check(lib.eavsr_affine_offsets_forward(
-            transform.data_ptr(), _strides(transform), translation.data_ptr(), _strides(translation),
-            _ptr(mask_logits), _strides(mask_logits) if mask_logits is not None else None,
-            _ptr(bT), _ptr(bt), _ptr(bm), offset.data_ptr(),
-            _ptr(mask), n, D, h, w, _dtype_code("affine_offsets_mask", transform), _stream(transform)),
-            "affine_offsets")
-        del bT, bt, bm
+    translation = translation.to(transform.dtype)
+    offset = torch.empty((n, 18 * D, h, w), dtype=torch.float32, device=transform.device)
+    mask = None
+    if mask_logits is not None:
+        mask_logits = mask_logits.to(transform.dtype)
+        mask = torch.empty((n, 9 * D, h, w), dtype=torch.float32, device=transform.device)
+    biases = [_param(t, transform.dtype) for t in (transform_bias, translation_bias, mask_bias)]
+    _launch("affine_offsets_forward", transform, _strides(transform), translation, _strides(translation),
+            mask_logits, _strides(mask_logits), *biases, offset, mask, n, D, h, w,
+            _dtype_code("affine_offsets_mask", transform))
     return offset, mask
 
 
@@ -708,26 +640,20 @@ def dcn_affine(x, affine, affine_bias, weight, bias, deform_groups: int = 8, sta
     Inference only; check `dcn_affine_eligible` first.  ``out`` may be a 64-channel slice (dim 1) of a wider
     channels_last bf16 buffer: the result is written in place there (no torch.cat copy afterwards)."""
     _require_cuda("dcn_affine", x, affine, weight)
-    lib = L.load()
     n, c, h, w = x.shape
-    with torch.cuda.device(x.device):
-        xd = x.contiguous(memory_format=torch.channels_last)
-        wd = weight.detach().to(x.dtype).contiguous()
-        bd = bias.detach().to(x.dtype).contiguous() if bias is not None else None
-        ab = affine_bias.detach().to(x.dtype).contiguous() if affine_bias is not None else None
-        if out is None:
-            out = torch.empty_like(xd)
-        else:
-            assert out.shape == xd.shape and out.dtype == xd.dtype and out.stride(1) == 1, "dcn_affine: bad out view"
-        code = _dtype_code("dcn_affine", xd)
-        ws_bytes = lib.eavsr_dcn_forward_workspace(64, 64, 3, 3, 1, deform_groups, code)
-        ws, packed, commit = _dcn_workspace(weight, x.dtype, ws_bytes, static_weight)
-        if packed:
-            flags |= DCN_WS_PACKED
-        L.check(lib.eavsr_dcn_affine_forward(xd.data_ptr(), _strides(xd), affine.data_ptr(), _ptr(ab), wd.data_ptr(),
-                                             _ptr(bd), out.data_ptr(), _strides(out), n, h, w, deform_groups, code,
-                                             ws.data_ptr(), ws.numel(), flags, _stream(xd)), "dcn_affine_forward")
-        commit()
+    xd = x.contiguous(memory_format=torch.channels_last)
+    if out is None:
+        out = torch.empty_like(xd)
+    else:
+        assert out.shape == xd.shape and out.dtype == xd.dtype and out.stride(1) == 1, "dcn_affine: bad out view"
+    code = _dtype_code("dcn_affine", xd)
+    ws_bytes = L.load().eavsr_dcn_forward_workspace(64, 64, 3, 3, 1, deform_groups, code)
+    ws, packed, commit = _dcn_workspace(weight, x.dtype, ws_bytes, static_weight)
+    if packed:
+        flags |= DCN_WS_PACKED
+    _launch("dcn_affine_forward", xd, _strides(xd), affine, _param(affine_bias, x.dtype), _param(weight, x.dtype),
+            _param(bias, x.dtype), out, _strides(out), n, h, w, deform_groups, code, ws, ws.numel(), flags)
+    commit()
     return out
 
 
@@ -736,21 +662,13 @@ def ca_residual(res, skip, w1, b1, w2, b2, reduction: int = 16, res_bias=None):
     (models/networks.py:449-465) with two kernels (channel sums; MLP + scale + residual).
     ``res_bias`` lets the producing convolution run bias-free.  res, skip: (n,64,h,w)."""
     _require_cuda("ca_residual", res, skip, w1, b1, w2, b2)
-    lib = L.load()
     n, c, h, w = res.shape
-    with torch.cuda.device(res.device):
-        rd = res.contiguous(memory_format=torch.channels_last)
-        sd = skip.to(res.dtype).contiguous(memory_format=torch.channels_last)
-        out = torch.empty_like(rd)
-        sums = torch.empty((n, c), dtype=torch.float32, device=res.device)
-        w1d, b1d, w2d, b2d = (_as(t, res.dtype) for t in (w1, b1, w2, b2))
-        rb = _b(res_bias, res)
-        L.check(lib.eavsr_ca_residual_forward(rd.data_ptr(), sd.data_ptr(), w1d.data_ptr(), b1d.data_ptr(),
-                                              w2d.data_ptr(), b2d.data_ptr(), _ptr(rb),
-                                              out.data_ptr(), sums.data_ptr(),
-                                              n, c, h, w, reduction, _dtype_code("ca_residual", rd), _stream(rd)),
-                "ca_residual")
-        del w1d, b1d, w2d, b2d, rb
+    rd = res.contiguous(memory_format=torch.channels_last)
+    out = torch.empty_like(rd)
+    sums = torch.empty((n, c), dtype=torch.float32, device=res.device)
+    _launch("ca_residual_forward", rd, skip.to(res.dtype).contiguous(memory_format=torch.channels_last),
+            *(_param(t, res.dtype) for t in (w1, b1, w2, b2, res_bias)), out, sums, n, c, h, w, reduction,
+            _dtype_code("ca_residual", rd))
     return out
 
 
@@ -758,16 +676,11 @@ def bias_act_(x, bias, negative_slope: float = 1.0):
     """In place ``x = LeakyReLU_slope(x + bias[c])`` on a channels_last tensor (slope 1: bias only,
     0: ReLU).  Returns x."""
     _require_cuda("bias_act_", x, bias)
-    lib = L.load()
     n, c, h, w = x.shape
     if not x.is_contiguous(memory_format=torch.channels_last):
         raise ValueError("bias_act_: x must be dense channels_last")
-    with torch.cuda.device(x.device):
-        bd = _as(bias, x.dtype)
-        L.check(lib.eavsr_bias_act_forward(x.data_ptr(), bd.data_ptr(), c, n * h * w,
-                                           float(negative_slope), _dtype_code("bias_act_", x), _stream(x)),
-                "bias_act")
-        del bd
+    _launch("bias_act_forward", x, _param(bias, x.dtype), c, n * h * w, float(negative_slope),
+            _dtype_code("bias_act_", x))
     return x
 
 
@@ -777,17 +690,13 @@ class _GroupedConv3x3Fn(Function):
 
     @staticmethod
     def forward(ctx, x, weight, bias):
-        lib = L.load()
         n, cin, h, w = x.shape
         cout = weight.shape[0]
-        with torch.cuda.device(x.device):
-            xd = x.contiguous(memory_format=torch.channels_last)
-            wd = weight.detach().to(xd.dtype).contiguous()
-            bd = None if bias is None else bias.detach().to(xd.dtype).contiguous()
-            out = torch.empty((n, cout, h, w), dtype=xd.dtype, device=xd.device, memory_format=torch.channels_last)
-            L.check(lib.eavsr_grouped_conv3x3_forward(xd.data_ptr(), wd.data_ptr(), _ptr(bd), out.data_ptr(), n, cin, cout,
-                                                      h, w, _dtype_code("grouped_conv3x3", xd), _stream(xd)),
-                    "grouped_conv3x3_forward")
+        xd = x.contiguous(memory_format=torch.channels_last)
+        wd = _param(weight, xd.dtype)
+        out = torch.empty((n, cout, h, w), dtype=xd.dtype, device=xd.device, memory_format=torch.channels_last)
+        _launch("grouped_conv3x3_forward", xd, wd, _param(bias, xd.dtype), out, n, cin, cout, h, w,
+                _dtype_code("grouped_conv3x3", xd))
         ctx.save_for_backward(xd, wd)
         ctx.has_bias, ctx.wdtype, ctx.bdtype = bias is not None, weight.dtype, None if bias is None else bias.dtype
         return out
@@ -796,23 +705,15 @@ class _GroupedConv3x3Fn(Function):
     @once_differentiable
     def backward(ctx, gout):
         xd, wd = ctx.saved_tensors
-        lib = L.load()
         n, cin, h, w = xd.shape
         cout = wd.shape[0]
         need_x, need_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2])
-        gx = gw = gb = None
-        with torch.cuda.device(xd.device):
-            g = gout.to(xd.dtype).contiguous(memory_format=torch.channels_last)
-            if need_x:
-                gx = torch.empty_like(xd)
-            if need_w:
-                gw = torch.zeros(wd.shape, dtype=torch.float32, device=xd.device)
-                gb = torch.zeros(cout, dtype=torch.float32, device=xd.device)
-            L.check(lib.eavsr_grouped_conv3x3_backward(g.data_ptr(), xd.data_ptr(), wd.data_ptr(), _ptr(gx), _ptr(gw), _ptr(gb),
-                                                       n, cin, cout, h, w, _dtype_code("grouped_conv3x3", xd), _stream(xd)),
-                    "grouped_conv3x3_backward")
-        return (gx, None if gw is None else gw.to(ctx.wdtype),
-                None if (gb is None or not ctx.has_bias) else gb.to(ctx.bdtype))
+        g = gout.to(xd.dtype).contiguous(memory_format=torch.channels_last)
+        gx = torch.empty_like(xd) if need_x else None
+        gw = torch.zeros(wd.shape, dtype=torch.float32, device=xd.device) if need_w else None
+        gb = torch.zeros(cout, dtype=torch.float32, device=xd.device) if need_w else None
+        _launch("grouped_conv3x3_backward", g, xd, wd, gx, gw, gb, n, cin, cout, h, w, _dtype_code("grouped_conv3x3", xd))
+        return gx, _grad(gw, ctx.wdtype), (_grad(gb, ctx.bdtype) if ctx.has_bias else None)
 
 
 def grouped_conv3x3_eligible(conv: nn.Conv2d, x) -> bool:
@@ -841,12 +742,9 @@ def grouped_conv3x3(conv: nn.Conv2d, x):
 
 def _channel_sums(x):
     """(n, 64) fp32 sums over (h, w) of a CUDA channels_last 64-channel fp32 / bf16 tensor."""
-    lib = L.load()
     n, c, h, w = x.shape
-    with torch.cuda.device(x.device):
-        sums = torch.empty((n, c), dtype=torch.float32, device=x.device)
-        L.check(lib.eavsr_channel_sum_forward(x.data_ptr(), sums.data_ptr(), n, c, h * w, _dtype_code("channel_sum", x),
-                                              _stream(x)), "channel_sum")
+    sums = torch.empty((n, c), dtype=torch.float32, device=x.device)
+    _launch("channel_sum_forward", x, sums, n, c, h * w, _dtype_code("channel_sum", x))
     return sums
 
 
@@ -918,11 +816,8 @@ class _ScaleResidualFn(Function):
         gscale = None
         if ctx.needs_input_grad[1]:
             n, c, h, w = res.shape
-            lib = L.load()
-            with torch.cuda.device(res.device):
-                sums = torch.empty((n, c), dtype=torch.float32, device=res.device)
-                L.check(lib.eavsr_channel_dot_forward(g.data_ptr(), res.data_ptr(), sums.data_ptr(), n, c, h * w,
-                                                      _dtype_code("scale_residual", res), _stream(res)), "channel_dot")
+            sums = torch.empty((n, c), dtype=torch.float32, device=res.device)
+            _launch("channel_dot_forward", g, res, sums, n, c, h * w, _dtype_code("scale_residual", res))
             gscale = sums.to(scale.dtype).view(n, c, 1, 1)
         return gres, gscale, gout if ctx.needs_input_grad[2] else None
 
@@ -965,15 +860,13 @@ def cat_channels(tensors, out=None, channel_offset: int = 0):
             return torch.cat(ts, 1)
         out[:, channel_offset:channel_offset + ctot].copy_(torch.cat(ts, 1) if len(ts) > 1 else x0)
         return out
-    lib = L.load()
     n, _, h, w = x0.shape
-    with torch.cuda.device(x0.device):
-        if out is None:
-            out = torch.empty((n, ctot, h, w), dtype=x0.dtype, device=x0.device, memory_format=torch.channels_last)
-        ptrs = (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
-        chans = (ctypes.c_int * len(ts))(*[t.shape[1] for t in ts])
-        L.check(lib.eavsr_nhwc_cat_forward(ptrs, chans, len(ts), out.data_ptr(), out.shape[1], channel_offset,
-                                           n * h * w, _dtype_code("cat_channels", x0), _stream(x0)), "nhwc_cat")
+    if out is None:
+        out = torch.empty((n, ctot, h, w), dtype=x0.dtype, device=x0.device, memory_format=torch.channels_last)
+    ptrs = (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
+    chans = (ctypes.c_int * len(ts))(*[t.shape[1] for t in ts])
+    _launch("nhwc_cat_forward", ptrs, chans, len(ts), out, out.shape[1], channel_offset, n * h * w,
+            _dtype_code("cat_channels", x0))
     return out
 
 
@@ -1013,11 +906,8 @@ def _packed_conv_weight(conv: nn.Conv2d, device) -> torch.Tensor:
     hit = getattr(conv, "_eavsr_packed", None)
     if hit is not None and hit[0] == key:
         return hit[1]
-    lib = L.load()
-    packed = torch.empty(lib.eavsr_conv3x3_packed_weight_bytes(), dtype=torch.uint8, device=device)
-    wb = w.detach().to(device=device, dtype=torch.bfloat16).contiguous()
-    L.check(lib.eavsr_conv3x3_pack_weight(wb.data_ptr(), packed.data_ptr(), 64, 64, L.BF16,
-                                          torch.cuda.current_stream(device).cuda_stream), "conv3x3_pack_weight")
+    packed = torch.empty(L.load().eavsr_conv3x3_packed_weight_bytes(), dtype=torch.uint8, device=device)
+    _launch("conv3x3_pack_weight", _param(w.to(device), torch.bfloat16), packed, 64, 64, L.BF16)
     conv._eavsr_packed = (key, packed)
     return packed
 
@@ -1028,25 +918,19 @@ def conv3x3_64(conv: nn.Conv2d, x, negative_slope: float = 1.0, want_sums: bool 
     output over (h, w) in fp32, computed in the epilogue; ``sums_out`` is an already ZEROED (n, 64)
     fp32 buffer to accumulate them into (one memset for a whole residual group instead of one per
     convolution).  Check `conv3x3_64_eligible` first."""
-    lib = L.load()
     n, c, h, w = x.shape
-    with torch.cuda.device(x.device):
-        xd = x.contiguous(memory_format=torch.channels_last)
-        out = torch.empty_like(xd)
-        sums = None
-        if want_sums:
-            if sums_out is not None:
-                assert sums_out.shape == (n, 64) and sums_out.dtype == torch.float32 and sums_out.is_contiguous()
-                sums = sums_out
-            else:
-                sums = torch.empty((n, 64), dtype=torch.float32, device=x.device)
-        packed = _packed_conv_weight(conv, x.device)
-        bias = conv.bias.detach().to(torch.bfloat16).contiguous() if conv.bias is not None else None
-        L.check(lib.eavsr_conv3x3_forward(xd.data_ptr(), packed.data_ptr(), _ptr(bias), out.data_ptr(), _ptr(sums),
-                                          n, 64, 64, h, w, float(negative_slope), L.BF16,
-                                          L.CONV_SUMS_PREZEROED if (want_sums and sums_out is not None) else 0,
-                                          _stream(xd)),
-                "conv3x3_forward")
+    xd = x.contiguous(memory_format=torch.channels_last)
+    out = torch.empty_like(xd)
+    sums = None
+    if want_sums:
+        if sums_out is not None:
+            assert sums_out.shape == (n, 64) and sums_out.dtype == torch.float32 and sums_out.is_contiguous()
+            sums = sums_out
+        else:
+            sums = torch.empty((n, 64), dtype=torch.float32, device=x.device)
+    _launch("conv3x3_forward", xd, _packed_conv_weight(conv, x.device), _param(conv.bias, torch.bfloat16), out, sums,
+            n, 64, 64, h, w, float(negative_slope), L.BF16,
+            L.CONV_SUMS_PREZEROED if (want_sums and sums_out is not None) else 0)
     return (out, sums) if want_sums else out
 
 
@@ -1056,27 +940,17 @@ def conv3x3_64_ca(conv: nn.Conv2d, skip, res, res_sums, w1, b1, w2, b2, negative
     ``LeakyReLU_slope(conv(y))``: returns ``(out, y)`` or ``(out, y, sums)``.  ``res_sums`` are the channel
     sums of ``res`` from the `conv3x3_64(..., want_sums=True)` call that produced it.  Same eligibility as
     `conv3x3_64`, batch <= 8."""
-    lib = L.load()
     n, c, h, w = skip.shape
-    with torch.cuda.device(skip.device):
-        sd = skip.contiguous(memory_format=torch.channels_last)
-        rd = res.contiguous(memory_format=torch.channels_last)
-        out = torch.empty_like(sd)
-        y = torch.empty_like(sd)
-        sums = None
-        if want_sums:
-            sums = sums_out if sums_out is not None else torch.empty((n, 64), dtype=torch.float32, device=skip.device)
-        packed = _packed_conv_weight(conv, skip.device)
-        bias = conv.bias.detach().to(torch.bfloat16).contiguous() if conv.bias is not None else None
-        w1d, b1d, w2d, b2d = (_as(t, skip.dtype) for t in (w1, b1, w2, b2))
-        L.check(lib.eavsr_conv3x3_ca_forward(sd.data_ptr(), rd.data_ptr(), res_sums.data_ptr(),
-                                             w1d.data_ptr(), b1d.data_ptr(), w2d.data_ptr(), b2d.data_ptr(),
-                                             y.data_ptr(), packed.data_ptr(), _ptr(bias), out.data_ptr(), _ptr(sums),
-                                             n, h, w, float(negative_slope), L.BF16,
-                                             L.CONV_SUMS_PREZEROED if (want_sums and sums_out is not None) else 0,
-                                             _stream(sd)),
-                "conv3x3_ca_forward")
-        del w1d, b1d, w2d, b2d
+    sd = skip.contiguous(memory_format=torch.channels_last)
+    out = torch.empty_like(sd)
+    y = torch.empty_like(sd)
+    sums = None
+    if want_sums:
+        sums = sums_out if sums_out is not None else torch.empty((n, 64), dtype=torch.float32, device=skip.device)
+    _launch("conv3x3_ca_forward", sd, res.contiguous(memory_format=torch.channels_last), res_sums,
+            *(_param(t, skip.dtype) for t in (w1, b1, w2, b2)), y, _packed_conv_weight(conv, skip.device),
+            _param(conv.bias, torch.bfloat16), out, sums, n, h, w, float(negative_slope), L.BF16,
+            L.CONV_SUMS_PREZEROED if (want_sums and sums_out is not None) else 0)
     return (out, y, sums) if want_sums else (out, y)
 
 
@@ -1092,72 +966,61 @@ def rca_group_chain(blocks, tail_conv, x):
     conv + ReLU with the previous block's channel attention folded into its input, conv + channel sums -- and the
     closing convolution.  ``blocks``: modules with ``res[0]``, ``res[2]`` (3x3 convs) and ``ca.conv_du`` (the
     squeeze-excite 1x1 convs); inference only (check `conv3x3_chain_eligible`)."""
-    lib = L.load()
     n, c, h, w = x.shape
     dev = x.device
-    with torch.cuda.device(dev):
-        xd = x.contiguous(memory_format=torch.channels_last)
-        # activations: h (conv1 output), res (conv2 output), y ping-pong (block outputs); sums one row per block
-        hbuf, rbuf, out = torch.empty_like(xd), torch.empty_like(xd), torch.empty_like(xd)
-        ybuf = [torch.empty_like(xd), torch.empty_like(xd)]
-        pool = torch.zeros((len(blocks), n, 64), dtype=torch.float32, device=dev)
-        sync = torch.empty(1, dtype=torch.int32, device=dev)
-        keep = []                      # converted parameters must outlive the launch
+    xd = x.contiguous(memory_format=torch.channels_last)
+    # activations: h (conv1 output), res (conv2 output), y ping-pong (block outputs); sums one row per block
+    hbuf, rbuf, out = torch.empty_like(xd), torch.empty_like(xd), torch.empty_like(xd)
+    ybuf = [torch.empty_like(xd), torch.empty_like(xd)]
+    pool = torch.zeros((len(blocks), n, 64), dtype=torch.float32, device=dev)
+    sync = torch.empty(1, dtype=torch.int32, device=dev)
+    keep = []                      # `arr` holds raw addresses: converted parameters must outlive the launch
 
-        def par(t):
-            t = _as(t, torch.bfloat16)
-            keep.append(t)
-            return t.data_ptr()
+    def par(t):
+        t = _param(t, torch.bfloat16)
+        keep.append(t)
+        return t.data_ptr()
 
-        layers = []
-        y = xd
-        for i, blk in enumerate(blocks):
-            c1, c2 = blk.res[0], blk.res[2]
-            if i == 0:
-                layers.append(dict(x=y, conv=c1, out=hbuf, slope=0.0))
-            else:
-                du = blocks[i - 1].ca.conv_du
-                ynew = ybuf[i & 1]
-                layers.append(dict(x=y, conv=c1, out=hbuf, slope=0.0, res=rbuf, res_sums=pool[i - 1], du=du, y_out=ynew))
-                y = ynew
-            layers.append(dict(x=hbuf, conv=c2, out=rbuf, slope=1.0, sums=pool[i]))
-        du = blocks[-1].ca.conv_du
-        layers.append(dict(x=y, conv=tail_conv, out=out, slope=1.0, res=rbuf, res_sums=pool[len(blocks) - 1], du=du,
-                           y_out=ybuf[len(blocks) & 1]))
-        arr = (L.ConvLayer * len(layers))()
-        for a, d in zip(arr, layers):
-            conv = d["conv"]
-            a.x, a.out = d["x"].data_ptr(), d["out"].data_ptr()
-            a.packed_weight = _packed_conv_weight(conv, dev).data_ptr()
-            a.bias = par(conv.bias) if conv.bias is not None else None
-            a.channel_sums = d["sums"].data_ptr() if "sums" in d else None
-            a.negative_slope = d["slope"]
-            if "res" in d:
-                du = d["du"]
-                a.res, a.res_sums, a.y_out = d["res"].data_ptr(), d["res_sums"].data_ptr(), d["y_out"].data_ptr()
-                a.w1, a.b1, a.w2, a.b2 = par(du[0].weight), par(du[0].bias), par(du[2].weight), par(du[2].bias)
-        L.check(lib.eavsr_conv3x3_chain_forward(arr, len(layers), n, h, w, L.BF16, sync.data_ptr(), _stream(xd)),
-                "conv3x3_chain_forward")
-        del keep
+    layers = []
+    y = xd
+    for i, blk in enumerate(blocks):
+        c1, c2 = blk.res[0], blk.res[2]
+        if i == 0:
+            layers.append(dict(x=y, conv=c1, out=hbuf, slope=0.0))
+        else:
+            du = blocks[i - 1].ca.conv_du
+            ynew = ybuf[i & 1]
+            layers.append(dict(x=y, conv=c1, out=hbuf, slope=0.0, res=rbuf, res_sums=pool[i - 1], du=du, y_out=ynew))
+            y = ynew
+        layers.append(dict(x=hbuf, conv=c2, out=rbuf, slope=1.0, sums=pool[i]))
+    du = blocks[-1].ca.conv_du
+    layers.append(dict(x=y, conv=tail_conv, out=out, slope=1.0, res=rbuf, res_sums=pool[len(blocks) - 1], du=du,
+                       y_out=ybuf[len(blocks) & 1]))
+    arr = (L.ConvLayer * len(layers))()
+    for a, d in zip(arr, layers):
+        conv = d["conv"]
+        a.x, a.out = d["x"].data_ptr(), d["out"].data_ptr()
+        a.packed_weight = _packed_conv_weight(conv, dev).data_ptr()
+        a.bias = par(conv.bias) if conv.bias is not None else None
+        a.channel_sums = d["sums"].data_ptr() if "sums" in d else None
+        a.negative_slope = d["slope"]
+        if "res" in d:
+            du = d["du"]
+            a.res, a.res_sums, a.y_out = d["res"].data_ptr(), d["res_sums"].data_ptr(), d["y_out"].data_ptr()
+            a.w1, a.b1, a.w2, a.b2 = par(du[0].weight), par(du[0].bias), par(du[2].weight), par(du[2].bias)
+    _launch("conv3x3_chain_forward", arr, len(layers), n, h, w, L.BF16, sync)
     return out
 
 
 def ca_scale(res, skip, sums, w1, b1, w2, b2, reduction: int = 16, res_bias=None):
     """``(res + res_bias) * sigmoid(MLP(sums / HW + res_bias)) + skip`` with channel sums that were
     produced by the convolution's epilogue (see `conv3x3_64`)."""
-    lib = L.load()
     n, c, h, w = res.shape
-    with torch.cuda.device(res.device):
-        rd = res.contiguous(memory_format=torch.channels_last)
-        sd = skip.to(res.dtype).contiguous(memory_format=torch.channels_last)
-        out = torch.empty_like(rd)
-        w1d, b1d, w2d, b2d = (_as(t, res.dtype) for t in (w1, b1, w2, b2))
-        rb = _b(res_bias, res)
-        L.check(lib.eavsr_ca_scale_forward(rd.data_ptr(), sd.data_ptr(), sums.data_ptr(),
-                                           w1d.data_ptr(), b1d.data_ptr(), w2d.data_ptr(), b2d.data_ptr(),
-                                           _ptr(rb), out.data_ptr(), n, c, h, w, reduction,
-                                           _dtype_code("ca_scale", rd), _stream(rd)), "ca_scale")
-        del w1d, b1d, w2d, b2d, rb
+    rd = res.contiguous(memory_format=torch.channels_last)
+    out = torch.empty_like(rd)
+    _launch("ca_scale_forward", rd, skip.to(res.dtype).contiguous(memory_format=torch.channels_last), sums,
+            *(_param(t, res.dtype) for t in (w1, b1, w2, b2, res_bias)), out, n, c, h, w, reduction,
+            _dtype_code("ca_scale", rd))
     return out
 
 
@@ -1171,17 +1034,11 @@ def conv2d_bias_act_shuffle(conv: nn.Conv2d, x, negative_slope: float = 1.0):
             or not x.is_contiguous(memory_format=torch.channels_last)):
         y = torch.nn.functional.pixel_shuffle(conv(x), 2)
         return y if negative_slope == 1.0 else torch.nn.functional.leaky_relu(y, negative_slope)
-    lib = L.load()
     y = torch.nn.functional.conv2d(x, conv.weight, None, conv.stride, conv.padding, conv.dilation, conv.groups)
     if not y.is_contiguous(memory_format=torch.channels_last):
         y = y.contiguous(memory_format=torch.channels_last)
     n, _, h, w = y.shape
-    with torch.cuda.device(x.device):
-        out = torch.empty((n, cout // 4, 2 * h, 2 * w), dtype=y.dtype, device=y.device,
-                          memory_format=torch.channels_last)
-        bd = _b(conv.bias, y)
-        L.check(lib.eavsr_bias_act_shuffle_forward(y.data_ptr(), _ptr(bd), out.data_ptr(), n, cout // 4,
-                                                   h, w, float(negative_slope), _dtype_code("bias_act_shuffle", y),
-                                                   _stream(y)), "bias_act_shuffle")
-        del bd
+    out = torch.empty((n, cout // 4, 2 * h, 2 * w), dtype=y.dtype, device=y.device, memory_format=torch.channels_last)
+    _launch("bias_act_shuffle_forward", y, _param(conv.bias, y.dtype), out, n, cout // 4, h, w, float(negative_slope),
+            _dtype_code("bias_act_shuffle", y))
     return out

@@ -13,10 +13,13 @@ from eavsr_b200 import _lib as L
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def declared_symbols():
+def header_text():
     text = open(os.path.join(ROOT, "include", "eavsr_b200.h")).read()
-    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
-    return sorted(set(re.findall(r"\b(eavsr_[a-z0-9_]+)\s*\(", text)))
+    return re.sub(r"/\*.*?\*/", "", text, flags=re.S)
+
+
+def declared_symbols():
+    return sorted(set(re.findall(r"\b(eavsr_[a-z0-9_]+)\s*\(", header_text())))
 
 
 def test_library_exports_every_declared_symbol():
@@ -26,6 +29,38 @@ def test_library_exports_every_declared_symbol():
     for n in names:
         assert hasattr(lib, n), n
     assert sorted(L.EXPORTED_SYMBOLS) == names      # the ctypes binding covers the whole header
+
+
+def test_constants_match_the_header_defines():
+    defines = {k: int(v) for k, v in re.findall(r"#define EAVSR_(\w+) (\d+)u?\b", header_text())}
+    consts = {k: v for k, v in vars(L).items() if k.isupper() and type(v) is int}
+    assert len(consts) >= 15
+    for name, value in consts.items():
+        assert defines.get(name) == value, name
+
+
+@pytest.mark.parametrize("cls, c_name", [(L.FlowTerm, "EavsrFlowTerm"), (L.ConvLayer, "EavsrConvLayer")])
+def test_structures_match_the_header_typedefs(cls, c_name):
+    body = re.search(r"typedef struct %s \{(.*?)\} %s;" % (c_name, c_name), header_text(), flags=re.S).group(1)
+    fields = []
+    for decl in body.split(";")[:-1]:
+        first, *more = decl.split(",")            # "int h, w" declares two fields
+        fields += [first.split()[-1].lstrip("*")] + [m.strip() for m in more]
+    assert [f for f, _ in cls._fields_] == fields
+
+
+def test_unreadable_header_fails_loudly(monkeypatch, tmp_path):
+    header = tmp_path / "eavsr_b200.h"
+    monkeypatch.setattr(L, "_HEADER", header)
+    L._signatures.cache_clear()
+    try:
+        with pytest.raises(L.EavsrError, match="not found"):
+            L._signatures()
+        header.write_text("int eavsr_f(const double x[4],\n            void* stream);\n")
+        with pytest.raises(L.EavsrError, match=r"eavsr_f uses `const double\[4\]`"):
+            L._signatures()
+    finally:
+        L._signatures.cache_clear()
 
 
 def test_library_loads_and_reports_version():
