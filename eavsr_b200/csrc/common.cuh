@@ -240,6 +240,13 @@ __device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t* r) {
       : "r"(taddr)
       : "memory");
 }
+// 32 lanes x 4 consecutive columns
+__device__ __forceinline__ void tmem_ld_32x4(uint32_t taddr, uint32_t* r) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(taddr)
+               : "memory");
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory"); }
 
 // K-major, 128-byte-swizzled operand tile: rows of 128 B, 8-row atoms of 1024 B (SBO),

@@ -29,7 +29,7 @@ from .ops import (ModulatedDeformConv2d, adapt_mix, grouped_conv3x3, grouped_con
                   dcn_affine, dcn_affine_eligible,
                   conv3x3_64, conv3x3_64_ca, conv3x3_64_eligible, conv3x3_chain_eligible, rca_group_chain,
                   flow_warp, flow_warp2, flow_warp_nhw2, flow_warp_pyramid, flow_warp_pyramid_eligible, fused_inference_ok,
-                  spynet_level_input,
+                  spynet_level_input, sr_tail_u8, sr_tail_u8_eligible,
                   modulated_deform_conv2d)
 
 __all__ = ["EAVSRP", "MultiAdSTN", "SPyNet"]
@@ -494,23 +494,61 @@ class EAVSRP(nn.Module):
         feats[branch] = outs[::-1] if backward else outs
         return feats
 
+    def _hr_features(self, feats, i):
+        """HR feature map of frame i: reconstruction, the pixel-shuffle stages and conv_hr + LeakyReLU -- everything
+        of the reconstruction up to conv_last."""
+        x = cat_channels([feats["spatial"][i]] + [feats[b][i] for b in _BRANCHES])
+        x = self.reconstruction(x)
+        # LeakyReLU commutes with PixelShuffle: fold it into the conv epilogue
+        x = conv2d_bias_act_shuffle(self.upsample1[0], x, 0.1)
+        if self.scale == 4:
+            x = conv2d_bias_act_shuffle(self.upsample2[0], x, 0.1)
+        return conv3x3_64(self.conv_hr, x, 0.1) if conv3x3_64_eligible(self.conv_hr, x) else \
+            conv2d_bias_act(self.conv_hr, x, 0.1)
+
+    def _sr_frame(self, lrs, x, i):
+        # the image-domain tail is fp32: residual (small) + bilinear base (the [0,1] frame itself)
+        base = F.interpolate(lrs[:, i].float(), scale_factor=self.scale, mode="bilinear", align_corners=False)
+        return self.conv_last(x).float() + base
+
     def _upsample(self, lrs, feats):
-        outs = []
-        for i in range(lrs.shape[1]):
-            x = cat_channels([feats["spatial"][i]] + [feats[b][i] for b in _BRANCHES])
-            x = self.reconstruction(x)
-            # LeakyReLU commutes with PixelShuffle: fold it into the conv epilogue
-            x = conv2d_bias_act_shuffle(self.upsample1[0], x, 0.1)
-            if self.scale == 4:
-                x = conv2d_bias_act_shuffle(self.upsample2[0], x, 0.1)
-            x = conv3x3_64(self.conv_hr, x, 0.1) if conv3x3_64_eligible(self.conv_hr, x) else \
-                conv2d_bias_act(self.conv_hr, x, 0.1)
-            # the image-domain tail is fp32: residual (small) + bilinear base (the [0,1] frame itself)
-            base = F.interpolate(lrs[:, i].float(), scale_factor=self.scale, mode="bilinear", align_corners=False)
-            outs.append(self.conv_last(x).float() + base)
-        return torch.stack(outs, 1)
+        return torch.stack([self._sr_frame(lrs, self._hr_features(feats, i), i) for i in range(lrs.shape[1])], 1)
 
     def forward(self, lrs):
+        return self._upsample(lrs, self._trunk(lrs))
+
+    def forward_uint8(self, frames):
+        """8-bit frames in, 8-bit SR frames out: ``frames`` (n, t, h, w, 3) uint8 RGB on the GPU -> (n, t, s*h, s*w, 3)
+        uint8, the reference's visuals ``clamp(sr * 255, 0, 255).round()`` (models/base_model.py:146-150) of the
+        forward on ``frames / 255``.  The clip is replicate-padded to multiples of 4 (`pad_clip`) and the output
+        cropped back.  With bf16 features, conv_last, the bilinear base and the quantisation run as one kernel per
+        frame that writes straight into the output (`ops.sr_tail_u8`); otherwise they are composed in PyTorch and the
+        result equals the visuals of `forward` bit for bit.  Inference only (runs under ``no_grad``); no host
+        synchronisation, so it can be captured in a CUDA graph like `forward`."""
+        if not isinstance(frames, torch.Tensor) or frames.dtype != torch.uint8:
+            raise TypeError(f"EAVSRP.forward_uint8 takes a uint8 tensor, got {getattr(frames, 'dtype', type(frames))}")
+        if frames.dim() != 5 or frames.shape[-1] != 3:
+            raise ValueError(f"EAVSRP.forward_uint8 takes (n, t, h, w, 3) RGB frames, got {tuple(frames.shape)}")
+        if not frames.is_cuda:
+            raise NotImplementedError("EAVSRP.forward_uint8: CUDA tensors only (the B200 library has no CPU fallback)")
+        n, t, h, w, _ = frames.shape
+        assert h >= 64 and w >= 64, f"The height and width of inputs should be at least 64, but got {h} and {w}."
+        s = self.scale
+        with torch.no_grad():
+            lrs = pad_clip(frames.permute(0, 1, 4, 2, 3).float().div(255).contiguous())
+            feats = self._trunk(lrs)
+            out = torch.empty((n, t, s * h, s * w, 3), dtype=torch.uint8, device=frames.device)
+            for i in range(t):
+                x = self._hr_features(feats, i)
+                if sr_tail_u8_eligible(self.conv_last, x):
+                    sr_tail_u8(self.conv_last, x, lrs[:, i], s, out[:, i], s * h, s * w)
+                else:
+                    sr = self._sr_frame(lrs, x, i)[..., :s * h, :s * w]
+                    out[:, i] = torch.clamp(sr * 255, 0, 255).round().permute(0, 2, 3, 1)
+        return out
+
+    def _trunk(self, lrs):
+        """Flows, encoder and the four propagation branches of a padded clip: the features `_hr_features` reads."""
         n, t, c, h, w = lrs.shape
         assert h >= 64 and w >= 64, f"The height and width of inputs should be at least 64, but got {h} and {w}."
         if h % 4 or w % 4:
@@ -530,7 +568,7 @@ class EAVSRP(nn.Module):
         feats = {"spatial": split(f1), "spatial_d2": split(f2), "spatial_d4": split(f4)}
         for b in _BRANCHES:
             feats = self._propagate(feats, flows_bwd if b.startswith("backward") else flows_fwd, b)
-        return self._upsample(lrs, feats)
+        return feats
 
 
 def pad_clip(lrs, multiple=4):

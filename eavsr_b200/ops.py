@@ -44,7 +44,7 @@ __all__ = [
     "FunctionCorrelation", "ModuleCorrelation", "dcn_uses_tensor_cores",
     "adapt_mix", "affine_offsets_mask", "ca_residual", "fused_inference_ok", "bias_act_", "conv2d_bias_act",
     "conv3x3_64", "conv3x3_64_ca", "conv3x3_64_eligible", "ca_scale", "conv2d_bias_act_shuffle",
-    "conv3x3_chain_eligible", "rca_group_chain",
+    "conv3x3_chain_eligible", "rca_group_chain", "sr_tail_u8", "sr_tail_u8_eligible",
 ]
 
 _DTYPES = {torch.float32: L.F32, torch.bfloat16: L.BF16}
@@ -898,16 +898,18 @@ def conv3x3_64_eligible(conv: nn.Conv2d, x) -> bool:
             and fused_inference_ok(x, conv.weight))
 
 
-def _packed_conv_weight(conv: nn.Conv2d, device) -> torch.Tensor:
-    """Weights re-packed once into the 9 swizzled 64x64 bf16 tiles the MMA reads (cached on the module,
-    invalidated by the parameter's version counter / storage)."""
+def _packed_conv_weight(conv: nn.Conv2d, device, kind: str = "conv3x3") -> torch.Tensor:
+    """Weights re-packed once into the swizzled bf16 tiles the MMA of ``eavsr_<kind>_*`` reads: 9 64x64 tiles for
+    ``conv3x3``, 9 16x64 tiles for ``sr_tail`` (cached on the module, invalidated by the parameter's version
+    counter / storage)."""
     w = conv.weight
-    key = (w.data_ptr(), w._version, str(device))
+    key = (kind, w.data_ptr(), w._version, str(device))
     hit = getattr(conv, "_eavsr_packed", None)
     if hit is not None and hit[0] == key:
         return hit[1]
-    packed = torch.empty(L.load().eavsr_conv3x3_packed_weight_bytes(), dtype=torch.uint8, device=device)
-    _launch("conv3x3_pack_weight", _param(w.to(device), torch.bfloat16), packed, 64, 64, L.BF16)
+    packed = torch.empty(getattr(L.load(), f"eavsr_{kind}_packed_weight_bytes")(), dtype=torch.uint8, device=device)
+    _launch(f"{kind}_pack_weight", _param(w.to(device), torch.bfloat16), packed, conv.in_channels, conv.out_channels,
+            L.BF16)
     conv._eavsr_packed = (key, packed)
     return packed
 
@@ -1041,4 +1043,37 @@ def conv2d_bias_act_shuffle(conv: nn.Conv2d, x, negative_slope: float = 1.0):
     out = torch.empty((n, cout // 4, 2 * h, 2 * w), dtype=y.dtype, device=y.device, memory_format=torch.channels_last)
     _launch("bias_act_shuffle_forward", y, _param(conv.bias, y.dtype), out, n, cout // 4, h, w, float(negative_slope),
             _dtype_code("bias_act_shuffle", y))
+    return out
+
+
+# ------------------------------------------------------------------------------------------
+# reconstruction tail -> uint8 frames on tcgen05 (conv_last + bilinear base + visuals)
+# ------------------------------------------------------------------------------------------
+def sr_tail_u8_eligible(conv_last: nn.Conv2d, x) -> bool:
+    """True when `sr_tail_u8` can run: ``conv_last`` is a 64 -> 3 3x3 stride-1 pad-1 convolution, ``x`` a dense
+    channels_last bf16 CUDA map of 64 channels, and no gradient is needed."""
+    return (isinstance(conv_last, nn.Conv2d) and conv_last.in_channels == 64 and conv_last.out_channels == 3
+            and conv_last.kernel_size == (3, 3) and conv_last.stride == (1, 1) and conv_last.padding == (1, 1)
+            and conv_last.dilation == (1, 1) and conv_last.groups == 1 and conv_last.padding_mode == "zeros"
+            and x.dtype == torch.bfloat16 and x.dim() == 4 and x.shape[1] == 64
+            and x.is_contiguous(memory_format=torch.channels_last) and fused_inference_ok(x, conv_last.weight))
+
+
+def sr_tail_u8(conv_last: nn.Conv2d, x, lr, scale: int, out, out_h: int, out_w: int):
+    """``out[n, y, x, :] = round(clamp(255 * (conv_last(x) + interpolate(lr, scale, bilinear)), 0, 255))`` for
+    ``y < out_h``, ``x < out_w`` in one kernel (models/eavsrp_model.py:350-364 and the visuals of
+    models/base_model.py:146-150).  ``x``: (n, 64, H, W) bf16 channels_last; ``lr``: (n, 3, H/scale, W/scale) fp32,
+    any strides; ``out``: (n, out_h, out_w, 3) uint8, any strides (e.g. ``clip[:, i]`` of an (n, t, Ho, Wo, 3)
+    tensor).  The residual is accumulated and added in fp32, never rounded to bf16.  Check `sr_tail_u8_eligible`
+    first.  Returns ``out``."""
+    _require_cuda("sr_tail_u8", x, lr, out)
+    n, c, h, w = x.shape
+    if lr.dtype != torch.float32 or tuple(lr.shape) != (n, 3, h // scale, w // scale):
+        raise ValueError(f"eavsr_b200.sr_tail_u8: lr must be fp32 (n, 3, H/s, W/s), got {lr.dtype} {tuple(lr.shape)}")
+    if out.dtype != torch.uint8 or tuple(out.shape) != (n, out_h, out_w, 3):
+        raise ValueError(f"eavsr_b200.sr_tail_u8: out must be uint8 (n, out_h, out_w, 3), got {out.dtype} "
+                         f"{tuple(out.shape)}")
+    _launch("sr_tail_u8_forward", x, _strides(x), _packed_conv_weight(conv_last, x.device, "sr_tail"),
+            _param(conv_last.bias, torch.bfloat16), lr, L.Strides(*lr.stride()), out, L.Strides(*out.stride()),
+            n, c, h, w, int(scale), int(out_h), int(out_w), L.BF16)
     return out

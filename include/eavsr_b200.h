@@ -1,5 +1,6 @@
 /*
- * eavsr_b200 -- C ABI of the B200-native (sm_100a) inter-frame alignment kernels for EAVSR.
+ * eavsr_b200 -- C ABI of the B200-native (sm_100a) inter-frame alignment kernels for EAVSR, and of the
+ * reconstruction tail that turns the network's HR features into 8-bit RGB frames.
  *
  * The reference (HITRainer/EAVSR) has no C ABI: its hot path is reached through Python
  * symbols.  Each entry point below replaces the native code that sits under one of those
@@ -336,6 +337,31 @@ typedef struct EavsrConvLayer {
 } EavsrConvLayer;
 int eavsr_conv3x3_chain_forward(const EavsrConvLayer* layers, int nlayers, int n, int h, int w, int dtype,
                                 void* sync_workspace, void* stream);
+
+/* ---- reconstruction tail to 8-bit frames on tcgen05 (EAVSRP.upsample, models/eavsrp_model.py:350-364, followed by
+ * the visuals of models/base_model.py:146-150) ------------------------------------------------------------------
+ * For y < out_h, x < out_w and c < 3:
+ *   out[n, y, x, c] = rint(clamp(255 * (bias[c] + sum_{ci, ky, kx} W[c, ci, ky, kx] * x[n, ci, y+ky-1, x+kx-1]
+ *                                        + up_s(lr)[n, c, y, x]), 0, 255))
+ * i.e. conv_last(x) + F.interpolate(lr, scale_factor=s, mode='bilinear', align_corners=False), then
+ * torch.clamp(sr * 255, 0, 255).round() as uint8.
+ *   x:    (n, 64, h, w) bf16, dense channels_last (x_strides = {h*w*64, 1, w*64, 64}), 16-byte aligned; zero
+ *         padding at the borders as nn.Conv2d(64, 3, 3, 1, 1).  Rows and columns beyond the crop are still read.
+ *   W, bias: conv_last's (3, 64, 3, 3) weight, packed once with eavsr_sr_tail_pack_weight into
+ *         eavsr_sr_tail_packed_weight_bytes() bytes (16-byte aligned), and its (3) bf16 bias or NULL.
+ *   lr:   (n, 3, h/s, w/s) fp32 by element strides lr_strides (n, c, h, w) -- e.g. one frame of a padded clip.
+ *         up_s is ATen's upsample_bilinear2d: source max((dst + 0.5) / s - 0.5, 0), upper neighbour clamped.
+ *   out:  uint8 by element strides out_strides in (n, y, x, c) order -- e.g. frame i of an (n, t, Ho, Wo, 3) clip.
+ * Products are bf16 x bf16 with fp32 accumulation; the sum, bias and bilinear base are added in fp32 (the residual
+ * is never rounded to bf16), and rint rounds half to even as torch.round does.  scale = s is 2 or 4; h and w are
+ * multiples of s; 0 < out_h <= h, 0 < out_w <= w (the crop of a replicate-padded clip).  Anything else returns
+ * EAVSR_ERR_INVALID; dtype other than EAVSR_BF16 returns EAVSR_ERR_UNSUPPORTED. */
+size_t eavsr_sr_tail_packed_weight_bytes(void);
+int eavsr_sr_tail_pack_weight(const void* weight /* (3,64,3,3) */, void* packed, int cin, int cout, int dtype,
+                              void* stream);
+int eavsr_sr_tail_u8_forward(const void* x, const int64_t x_strides[4], const void* packed_weight, const void* bias,
+                             const float* lr, const int64_t lr_strides[4], void* out, const int64_t out_strides[4],
+                             int n, int c, int h, int w, int scale, int out_h, int out_w, int dtype, void* stream);
 
 #ifdef __cplusplus
 }
