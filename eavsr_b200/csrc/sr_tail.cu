@@ -24,6 +24,8 @@
 //              shifted sum, + bias, quantise, 3 byte stores per pixel
 #include <cuda.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace eavsr {
@@ -52,6 +54,21 @@ struct StSmem {
   static constexpr int DYN = TOTAL + 1024;
 };
 
+// The epilogue's store, a template parameter of the kernel: interleaved RGB, or Y'CbCr 4:2:0 planes.
+struct RgbOut {
+  uint8_t* p;
+  long long s_n, s_y, s_x, s_c;
+};
+struct PlaneOut {
+  uint8_t* p;
+  long long s_n, s_y, s_x;
+};
+struct Yuv420Out {
+  PlaneOut y, u, v;                // u, v: (out_h / 2, out_w / 2)
+  float kr, kg, kb, cu, cv;        // fp32 coefficients of eavsr_b200/yuv.py: cu = 112 / (1 - kb), cv = 112 / (1 - kr)
+};
+
+template <class Out>
 struct TailParams {
   // (64 ch, W, H, N) bf16 view of X, box (64, 32, 6, 1), 128-byte swizzle, out-of-image pixels zero-filled
   alignas(64) CUtensorMap tm;
@@ -59,11 +76,16 @@ struct TailParams {
   const __nv_bfloat16* bias;       // (3) or null
   const float* lr;
   long long ls_n, ls_c, ls_h, ls_w;
-  uint8_t* out;
-  long long os_n, os_y, os_x, os_c;
+  Out out;
   int out_h, out_w, lr_h, lr_w, tiles_x, tiles_per_img, total_tiles;
   float inv_scale;
 };
+
+// 4:2:0: the odd-row warp of each (q, q + 1) pair hands its horizontal pair sums to the even-row warp through a
+// double-buffered slot of 2 x 3 x 16 floats; one named barrier per pair (ids 1-4)
+constexpr int ST_XCH = 4 * 2 * 3 * 16 * 4;
+template <class Out>
+constexpr int st_dyn() { return StSmem::DYN + (std::is_same<Out, Yuv420Out>::value ? ST_XCH : 0); }
 
 // packed[tap][o][ci] (o < 16, K-major SW128) = W[o, ci, tap] for o < 3, 0 otherwise
 __global__ void sr_tail_pack_weight_kernel(const __nv_bfloat16* __restrict__ w, uint8_t* __restrict__ packed) {
@@ -74,7 +96,9 @@ __global__ void sr_tail_pack_weight_kernel(const __nv_bfloat16* __restrict__ w, 
       o < 3 ? w[((size_t)o * ST_CH + ci) * 9 + t] : __float2bfloat16_rn(0.f);
 }
 
-__global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_constant__ TailParams P) {
+template <class Out>
+__global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_constant__ TailParams<Out> P) {
+  constexpr bool YUV = std::is_same<Out, Yuv420Out>::value;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
@@ -205,14 +229,55 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_acce + 8 * team);          // accumulator drained: tile tl + 2 may start
-      uint8_t* op = P.out + n * P.os_n + (long long)y * P.os_y + (long long)x * P.os_x;
+      if constexpr (!YUV) {
+        uint8_t* op = P.out.p + n * P.out.s_n + (long long)y * P.out.s_y + (long long)x * P.out.s_x;
 #pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        const float t = __uint_as_float(a0[c]) + __shfl_down_sync(0xffffffffu, __uint_as_float(a1[c]), 1) +
-                        __shfl_down_sync(0xffffffffu, __uint_as_float(a2[c]), 2);
-        // the reference's visuals: clamp(sr * 255, 0, 255).round(), round half to even
-        const float v = fminf(fmaxf(255.f * ((t + bias[c]) + up[c]), 0.f), 255.f);
-        if (valid) op[c * P.os_c] = (uint8_t)__float2int_rn(v);
+        for (int c = 0; c < 3; ++c) {
+          const float t = __uint_as_float(a0[c]) + __shfl_down_sync(0xffffffffu, __uint_as_float(a1[c]), 1) +
+                          __shfl_down_sync(0xffffffffu, __uint_as_float(a2[c]), 2);
+          // the reference's visuals: clamp(sr * 255, 0, 255).round(), round half to even
+          const float v = fminf(fmaxf(255.f * ((t + bias[c]) + up[c]), 0.f), 255.f);
+          if (valid) op[c * P.out.s_c] = (uint8_t)__float2int_rn(v);
+        }
+      } else {
+        // rgb_to_yuv420 of eavsr_b200/yuv.py in its fp32 order of operations (no contraction into FMAs)
+        const Yuv420Out& o = P.out;
+        float v[3], s[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const float t = __uint_as_float(a0[c]) + __shfl_down_sync(0xffffffffu, __uint_as_float(a1[c]), 1) +
+                          __shfl_down_sync(0xffffffffu, __uint_as_float(a2[c]), 2);
+          v[c] = fminf(fmaxf((t + bias[c]) + up[c], 0.f), 1.f);
+          s[c] = __fadd_rn(v[c], __shfl_xor_sync(0xffffffffu, v[c], 1));      // p(x) + p(x + 1), x even
+        }
+        const float yc = __fadd_rn(__fadd_rn(__fmul_rn(o.kr, v[0]), __fmul_rn(o.kg, v[1])), __fmul_rn(o.kb, v[2]));
+        if (valid)
+          o.y.p[n * o.y.s_n + (long long)y * o.y.s_y + (long long)x * o.y.s_x] =
+              (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(219.f, yc), 16.f));
+        // tile origins are even and out_h, out_w are even: a 2x2 block is lanes (2k, 2k + 1) of warps q, q + 1 of
+        // one team, and it is valid as a whole.  The slot is double-buffered over the team's tiles, so the write
+        // for its next tile lands in the other buffer, and the one after that waits at the barrier for this read
+        float* xch = reinterpret_cast<float*>(smem + StSmem::TOTAL) + ((team * 2 + (q >> 1)) * 2 + ((tl >> 1) & 1)) * 48;
+        const int bar_id = 1 + team * 2 + (q >> 1);
+        if (q & 1) {
+          if (!(lane & 1))
+#pragma unroll
+            for (int c = 0; c < 3; ++c) xch[c * 16 + (lane >> 1)] = s[c];
+          asm volatile("bar.sync %0, 64;\n" ::"r"(bar_id) : "memory");
+        } else {
+          asm volatile("bar.sync %0, 64;\n" ::"r"(bar_id) : "memory");
+          if (valid && !(lane & 1)) {
+            float m[3];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) m[c] = __fmul_rn(__fadd_rn(s[c], xch[c * 16 + (lane >> 1)]), 0.25f);
+            const float ym = __fadd_rn(__fadd_rn(__fmul_rn(o.kr, m[0]), __fmul_rn(o.kg, m[1])), __fmul_rn(o.kb, m[2]));
+            const long long yh = y >> 1, xh = x >> 1;
+            o.u.p[n * o.u.s_n + yh * o.u.s_y + xh * o.u.s_x] =
+                (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[2], ym), o.cu), 128.f));
+            o.v.p[n * o.v.s_n + yh * o.v.s_y + xh * o.v.s_x] =
+                (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[0], ym), o.cv), 128.f));
+          }
+        }
       }
     }
   }
@@ -220,6 +285,55 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
   tc_fence_before();
   __syncthreads();
   if (warp == 1) tmem_dealloc<ST_TMEM>(tmem_d);
+}
+
+// checks, tensor map and launch shared by the RGB and the 4:2:0 entry points
+template <class Out>
+int sr_tail_launch(const char* who, const void* x, const int64_t x_strides[4], const void* packed_weight,
+                   const void* bias, const float* lr, const int64_t lr_strides[4], const Out& out, int n, int c, int h,
+                   int w, int scale, int out_h, int out_w, int dtype, void* stream) {
+  EAVSR_REQUIRE(c == ST_CH, "%s: the feature map must have 64 channels (got %d)", who, c);
+  EAVSR_REQUIRE(scale == 2 || scale == 4, "%s: scale must be 2 or 4 (got %d)", who, scale);
+  EAVSR_REQUIRE(n > 0 && h > 0 && w > 0 && h % scale == 0 && w % scale == 0,
+                "%s: bad map %dx%dx%d for scale %d", who, n, h, w, scale);
+  EAVSR_REQUIRE(out_h > 0 && out_w > 0 && out_h <= h && out_w <= w,
+                "%s: crop %dx%d outside the %dx%d map", who, out_h, out_w, h, w);
+  EAVSR_REQUIRE(x_strides[0] == (int64_t)h * w * ST_CH && x_strides[1] == 1 && x_strides[2] == (int64_t)w * ST_CH &&
+                    x_strides[3] == ST_CH,
+                "%s: x must be dense channels_last (NHWC)", who);
+  EAVSR_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(packed_weight)) & 15u) == 0,
+                "%s: x and the packed weights must be 16-byte aligned", who);
+  if (dtype != EAVSR_BF16) {
+    set_error("%s: only bf16 features are implemented (dtype %d)", who, dtype);
+    return EAVSR_ERR_UNSUPPORTED;
+  }
+  const int tiles_x = ceil_div(out_w, ST_TC), tiles_y = ceil_div(out_h, ST_TR);
+  const long long total = (long long)tiles_x * tiles_y * n;
+  EAVSR_REQUIRE(total < (1ll << 31), "%s: too many tiles", who);
+  static thread_local TailParams<Out> P;
+  const unsigned long long dims[4] = {ST_CH, (unsigned long long)w, (unsigned long long)h, (unsigned long long)n};
+  const unsigned long long str[3] = {ST_CH * 2ull, (unsigned long long)w * ST_CH * 2,
+                                     (unsigned long long)h * w * ST_CH * 2};
+  const unsigned box[4] = {ST_CH, ST_PW, ST_TR + 2, 1};
+  if (!encode_tensor_map(&P.tm, EAVSR_BF16, 4, x, dims, str, box, 3 /* CU_TENSOR_MAP_SWIZZLE_128B */)) {
+    set_error("%s: the tensor map of x was rejected", who);
+    return EAVSR_ERR_UNSUPPORTED;
+  }
+  P.wpacked = (const uint8_t*)packed_weight;
+  P.bias = (const __nv_bfloat16*)bias;
+  P.lr = lr;
+  P.ls_n = lr_strides[0]; P.ls_c = lr_strides[1]; P.ls_h = lr_strides[2]; P.ls_w = lr_strides[3];
+  P.out = out;
+  P.out_h = out_h; P.out_w = out_w; P.lr_h = h / scale; P.lr_w = w / scale;
+  P.tiles_x = tiles_x; P.tiles_per_img = tiles_x * tiles_y; P.total_tiles = (int)total;
+  P.inv_scale = 1.f / (float)scale;
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  cudaError_t e = cudaFuncSetAttribute(sr_tail_u8_kernel<Out>, cudaFuncAttributeMaxDynamicSharedMemorySize, st_dyn<Out>());
+  if (e != cudaSuccess) { set_error("%s: smem attr: %s", who, cudaGetErrorString(e)); return EAVSR_ERR_CUDA; }
+  sr_tail_u8_kernel<Out><<<(int)(total < sms ? total : sms), ST_THREADS, st_dyn<Out>(), (cudaStream_t)stream>>>(P);
+  return check_launch(who);
 }
 
 }  // namespace
@@ -247,47 +361,30 @@ extern "C" int eavsr_sr_tail_u8_forward(const void* x, const int64_t x_strides[4
                                         int out_w, int dtype, void* stream) {
   EAVSR_REQUIRE(x && x_strides && packed_weight && lr && lr_strides && out && out_strides,
                 "sr_tail_u8_forward: null pointer");
-  EAVSR_REQUIRE(c == ST_CH, "sr_tail_u8_forward: the feature map must have 64 channels (got %d)", c);
-  EAVSR_REQUIRE(scale == 2 || scale == 4, "sr_tail_u8_forward: scale must be 2 or 4 (got %d)", scale);
-  EAVSR_REQUIRE(n > 0 && h > 0 && w > 0 && h % scale == 0 && w % scale == 0,
-                "sr_tail_u8_forward: bad map %dx%dx%d for scale %d", n, h, w, scale);
-  EAVSR_REQUIRE(out_h > 0 && out_w > 0 && out_h <= h && out_w <= w,
-                "sr_tail_u8_forward: crop %dx%d outside the %dx%d map", out_h, out_w, h, w);
-  EAVSR_REQUIRE(x_strides[0] == (int64_t)h * w * ST_CH && x_strides[1] == 1 && x_strides[2] == (int64_t)w * ST_CH &&
-                    x_strides[3] == ST_CH,
-                "sr_tail_u8_forward: x must be dense channels_last (NHWC)");
-  EAVSR_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(packed_weight)) & 15u) == 0,
-                "sr_tail_u8_forward: x and the packed weights must be 16-byte aligned");
-  if (dtype != EAVSR_BF16) {
-    set_error("sr_tail_u8_forward: only bf16 features are implemented (dtype %d)", dtype);
-    return EAVSR_ERR_UNSUPPORTED;
-  }
-  const int tiles_x = ceil_div(out_w, ST_TC), tiles_y = ceil_div(out_h, ST_TR);
-  const long long total = (long long)tiles_x * tiles_y * n;
-  EAVSR_REQUIRE(total < (1ll << 31), "sr_tail_u8_forward: too many tiles");
-  static thread_local TailParams P;
-  const unsigned long long dims[4] = {ST_CH, (unsigned long long)w, (unsigned long long)h, (unsigned long long)n};
-  const unsigned long long str[3] = {ST_CH * 2ull, (unsigned long long)w * ST_CH * 2,
-                                     (unsigned long long)h * w * ST_CH * 2};
-  const unsigned box[4] = {ST_CH, ST_PW, ST_TR + 2, 1};
-  if (!encode_tensor_map(&P.tm, EAVSR_BF16, 4, x, dims, str, box, 3 /* CU_TENSOR_MAP_SWIZZLE_128B */)) {
-    set_error("sr_tail_u8_forward: the tensor map of x was rejected");
-    return EAVSR_ERR_UNSUPPORTED;
-  }
-  P.wpacked = (const uint8_t*)packed_weight;
-  P.bias = (const __nv_bfloat16*)bias;
-  P.lr = lr;
-  P.ls_n = lr_strides[0]; P.ls_c = lr_strides[1]; P.ls_h = lr_strides[2]; P.ls_w = lr_strides[3];
-  P.out = (uint8_t*)out;
-  P.os_n = out_strides[0]; P.os_y = out_strides[1]; P.os_x = out_strides[2]; P.os_c = out_strides[3];
-  P.out_h = out_h; P.out_w = out_w; P.lr_h = h / scale; P.lr_w = w / scale;
-  P.tiles_x = tiles_x; P.tiles_per_img = tiles_x * tiles_y; P.total_tiles = (int)total;
-  P.inv_scale = 1.f / (float)scale;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  cudaError_t e = cudaFuncSetAttribute(sr_tail_u8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, StSmem::DYN);
-  if (e != cudaSuccess) { set_error("sr_tail_u8_forward: smem attr: %s", cudaGetErrorString(e)); return EAVSR_ERR_CUDA; }
-  sr_tail_u8_kernel<<<(int)(total < sms ? total : sms), ST_THREADS, StSmem::DYN, (cudaStream_t)stream>>>(P);
-  return check_launch("sr_tail_u8_forward");
+  const RgbOut o = {(uint8_t*)out, out_strides[0], out_strides[1], out_strides[2], out_strides[3]};
+  return sr_tail_launch("sr_tail_u8_forward", x, x_strides, packed_weight, bias, lr, lr_strides, o, n, c, h, w, scale,
+                        out_h, out_w, dtype, stream);
+}
+
+extern "C" int eavsr_sr_tail_yuv420_forward(const void* x, const int64_t x_strides[4], const void* packed_weight,
+                                            const void* bias, const float* lr, const int64_t lr_strides[4],
+                                            void* out_y, const int64_t y_strides[4], void* out_u,
+                                            const int64_t u_strides[4], void* out_v, const int64_t v_strides[4], int n,
+                                            int c, int h, int w, int scale, int out_h, int out_w, float kr, float kb,
+                                            int dtype, void* stream) {
+  EAVSR_REQUIRE(x && x_strides && packed_weight && lr && lr_strides && out_y && y_strides && out_u && u_strides &&
+                    out_v && v_strides,
+                "sr_tail_yuv420_forward: null pointer");
+  EAVSR_REQUIRE(out_h % 2 == 0 && out_w % 2 == 0, "sr_tail_yuv420_forward: 4:2:0 needs an even crop (got %dx%d)",
+                out_h, out_w);
+  EAVSR_REQUIRE(kr > 0.f && kb > 0.f && kr + kb < 1.f, "sr_tail_yuv420_forward: bad matrix (kr %g, kb %g)", kr, kb);
+  Yuv420Out o;
+  o.y = {(uint8_t*)out_y, y_strides[0], y_strides[2], y_strides[3]};
+  o.u = {(uint8_t*)out_u, u_strides[0], u_strides[2], u_strides[3]};
+  o.v = {(uint8_t*)out_v, v_strides[0], v_strides[2], v_strides[3]};
+  // the fp32 coefficients of eavsr_b200/yuv.py, in its order
+  o.kr = kr; o.kb = kb; o.kg = (1.f - kr) - kb;
+  o.cu = 112.f / (1.f - kb); o.cv = 112.f / (1.f - kr);
+  return sr_tail_launch("sr_tail_yuv420_forward", x, x_strides, packed_weight, bias, lr, lr_strides, o, n, c, h, w,
+                        scale, out_h, out_w, dtype, stream);
 }

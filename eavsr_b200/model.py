@@ -29,8 +29,9 @@ from .ops import (ModulatedDeformConv2d, adapt_mix, grouped_conv3x3, grouped_con
                   dcn_affine, dcn_affine_eligible,
                   conv3x3_64, conv3x3_64_ca, conv3x3_64_eligible, conv3x3_chain_eligible, rca_group_chain,
                   flow_warp, flow_warp2, flow_warp_nhw2, flow_warp_pyramid, flow_warp_pyramid_eligible, fused_inference_ok,
-                  spynet_level_input, sr_tail_u8, sr_tail_u8_eligible,
+                  spynet_level_input, sr_tail_u8, sr_tail_u8_eligible, sr_tail_yuv420,
                   modulated_deform_conv2d)
+from .yuv import MATRICES, rgb_to_yuv420, yuv420_to_rgb
 
 __all__ = ["EAVSRP", "MultiAdSTN", "SPyNet"]
 
@@ -535,17 +536,82 @@ class EAVSRP(nn.Module):
         assert h >= 64 and w >= 64, f"The height and width of inputs should be at least 64, but got {h} and {w}."
         s = self.scale
         with torch.no_grad():
-            lrs = pad_clip(frames.permute(0, 1, 4, 2, 3).float().div(255).contiguous())
-            feats = self._trunk(lrs)
+            lrs = frames.permute(0, 1, 4, 2, 3).float().div(255).contiguous()
             out = torch.empty((n, t, s * h, s * w, 3), dtype=torch.uint8, device=frames.device)
-            for i in range(t):
-                x = self._hr_features(feats, i)
-                if sr_tail_u8_eligible(self.conv_last, x):
-                    sr_tail_u8(self.conv_last, x, lrs[:, i], s, out[:, i], s * h, s * w)
-                else:
-                    sr = self._sr_frame(lrs, x, i)[..., :s * h, :s * w]
-                    out[:, i] = torch.clamp(sr * 255, 0, 255).round().permute(0, 2, 3, 1)
+
+            def fused(i, x, lr):
+                sr_tail_u8(self.conv_last, x, lr, s, out[:, i], s * h, s * w)
+
+            def composed(i, sr):
+                out[:, i] = torch.clamp(sr * 255, 0, 255).round().permute(0, 2, 3, 1)
+            self._sr_frames(lrs, fused, composed)
         return out
+
+    def forward_yuv420(self, y, u, v, matrix="bt709", out=None):
+        """8-bit limited-range Y'CbCr 4:2:0 frames in and out, as video decoders and encoders exchange them.
+
+        ``y`` (n, t, h, w) and ``u``, ``v`` (n, t, h/2, w/2) are uint8 planes on the GPU with any strides (I420
+        planes, or the NV12 views ``uv[..., 0::2]``, ``uv[..., 1::2]``); h and w are even and at least 64.  Returns
+        ``(Y, U, V)``: (n, t, s*h, s*w) and (n, t, s*h/2, s*w/2) uint8, or writes into ``out = (Y, U, V)``, caller
+        planes of those shapes with any strides (NV12 output).  ``matrix`` is "bt709" or "bt601" (`yuv.MATRICES`).
+
+        The result is ``rgb_to_yuv420(crop(forward(pad_clip(yuv420_to_rgb(y, u, v)))))`` (`eavsr_b200.yuv`,
+        centre-sited chroma).  With bf16 features conv_last, the bilinear base and the conversion run as one kernel
+        per frame that writes the three planes (`ops.sr_tail_yuv420`), keeping the residual in fp32; otherwise they
+        are composed in PyTorch.  Inference only (``no_grad``); no host synchronisation, so it can be captured in a
+        CUDA graph."""
+        planes = (y, u, v) + (tuple(out) if out is not None else ())
+        for p in planes:
+            if not isinstance(p, torch.Tensor) or p.dtype != torch.uint8:
+                raise TypeError(f"EAVSRP.forward_yuv420 takes uint8 planes, got {getattr(p, 'dtype', type(p))}")
+        if matrix not in MATRICES:
+            raise ValueError(f"EAVSRP.forward_yuv420: matrix must be one of {sorted(MATRICES)}, got {matrix!r}")
+        if y.dim() != 4:
+            raise ValueError(f"EAVSRP.forward_yuv420 takes an (n, t, h, w) Y plane, got {tuple(y.shape)}")
+        n, t, h, w = y.shape
+        if h % 2 or w % 2 or h < 64 or w < 64:
+            raise ValueError(f"EAVSRP.forward_yuv420 needs an even height and width of at least 64, got {h}x{w}")
+        s = self.scale
+        shapes = [(n, t, h, w), (n, t, h // 2, w // 2), (n, t, h // 2, w // 2)]
+        if out is not None:
+            if len(out) != 3:
+                raise ValueError(f"EAVSRP.forward_yuv420: out must be three planes (Y, U, V), got {len(out)}")
+            shapes += [(n, t, s * h, s * w), (n, t, s * h // 2, s * w // 2), (n, t, s * h // 2, s * w // 2)]
+        for name, p, shape in zip(("y", "u", "v", "out Y", "out U", "out V"), planes, shapes):
+            if tuple(p.shape) != shape:
+                raise ValueError(f"EAVSRP.forward_yuv420: {name} must be {shape}, got {tuple(p.shape)}")
+        if not all(p.is_cuda for p in planes):
+            raise NotImplementedError("EAVSRP.forward_yuv420: CUDA tensors only (the B200 library has no CPU fallback)")
+        kr, kb = MATRICES[matrix]
+        with torch.no_grad():
+            if out is None:
+                out = (torch.empty((n, t, s * h, s * w), dtype=torch.uint8, device=y.device),) + tuple(
+                    torch.empty((n, t, s * h // 2, s * w // 2), dtype=torch.uint8, device=y.device) for _ in range(2))
+            Y, U, V = out
+
+            def fused(i, x, lr):
+                sr_tail_yuv420(self.conv_last, x, lr, s, Y[:, i], U[:, i], V[:, i], s * h, s * w, kr, kb)
+
+            def composed(i, sr):
+                Y[:, i], U[:, i], V[:, i] = rgb_to_yuv420(sr, kr, kb)
+            self._sr_frames(yuv420_to_rgb(y, u, v, kr, kb), fused, composed)
+        return tuple(out)
+
+    def _sr_frames(self, lrs, fused, composed):
+        """The 8-bit forwards' common part, under ``no_grad``: pad the (n, t, 3, h, w) clip `lrs` (`pad_clip`), run
+        `_trunk`, then per frame i `_hr_features` and the tail -- ``fused(i, x, lr_i)`` when the fused tail kernel can
+        run on the HR features ``x`` (`ops.sr_tail_u8_eligible`), else ``composed(i, sr_i)`` with the SR frame of
+        `_sr_frame` cropped to (s*h, s*w)."""
+        h, w = lrs.shape[-2:]
+        s = self.scale
+        lrs = pad_clip(lrs)
+        feats = self._trunk(lrs)
+        for i in range(lrs.shape[1]):
+            x = self._hr_features(feats, i)
+            if sr_tail_u8_eligible(self.conv_last, x):
+                fused(i, x, lrs[:, i])
+            else:
+                composed(i, self._sr_frame(lrs, x, i)[..., :s * h, :s * w])
 
     def _trunk(self, lrs):
         """Flows, encoder and the four propagation branches of a padded clip: the features `_hr_features` reads."""

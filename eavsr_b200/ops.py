@@ -44,7 +44,7 @@ __all__ = [
     "FunctionCorrelation", "ModuleCorrelation", "dcn_uses_tensor_cores",
     "adapt_mix", "affine_offsets_mask", "ca_residual", "fused_inference_ok", "bias_act_", "conv2d_bias_act",
     "conv3x3_64", "conv3x3_64_ca", "conv3x3_64_eligible", "ca_scale", "conv2d_bias_act_shuffle",
-    "conv3x3_chain_eligible", "rca_group_chain", "sr_tail_u8", "sr_tail_u8_eligible",
+    "conv3x3_chain_eligible", "rca_group_chain", "sr_tail_u8", "sr_tail_u8_eligible", "sr_tail_yuv420",
 ]
 
 _DTYPES = {torch.float32: L.F32, torch.bfloat16: L.BF16}
@@ -1059,6 +1059,12 @@ def sr_tail_u8_eligible(conv_last: nn.Conv2d, x) -> bool:
             and x.is_contiguous(memory_format=torch.channels_last) and fused_inference_ok(x, conv_last.weight))
 
 
+def _check_tail_lr(name: str, x, lr, scale: int) -> None:
+    n, c, h, w = x.shape
+    if lr.dtype != torch.float32 or tuple(lr.shape) != (n, 3, h // scale, w // scale):
+        raise ValueError(f"eavsr_b200.{name}: lr must be fp32 (n, 3, H/s, W/s), got {lr.dtype} {tuple(lr.shape)}")
+
+
 def sr_tail_u8(conv_last: nn.Conv2d, x, lr, scale: int, out, out_h: int, out_w: int):
     """``out[n, y, x, :] = round(clamp(255 * (conv_last(x) + interpolate(lr, scale, bilinear)), 0, 255))`` for
     ``y < out_h``, ``x < out_w`` in one kernel (models/eavsrp_model.py:350-364 and the visuals of
@@ -1068,8 +1074,7 @@ def sr_tail_u8(conv_last: nn.Conv2d, x, lr, scale: int, out, out_h: int, out_w: 
     first.  Returns ``out``."""
     _require_cuda("sr_tail_u8", x, lr, out)
     n, c, h, w = x.shape
-    if lr.dtype != torch.float32 or tuple(lr.shape) != (n, 3, h // scale, w // scale):
-        raise ValueError(f"eavsr_b200.sr_tail_u8: lr must be fp32 (n, 3, H/s, W/s), got {lr.dtype} {tuple(lr.shape)}")
+    _check_tail_lr("sr_tail_u8", x, lr, scale)
     if out.dtype != torch.uint8 or tuple(out.shape) != (n, out_h, out_w, 3):
         raise ValueError(f"eavsr_b200.sr_tail_u8: out must be uint8 (n, out_h, out_w, 3), got {out.dtype} "
                          f"{tuple(out.shape)}")
@@ -1077,3 +1082,26 @@ def sr_tail_u8(conv_last: nn.Conv2d, x, lr, scale: int, out, out_h: int, out_w: 
             _param(conv_last.bias, torch.bfloat16), lr, L.Strides(*lr.stride()), out, L.Strides(*out.stride()),
             n, c, h, w, int(scale), int(out_h), int(out_w), L.BF16)
     return out
+
+
+def sr_tail_yuv420(conv_last: nn.Conv2d, x, lr, scale: int, y_out, u_out, v_out, out_h: int, out_w: int, kr: float,
+                   kb: float):
+    """The tail of `sr_tail_u8` written as 8-bit limited-range Y'CbCr 4:2:0 planes: ``rgb_to_yuv420(conv_last(x) +
+    interpolate(lr, scale, bilinear), kr, kb)`` (`eavsr_b200.yuv`) cropped to ``out_h`` x ``out_w``, in one kernel.
+    ``y_out``: (n, out_h, out_w) uint8; ``u_out``, ``v_out``: (n, out_h/2, out_w/2) uint8; any strides, so I420
+    planes or the interleaved chroma of NV12 (``uv[..., 0::2]``, ``uv[..., 1::2]``) are written in place.  ``x`` and
+    ``lr`` as for `sr_tail_u8`, with the same eligibility (`sr_tail_u8_eligible`).  Returns ``(y_out, u_out, v_out)``."""
+    if out_h % 2 or out_w % 2:
+        raise ValueError(f"eavsr_b200.sr_tail_yuv420: 4:2:0 needs an even crop, got {out_h}x{out_w}")
+    n = x.shape[0]
+    _check_tail_lr("sr_tail_yuv420", x, lr, scale)
+    for name, p, shape in (("y_out", y_out, (n, out_h, out_w)), ("u_out", u_out, (n, out_h // 2, out_w // 2)),
+                           ("v_out", v_out, (n, out_h // 2, out_w // 2))):
+        if p.dtype != torch.uint8 or tuple(p.shape) != shape:
+            raise ValueError(f"eavsr_b200.sr_tail_yuv420: {name} must be uint8 {shape}, got {p.dtype} {tuple(p.shape)}")
+    _require_cuda("sr_tail_yuv420", x, lr, y_out, u_out, v_out)
+    planes = [a for p in (y_out, u_out, v_out) for a in (p, L.Strides(*p.unsqueeze(1).stride()))]
+    _launch("sr_tail_yuv420_forward", x, _strides(x), _packed_conv_weight(conv_last, x.device, "sr_tail"),
+            _param(conv_last.bias, torch.bfloat16), lr, L.Strides(*lr.stride()), *planes,
+            n, x.shape[1], x.shape[2], x.shape[3], int(scale), int(out_h), int(out_w), float(kr), float(kb), L.BF16)
+    return y_out, u_out, v_out

@@ -363,6 +363,25 @@ int eavsr_sr_tail_u8_forward(const void* x, const int64_t x_strides[4], const vo
                              const float* lr, const int64_t lr_strides[4], void* out, const int64_t out_strides[4],
                              int n, int c, int h, int w, int scale, int out_h, int out_w, int dtype, void* stream);
 
+/* ---- the same tail to 8-bit limited-range Y'CbCr 4:2:0 planes ---------------------------------------------------
+ * With v = clamp(bias + conv_last(x) + up_s(lr), 0, 1) per pixel (the residual in fp32, as above), writes
+ *   Y[n, y, x]           = rint(16 + 219 * Yc(v[n, :, y, x]))                           for y < out_h, x < out_w
+ *   U[n, y/2, x/2]       = rint(128 + 112 / (1 - kb) * (m_b - Yc(m))),  V likewise with m_r and kr,
+ * where Yc(p) = kr p_r + kg p_g + kb p_b, kg = 1 - kr - kb, and m is the mean of v over the 2x2 block of even y, x
+ * (centre-sited chroma).  The fp32 order of operations is that of rgb_to_yuv420 in eavsr_b200/yuv.py.  kr, kb are
+ * the matrix (BT.709: 0.2126, 0.0722; BT.601: 0.299, 0.114).
+ *   x, W, bias, lr: as eavsr_sr_tail_u8_forward, with the same packed weight.
+ *   out_y, out_u, out_v: uint8 planes by element strides of the plane viewed as (n, 1, H, W) (the second stride is
+ *         not read); out_u and out_v are (out_h/2, out_w/2).  Arbitrary strides write I420 planes or NV12 (u = uv[...,
+ *         0::2], v = uv[..., 1::2]).
+ * out_h and out_w must be even; everything eavsr_sr_tail_u8_forward rejects, and a bad matrix, returns
+ * EAVSR_ERR_INVALID; dtype other than EAVSR_BF16 returns EAVSR_ERR_UNSUPPORTED. */
+int eavsr_sr_tail_yuv420_forward(const void* x, const int64_t x_strides[4], const void* packed_weight, const void* bias,
+                                 const float* lr, const int64_t lr_strides[4], void* out_y, const int64_t y_strides[4],
+                                 void* out_u, const int64_t u_strides[4], void* out_v, const int64_t v_strides[4],
+                                 int n, int c, int h, int w, int scale, int out_h, int out_w, float kr, float kb,
+                                 int dtype, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
