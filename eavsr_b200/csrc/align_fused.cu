@@ -12,6 +12,8 @@
 //   affine_offsets   T*R - R + t expansion + sigmoid(mask)   models/networks.py:302-313
 //   channel_sum /    CALayer (global mean -> 1x1 -> ReLU -> 1x1 -> sigmoid -> scale) + residual add
 //   ca_scale_residual                                        models/networks.py:449-465 (RCABlock)
+#include <cuda.h>
+
 #include "common.cuh"
 
 namespace eavsr {
@@ -20,169 +22,230 @@ namespace {
 // ---------------------------------------------------------------------------------------------
 // adapt_mix
 // ---------------------------------------------------------------------------------------------
-constexpr int MX_TH = 8, MX_TW = 16;            // output tile
-constexpr int MX_IH = MX_TH + 4, MX_IW = MX_TW + 4;
-constexpr int MX_YH = MX_TH + 2, MX_YW = MX_TW + 2;
+// Persistent: each CTA stages both halves' weights once, then walks work items (image, tile, half) with a stride of
+// the grid.  A tile's input (2-pixel halo, zero outside the image) arrives as one 4-D TMA tensor load into a
+// two-deep mbarrier ring: the load of item j + 2 is issued as soon as item j's stage 1 has read its buffer, so it
+// overlaps two items of math.  bf16 tiles stay small enough for two CTAs per SM (16 warps): the two __syncthreads
+// of an item stall one CTA while the other computes.
 constexpr int MX_C = 64;                        // channels of each input
-constexpr int MX_THREADS = 256;
+constexpr int MX_NS = 2;                        // input ring depth
 
-// 8 consecutive channels from shared memory, widened to fp32 (one / two 16-byte LDS)
-__device__ __forceinline__ void lds8(const __nv_bfloat16* p, float* f) {
-  const uint4 u = *reinterpret_cast<const uint4*>(p);
-  f[0] = bf16lo_to_f32(u.x); f[1] = bf16hi_to_f32(u.x); f[2] = bf16lo_to_f32(u.y); f[3] = bf16hi_to_f32(u.y);
-  f[4] = bf16lo_to_f32(u.z); f[5] = bf16hi_to_f32(u.z); f[6] = bf16lo_to_f32(u.w); f[7] = bf16hi_to_f32(u.w);
-}
-__device__ __forceinline__ void lds8(const float* p, float* f) {
-  const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
-  f[0] = a.x; f[1] = a.y; f[2] = a.z; f[3] = a.w; f[4] = b.x; f[5] = b.y; f[6] = b.z; f[7] = b.w;
-}
+// output tile, threads and CTAs per SM of each instantiation
+template <typename T> struct MixTile;
+template <> struct MixTile<__nv_bfloat16> { static constexpr int TH = 8, TW = 16, THREADS = 256, MINB = 2; };
+// fp32: the 8x16 tile's ring + y (178 KB) leaves one CTA per SM; measured faster than two CTAs on 8x8 tiles, which
+// pay 1.56x stage-1 recompute and twice the per-item overhead
+template <> struct MixTile<float> { static constexpr int TH = 8, TW = 16, THREADS = 256, MINB = 1; };
 
 template <typename T> struct MixSmem {
-  T in[MX_IH * MX_IW][MX_C];
-  T y[MX_YH * MX_YW][MX_C];
-  float w1[9][MX_C];
-  float w2[9][MX_C];
-  float b1[MX_C];
-  float b2[MX_C / 2];
+  static constexpr int TH = MixTile<T>::TH, TW = MixTile<T>::TW;
+  static constexpr int IH = TH + 4, IW = TW + 4, YH = TH + 2, YW = TW + 2;
+  static constexpr uint32_t STAGE_BYTES = IH * IW * MX_C * sizeof(T);
+  T in[MX_NS][IH * IW][MX_C];
+  T y[YH * YW][MX_C];
+  T w1[2][9][MX_C];                             // [half][tap][c]: depthwise weight of cat channel half * 64 + c
+  T w2[2][9][MX_C];                             // [half][tap][c]: weight of y channel c into out channel half * 32 + c / 2
+  float b1[2 * MX_C];
+  float b2[MX_C];
+  uint64_t full[MX_NS];
+};
+static_assert(MixSmem<__nv_bfloat16>::STAGE_BYTES % 128 == 0 && MixSmem<float>::STAGE_BYTES % 128 == 0,
+              "ring stages must stay 128-byte aligned for the tensor loads");
+
+struct MixParams {
+  // (64 ch, W, H, N) views of a and b, box (64, TW + 4, TH + 4, 1), no swizzle, out-of-image pixels zero-filled
+  alignas(64) CUtensorMap ta;
+  alignas(64) CUtensorMap tb;
+  const void* w1;
+  const void* b1;
+  const void* w2;
+  const void* b2;
+  void* out;
+  int H, W, tiles_x, tiles_y, total;
+  float slope;
+};
+
+// 8 consecutive channels as 32-bit registers and one multiply-add of channel e.  bf16 keeps the channels packed
+// (4 registers) and multiplies them as they are: fma.rn.f32.bf16 (FHFMA.BF16 reading either half of a register)
+// forms the exact product of two bf16 values and rounds its fp32 sum once, the same bits as widening both operands
+// and issuing FFMA, without the 96 widening instructions per 144 FMAs that bound the kernel before.
+template <typename T> struct MixMath;
+template <> struct MixMath<__nv_bfloat16> {
+  static constexpr int NR = 4;
+  static __device__ __forceinline__ void ld(const __nv_bfloat16* p, uint32_t* r) {
+    const uint4 u = *reinterpret_cast<const uint4*>(p);
+    r[0] = u.x; r[1] = u.y; r[2] = u.z; r[3] = u.w;
+  }
+  static __device__ __forceinline__ float fma(const uint32_t* w, const uint32_t* v, int e, float c) {
+    const uint32_t a = w[e >> 1], b = v[e >> 1];
+    const unsigned short x = (e & 1) ? (unsigned short)(a >> 16) : (unsigned short)(a & 0xffffu);
+    const unsigned short y = (e & 1) ? (unsigned short)(b >> 16) : (unsigned short)(b & 0xffffu);
+    float d;
+    asm("fma.rn.f32.bf16 %0, %1, %2, %3;" : "=f"(d) : "h"(x), "h"(y), "f"(c));
+    return d;
+  }
+  static __device__ __forceinline__ void st8(__nv_bfloat16* p, const float* f) { VecLoad<__nv_bfloat16, 8>::st(p, f); }
+  static __device__ __forceinline__ void st4(__nv_bfloat16* p, const float* f) {
+    *reinterpret_cast<uint2*>(p) = make_uint2(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]));
+  }
+};
+template <> struct MixMath<float> {
+  static constexpr int NR = 8;
+  static __device__ __forceinline__ void ld(const float* p, uint32_t* r) {
+    const uint4 a = *reinterpret_cast<const uint4*>(p), b = *reinterpret_cast<const uint4*>(p + 4);
+    r[0] = a.x; r[1] = a.y; r[2] = a.z; r[3] = a.w; r[4] = b.x; r[5] = b.y; r[6] = b.z; r[7] = b.w;
+  }
+  static __device__ __forceinline__ float fma(const uint32_t* w, const uint32_t* v, int e, float c) {
+    return fmaf(__uint_as_float(w[e]), __uint_as_float(v[e]), c);
+  }
+  static __device__ __forceinline__ void st8(float* p, const float* f) {
+    *reinterpret_cast<float4*>(p) = make_float4(f[0], f[1], f[2], f[3]);
+    *reinterpret_cast<float4*>(p + 4) = make_float4(f[4], f[5], f[6], f[7]);
+  }
+  static __device__ __forceinline__ void st4(float* p, const float* f) {
+    *reinterpret_cast<float4*>(p) = make_float4(f[0], f[1], f[2], f[3]);
+  }
 };
 
 template <typename T>
-__global__ void __launch_bounds__(MX_THREADS)
-adapt_mix_kernel(const T* __restrict__ a, const T* __restrict__ b, const T* __restrict__ w1g,
-                 const T* __restrict__ b1g, const T* __restrict__ w2g, const T* __restrict__ b2g,
-                 T* __restrict__ out, int H, int W, float slope) {
-  extern __shared__ __align__(16) uint8_t mix_smem_raw[];
-  MixSmem<T>& S = *reinterpret_cast<MixSmem<T>*>(mix_smem_raw);
-  constexpr int VEC = 16 / sizeof(T);           // channels per 16-byte chunk
-  constexpr int CPP = MX_C / VEC;               // chunks per pixel
-  const int half = blockIdx.z & 1, n = blockIdx.z >> 1;
-  const int y0 = blockIdx.y * MX_TH, x0 = blockIdx.x * MX_TW;
-  const T* src = (half ? b : a) + (size_t)n * H * W * MX_C;
+__global__ void __launch_bounds__(MixTile<T>::THREADS, MixTile<T>::MINB) adapt_mix_kernel(const __grid_constant__ MixParams P) {
+  using S_ = MixSmem<T>;
+  using M = MixMath<T>;
+  constexpr int TH = S_::TH, TW = S_::TW, IW = S_::IW, YH = S_::YH, YW = S_::YW, NR = M::NR;
+  constexpr int NT = MixTile<T>::THREADS;
+  extern __shared__ uint8_t mix_smem_raw[];
+  S_& S = *reinterpret_cast<S_*>(mix_smem_raw + ((128u - (smem_u32(mix_smem_raw) & 127u)) & 127u));
   const int tid = threadIdx.x;
+  const int my_items = (P.total - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
 
-  // weights of this half: cat channels [half*64, half*64+64) -> out channels [half*32, half*32+32)
-  for (int i = tid; i < 9 * MX_C; i += MX_THREADS) {
-    const int tap = i / MX_C, c = i % MX_C;
-    S.w1[tap][c] = to_f32<T>(w1g[(size_t)(half * MX_C + c) * 9 + tap]);
-    // y channel c feeds out channel half*32 + c/2 as its input (c & 1)
-    S.w2[tap][c] = to_f32<T>(w2g[((size_t)(half * (MX_C / 2) + (c >> 1)) * 2 + (c & 1)) * 9 + tap]);
-  }
-  for (int i = tid; i < MX_C; i += MX_THREADS) S.b1[i] = to_f32<T>(b1g[half * MX_C + i]);
-  for (int i = tid; i < MX_C / 2; i += MX_THREADS) S.b2[i] = to_f32<T>(b2g[half * (MX_C / 2) + i]);
-
-  // input tile with a 2-pixel halo, zero outside the image (conv zero padding)
-  // (cp.async: all 7-8 copies of a thread in flight at once -- with a load -> store loop the tile fill was a
-  // chain of dependent L2 round trips and 28 % of the kernel's stall samples sat on its STS)
-  for (int i = tid; i < MX_IH * MX_IW * CPP; i += MX_THREADS) {
-    const int p = i / CPP, ch = i % CPP;
-    const int gy = y0 - 2 + p / MX_IW, gx = x0 - 2 + p % MX_IW;
-    const bool ok = gy >= 0 && gy < H && gx >= 0 && gx < W;
-    const T* g = ok ? src + ((size_t)gy * W + gx) * MX_C + ch * VEC : src;
-    const int sz = ok ? 16 : 0;
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(smem_u32(&S.in[p][ch * VEC])), "l"(g), "r"(sz));
-  }
-  cp_async_commit();
-  cp_async_wait<0>();
-  __syncthreads();
-
-  // Every thread works on ONE 8-channel chunk for the whole kernel (256 % 8 == 0), so its 9x8 weights
-  // live in registers: the inner loops are one 16-byte LDS + 8 FMAs per tap.
-  const int c0 = (tid & 7) * 8;
-  float wr[9][8], br[8];
-#pragma unroll
-  for (int tap = 0; tap < 9; ++tap)
-#pragma unroll
-    for (int e = 0; e < 8; ++e) wr[tap][e] = S.w1[tap][c0 + e];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) br[e] = S.b1[c0 + e];
-
-  // Both phases are instruction bound (bf16 -> fp32 widening is 40 % of the work), so every thread computes
-  // TWO horizontally adjacent pixels per item: 3 x 4 chunk loads and conversions feed 2 x 72 FMAs instead
-  // of 2 x (3 x 3), and results leave as one 16-byte / 8-byte store per pixel.
-  auto st8 = [](T* p, const float* f) {
-    if constexpr (sizeof(T) == 2) {
-      VecLoad<T, 8>::st(p, f);
-    } else {
-      *reinterpret_cast<float4*>(p) = make_float4(f[0], f[1], f[2], f[3]);
-      *reinterpret_cast<float4*>(p + 4) = make_float4(f[4], f[5], f[6], f[7]);
-    }
+  // item j of this CTA: half fastest, so the a and b tiles of one place run side by side and the two 64-byte
+  // halves of an output pixel reach L2 together
+  auto item_at = [&](int j, int& n, int& half, int& y0, int& x0) {
+    int t = (int)blockIdx.x + j * (int)gridDim.x;
+    half = t & 1;
+    t >>= 1;
+    const int tx = t % P.tiles_x;
+    t /= P.tiles_x;
+    y0 = (t % P.tiles_y) * TH;
+    n = t / P.tiles_y;
+    x0 = tx * TW;
   };
-  // phase 1: y = lrelu(depthwise3x3(in) + b1) on the (TH+2)x(TW+2) ring, 0 outside the image
-  static_assert(MX_YW % 2 == 0 && MX_TW % 2 == 0, "pixel pairs");
-  for (int i = tid; i < MX_YH * (MX_YW / 2) * (MX_C / 8); i += MX_THREADS) {
-    const int pp = i / (MX_C / 8);
-    const int yy = pp / (MX_YW / 2), xx = (pp % (MX_YW / 2)) * 2;
-    float acc[2][8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) acc[0][e] = acc[1][e] = br[e];
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-      float v[4][8];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) lds8(&S.in[(yy + r) * MX_IW + xx + c][c0], v[c]);
-#pragma unroll
-      for (int t = 0; t < 3; ++t)
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          acc[0][e] += wr[r * 3 + t][e] * v[t][e];
-          acc[1][e] += wr[r * 3 + t][e] * v[t + 1][e];
-        }
+  auto issue = [&](int j) {
+    int n, half, y0, x0;
+    item_at(j, n, half, y0, x0);
+    const uint32_t bar = smem_u32(&S.full[j % MX_NS]);
+    mbar_arrive_expect_tx(bar, S_::STAGE_BYTES);
+    asm volatile(
+        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];\n" ::
+            "r"(smem_u32(&S.in[j % MX_NS][0][0])),
+        "l"(reinterpret_cast<uint64_t>(half ? &P.tb : &P.ta)), "r"(0), "r"(x0 - 2), "r"(y0 - 2), "r"(n), "r"(bar)
+        : "memory");
+  };
+
+  if (tid == 0) {
+    for (int s = 0; s < MX_NS; ++s) mbar_init(smem_u32(&S.full[s]), 1);
+    fence_mbar_init();
+    for (int j = 0; j < MX_NS && j < my_items; ++j) issue(j);
+  }
+  {
+    const T* w1g = static_cast<const T*>(P.w1);
+    const T* w2g = static_cast<const T*>(P.w2);
+    for (int i = tid; i < 2 * 9 * MX_C; i += NT) {
+      const int half = i / (9 * MX_C), tap = (i / MX_C) % 9, c = i % MX_C;
+      S.w1[half][tap][c] = w1g[(size_t)(half * MX_C + c) * 9 + tap];
+      S.w2[half][tap][c] = w2g[((size_t)(half * (MX_C / 2) + (c >> 1)) * 2 + (c & 1)) * 9 + tap];
     }
-    const int gy = y0 - 1 + yy;
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      const int gx = x0 - 1 + xx + k;
-      const bool inside = gy >= 0 && gy < H && gx >= 0 && gx < W;
-      float o[8];
-#pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        const float v = acc[k][e] > 0.f ? acc[k][e] : acc[k][e] * slope;
-        o[e] = inside ? v : 0.f;
-      }
-      st8(&S.y[yy * MX_YW + xx + k][c0], o);
-    }
+    for (int i = tid; i < 2 * MX_C; i += NT) S.b1[i] = to_f32<T>(static_cast<const T*>(P.b1)[i]);
+    for (int i = tid; i < MX_C; i += NT) S.b2[i] = to_f32<T>(static_cast<const T*>(P.b2)[i]);
   }
   __syncthreads();
 
-  // phase 2: out[o] = lrelu(b2[o] + sum_tap w2[tap][2o] y[2o] + w2[tap][2o+1] y[2o+1])
+  // Every thread works on ONE 8-channel chunk for the whole kernel (NT % 8 == 0), so its 9 x 8 weights of a
+  // stage live in registers and every tap is one 16-byte LDS + 8 FMAs per pixel.  Each thread computes TWO
+  // horizontally adjacent pixels per step: 3 x 4 chunk loads feed 2 x 72 FMAs.
+  const int c0 = (tid & 7) * 8;
+  static_assert(YW % 2 == 0 && TW % 2 == 0 && NT % 8 == 0, "pixel pairs, whole chunk groups");
+  T* out = static_cast<T*>(P.out);
+  for (int j = 0; j < my_items; ++j) {
+    int n, half, y0, x0;
+    item_at(j, n, half, y0, x0);
+    const int s = j % MX_NS;
+    uint32_t wr[9][NR];
 #pragma unroll
-  for (int tap = 0; tap < 9; ++tap)
+    for (int tap = 0; tap < 9; ++tap) M::ld(&S.w1[half][tap][c0], wr[tap]);
+    mbar_wait(smem_u32(&S.full[s]), (j / MX_NS) & 1);
+
+    // stage 1: y = lrelu(b1 + depthwise3x3(in)) on the (TH+2)x(TW+2) ring, rounded to T, 0 outside the image
+    for (int i = tid; i < YH * (YW / 2) * (MX_C / 8); i += NT) {
+      const int pp = i / (MX_C / 8);
+      const int yy = pp / (YW / 2), xx = (pp % (YW / 2)) * 2;
+      float acc[2][8];
 #pragma unroll
-    for (int e = 0; e < 8; ++e) wr[tap][e] = S.w2[tap][c0 + e];
-  for (int i = tid; i < MX_TH * (MX_TW / 2) * (MX_C / 8); i += MX_THREADS) {
-    const int pp = i / (MX_C / 8);
-    const int yy = pp / (MX_TW / 2), xx = (pp % (MX_TW / 2)) * 2;
-    const int gy = y0 + yy, gx = x0 + xx;
-    if (gy >= H || gx >= W) continue;
-    float acc[2][4];
+      for (int e = 0; e < 8; ++e) acc[0][e] = acc[1][e] = S.b1[half * MX_C + c0 + e];
 #pragma unroll
-    for (int e = 0; e < 4; ++e) acc[0][e] = acc[1][e] = S.b2[(c0 >> 1) + e];
+      for (int r = 0; r < 3; ++r) {
+        uint32_t v[4][NR];
 #pragma unroll
-    for (int r = 0; r < 3; ++r) {
-      float v[4][8];
+        for (int c = 0; c < 4; ++c) M::ld(&S.in[s][(yy + r) * IW + xx + c][c0], v[c]);
 #pragma unroll
-      for (int c = 0; c < 4; ++c) lds8(&S.y[(yy + r) * MX_YW + xx + c][c0], v[c]);
+        for (int t = 0; t < 3; ++t)
 #pragma unroll
-      for (int t = 0; t < 3; ++t)
+          for (int e = 0; e < 8; ++e) {
+            acc[0][e] = M::fma(wr[r * 3 + t], v[t], e, acc[0][e]);
+            acc[1][e] = M::fma(wr[r * 3 + t], v[t + 1], e, acc[1][e]);
+          }
+      }
+      const int gy = y0 - 1 + yy;
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        const int gx = x0 - 1 + xx + k;
+        const bool inside = gy >= 0 && gy < P.H && gx >= 0 && gx < P.W;
+        float o[8];
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
-          acc[0][e >> 1] += wr[r * 3 + t][e] * v[t][e];
-          acc[1][e >> 1] += wr[r * 3 + t][e] * v[t + 1][e];
+          const float v = acc[k][e] > 0.f ? acc[k][e] : acc[k][e] * P.slope;
+          o[e] = inside ? v : 0.f;
         }
-    }
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      if (gx + k >= W) continue;
-      T* op = out + ((size_t)n * H * W + (size_t)gy * W + gx + k) * MX_C + half * (MX_C / 2) + (c0 >> 1);
-      float o[4];
-#pragma unroll
-      for (int e = 0; e < 4; ++e) o[e] = acc[k][e] > 0.f ? acc[k][e] : acc[k][e] * slope;
-      if constexpr (sizeof(T) == 2) {
-        *reinterpret_cast<uint2*>(op) = make_uint2(pack_bf16x2(o[0], o[1]), pack_bf16x2(o[2], o[3]));
-      } else {
-        *reinterpret_cast<float4*>(op) = make_float4(o[0], o[1], o[2], o[3]);
+        M::st8(&S.y[yy * YW + xx + k][c0], o);
       }
     }
+    __syncthreads();                            // y complete; every thread is done reading in[s]
+    if (tid == 0 && j + MX_NS < my_items) issue(j + MX_NS);
+
+    // stage 2: out[o] = lrelu(b2[o] + sum_tap w2[tap][2o] y[2o] + w2[tap][2o+1] y[2o+1])
+#pragma unroll
+    for (int tap = 0; tap < 9; ++tap) M::ld(&S.w2[half][tap][c0], wr[tap]);
+    for (int i = tid; i < TH * (TW / 2) * (MX_C / 8); i += NT) {
+      const int pp = i / (MX_C / 8);
+      const int yy = pp / (TW / 2), xx = (pp % (TW / 2)) * 2;
+      const int gy = y0 + yy, gx = x0 + xx;
+      if (gy >= P.H || gx >= P.W) continue;
+      float acc[2][4];
+#pragma unroll
+      for (int e = 0; e < 4; ++e) acc[0][e] = acc[1][e] = S.b2[half * (MX_C / 2) + (c0 >> 1) + e];
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        uint32_t v[4][NR];
+#pragma unroll
+        for (int c = 0; c < 4; ++c) M::ld(&S.y[(yy + r) * YW + xx + c][c0], v[c]);
+#pragma unroll
+        for (int t = 0; t < 3; ++t)
+#pragma unroll
+          for (int e = 0; e < 8; ++e) {
+            acc[0][e >> 1] = M::fma(wr[r * 3 + t], v[t], e, acc[0][e >> 1]);
+            acc[1][e >> 1] = M::fma(wr[r * 3 + t], v[t + 1], e, acc[1][e >> 1]);
+          }
+      }
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        if (gx + k >= P.W) continue;
+        float o[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) o[e] = acc[k][e] > 0.f ? acc[k][e] : acc[k][e] * P.slope;
+        M::st4(out + ((size_t)n * P.H * P.W + (size_t)gy * P.W + gx + k) * MX_C + half * (MX_C / 2) + (c0 >> 1), o);
+      }
+    }
+    __syncthreads();                            // y is rewritten by the next item's stage 1
   }
 }
 
@@ -395,13 +458,36 @@ bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 template <typename T>
 int mix_launch(const void* a, const void* b, const void* w1, const void* b1, const void* w2, const void* b2,
                void* out, int n, int h, int w, float slope, cudaStream_t st) {
+  using S_ = MixSmem<T>;
+  const int dt = sizeof(T) == 2 ? EAVSR_BF16 : EAVSR_F32;
+  const long long total = 2ll * n * ceil_div(h, S_::TH) * ceil_div(w, S_::TW);
+  EAVSR_REQUIRE(total < (1ll << 31), "adapt_mix: too many tiles");
+  MixParams P;
+  const unsigned long long dims[4] = {MX_C, (unsigned long long)w, (unsigned long long)h, (unsigned long long)n};
+  const unsigned long long str[3] = {MX_C * sizeof(T), (unsigned long long)w * MX_C * sizeof(T),
+                                     (unsigned long long)h * w * MX_C * sizeof(T)};
+  const unsigned box[4] = {MX_C, S_::IW, S_::IH, 1};
+  if (!encode_tensor_map(&P.ta, dt, 4, a, dims, str, box, 0 /* CU_TENSOR_MAP_SWIZZLE_NONE */) ||
+      !encode_tensor_map(&P.tb, dt, 4, b, dims, str, box, 0)) {
+    set_error("adapt_mix: the tensor maps of the inputs were rejected");
+    return EAVSR_ERR_UNSUPPORTED;
+  }
+  P.w1 = w1; P.b1 = b1; P.w2 = w2; P.b2 = b2; P.out = out;
+  P.H = h; P.W = w;
+  P.tiles_x = ceil_div(w, S_::TW); P.tiles_y = ceil_div(h, S_::TH);
+  P.total = (int)total;
+  P.slope = slope;
   auto k = adapt_mix_kernel<T>;
-  const int smem = (int)sizeof(MixSmem<T>);
+  const int smem = (int)sizeof(S_) + 128;       // + alignment slack of the ring
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) { set_error("adapt_mix: smem attr: %s", cudaGetErrorString(e)); return EAVSR_ERR_CUDA; }
-  dim3 grid(ceil_div(w, MX_TW), ceil_div(h, MX_TH), n * 2);
-  k<<<grid, MX_THREADS, smem, st>>>((const T*)a, (const T*)b, (const T*)w1, (const T*)b1, (const T*)w2,
-                                    (const T*)b2, (T*)out, h, w, slope);
+  int dev = 0, sms = 148, per_sm = 1;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, MixTile<T>::THREADS, smem);
+  if (e != cudaSuccess || per_sm < 1) { set_error("adapt_mix: occupancy: %s", cudaGetErrorString(e)); return EAVSR_ERR_CUDA; }
+  const long long grid = total < (long long)sms * per_sm ? total : (long long)sms * per_sm;
+  k<<<(unsigned)grid, MixTile<T>::THREADS, smem, st>>>(P);
   return check_launch("adapt_mix");
 }
 
@@ -417,7 +503,6 @@ extern "C" int eavsr_adapt_mix_forward(const void* a, const void* b, const void*
   EAVSR_REQUIRE(n > 0 && h > 0 && w > 0, "adapt_mix: empty tensor");
   if (c != MX_C) { set_error("adapt_mix: only %d-channel inputs are fused (got %d)", MX_C, c); return EAVSR_ERR_UNSUPPORTED; }
   EAVSR_REQUIRE(al16(a) && al16(b) && al16(out), "adapt_mix: tensors must be 16-byte aligned dense NHWC");
-  EAVSR_REQUIRE(2 * n <= 65535 && ceil_div(h, MX_TH) <= 65535, "adapt_mix: batch/height too large");
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == EAVSR_F32) return mix_launch<float>(a, b, w1, b1, w2, b2, out, n, h, w, negative_slope, st);
   if (dtype == EAVSR_BF16) return mix_launch<__nv_bfloat16>(a, b, w1, b1, w2, b2, out, n, h, w, negative_slope, st);
