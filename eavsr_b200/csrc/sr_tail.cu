@@ -1,5 +1,6 @@
 // Reconstruction tail of EAVSR+ as one tcgen05 kernel, writing 8-bit frames (models/eavsrp_model.py:350-364 followed
-// by the visuals of models/base_model.py:146-150):
+// by the visuals of models/base_model.py:146-150), or 16-bit ones (M = 2^bits - 1 in place of 255), or Y'CbCr 4:2:0
+// planes of 8- or 16-bit samples (the store types below):
 //
 //   out[n, y, x, c] = rint(clamp(255 * (b[c] + sum_{k,ci} W[c,ci,k] X[n,ci,y+ky-1,x+kx-1] + up_s(lr)[n,c,y,x]), 0, 255))
 //
@@ -54,19 +55,40 @@ struct StSmem {
   static constexpr int DYN = TOTAL + 1024;
 };
 
-// The epilogue's store, a template parameter of the kernel: interleaved RGB, or Y'CbCr 4:2:0 planes.
+// The epilogue's store, a template parameter of the kernel: interleaved RGB, or Y'CbCr 4:2:0 planes, of 8-bit samples
+// or of 16-bit samples (10-, 12- or 16-bit codes).  T is the sample type; the 8-bit stores keep their constants as
+// immediates, the 16-bit ones carry theirs.
 struct RgbOut {
+  using T = uint8_t;
   uint8_t* p;
   long long s_n, s_y, s_x, s_c;
 };
-struct PlaneOut {
-  uint8_t* p;
+struct Rgb16Out {
+  using T = uint16_t;
+  uint16_t* p;
+  long long s_n, s_y, s_x, s_c;
+  float m;                         // 2^bits - 1
+};
+template <class T>
+struct PlaneOutT {
+  T* p;
   long long s_n, s_y, s_x;
 };
+using PlaneOut = PlaneOutT<uint8_t>;
 struct Yuv420Out {
+  using T = uint8_t;
   PlaneOut y, u, v;                // u, v: (out_h / 2, out_w / 2)
   float kr, kg, kb, cu, cv;        // fp32 coefficients of eavsr_b200/yuv.py: cu = 112 / (1 - kb), cv = 112 / (1 - kr)
 };
+struct Yuv420Out16 {
+  using T = uint16_t;
+  PlaneOutT<uint16_t> y, u, v;
+  float kr, kg, kb, cu, cv;        // with k = 2^(bits - 8): cu = 112k / (1 - kb), cv = 112k / (1 - kr)
+  float ys, yo, co;                // 219k, 16k, 128k
+  int shift;                       // codes are stored times 2^shift
+};
+template <class Out>
+constexpr bool is_yuv420 = std::is_same<Out, Yuv420Out>::value || std::is_same<Out, Yuv420Out16>::value;
 
 template <class Out>
 struct TailParams {
@@ -85,7 +107,7 @@ struct TailParams {
 // double-buffered slot of 2 x 3 x 16 floats; one named barrier per pair (ids 1-4)
 constexpr int ST_XCH = 4 * 2 * 3 * 16 * 4;
 template <class Out>
-constexpr int st_dyn() { return StSmem::DYN + (std::is_same<Out, Yuv420Out>::value ? ST_XCH : 0); }
+constexpr int st_dyn() { return StSmem::DYN + (is_yuv420<Out> ? ST_XCH : 0); }
 
 // packed[tap][o][ci] (o < 16, K-major SW128) = W[o, ci, tap] for o < 3, 0 otherwise
 __global__ void sr_tail_pack_weight_kernel(const __nv_bfloat16* __restrict__ w, uint8_t* __restrict__ packed) {
@@ -98,7 +120,8 @@ __global__ void sr_tail_pack_weight_kernel(const __nv_bfloat16* __restrict__ w, 
 
 template <class Out>
 __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_constant__ TailParams<Out> P) {
-  constexpr bool YUV = std::is_same<Out, Yuv420Out>::value;
+  constexpr bool YUV = is_yuv420<Out>;
+  using T = typename Out::T;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
@@ -230,18 +253,24 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_acce + 8 * team);          // accumulator drained: tile tl + 2 may start
       if constexpr (!YUV) {
-        uint8_t* op = P.out.p + n * P.out.s_n + (long long)y * P.out.s_y + (long long)x * P.out.s_x;
+        T* op = P.out.p + n * P.out.s_n + (long long)y * P.out.s_y + (long long)x * P.out.s_x;
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
           const float t = __uint_as_float(a0[c]) + __shfl_down_sync(0xffffffffu, __uint_as_float(a1[c]), 1) +
                           __shfl_down_sync(0xffffffffu, __uint_as_float(a2[c]), 2);
-          // the reference's visuals: clamp(sr * 255, 0, 255).round(), round half to even
-          const float v = fminf(fmaxf(255.f * ((t + bias[c]) + up[c]), 0.f), 255.f);
-          if (valid) op[c * P.out.s_c] = (uint8_t)__float2int_rn(v);
+          if constexpr (sizeof(T) == 1) {
+            // the reference's visuals: clamp(sr * 255, 0, 255).round(), round half to even
+            const float v = fminf(fmaxf(255.f * ((t + bias[c]) + up[c]), 0.f), 255.f);
+            if (valid) op[c * P.out.s_c] = (uint8_t)__float2int_rn(v);
+          } else {
+            // the same at M = 2^bits - 1
+            const float v = fminf(fmaxf(P.out.m * ((t + bias[c]) + up[c]), 0.f), P.out.m);
+            if (valid) op[c * P.out.s_c] = (uint16_t)__float2int_rn(v);
+          }
         }
       } else {
         // rgb_to_yuv420 of eavsr_b200/yuv.py in its fp32 order of operations (no contraction into FMAs)
-        const Yuv420Out& o = P.out;
+        const Out& o = P.out;
         float v[3], s[3];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
@@ -251,9 +280,15 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
           s[c] = __fadd_rn(v[c], __shfl_xor_sync(0xffffffffu, v[c], 1));      // p(x) + p(x + 1), x even
         }
         const float yc = __fadd_rn(__fadd_rn(__fmul_rn(o.kr, v[0]), __fmul_rn(o.kg, v[1])), __fmul_rn(o.kb, v[2]));
-        if (valid)
-          o.y.p[n * o.y.s_n + (long long)y * o.y.s_y + (long long)x * o.y.s_x] =
-              (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(219.f, yc), 16.f));
+        if constexpr (sizeof(T) == 1) {
+          if (valid)
+            o.y.p[n * o.y.s_n + (long long)y * o.y.s_y + (long long)x * o.y.s_x] =
+                (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(219.f, yc), 16.f));
+        } else {
+          if (valid)
+            o.y.p[n * o.y.s_n + (long long)y * o.y.s_y + (long long)x * o.y.s_x] =
+                (uint16_t)(__float2int_rn(__fadd_rn(__fmul_rn(o.ys, yc), o.yo)) << o.shift);
+        }
         // tile origins are even and out_h, out_w are even: a 2x2 block is lanes (2k, 2k + 1) of warps q, q + 1 of
         // one team, and it is valid as a whole.  The slot is double-buffered over the team's tiles, so the write
         // for its next tile lands in the other buffer, and the one after that waits at the barrier for this read
@@ -272,10 +307,17 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
             for (int c = 0; c < 3; ++c) m[c] = __fmul_rn(__fadd_rn(s[c], xch[c * 16 + (lane >> 1)]), 0.25f);
             const float ym = __fadd_rn(__fadd_rn(__fmul_rn(o.kr, m[0]), __fmul_rn(o.kg, m[1])), __fmul_rn(o.kb, m[2]));
             const long long yh = y >> 1, xh = x >> 1;
-            o.u.p[n * o.u.s_n + yh * o.u.s_y + xh * o.u.s_x] =
-                (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[2], ym), o.cu), 128.f));
-            o.v.p[n * o.v.s_n + yh * o.v.s_y + xh * o.v.s_x] =
-                (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[0], ym), o.cv), 128.f));
+            if constexpr (sizeof(T) == 1) {
+              o.u.p[n * o.u.s_n + yh * o.u.s_y + xh * o.u.s_x] =
+                  (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[2], ym), o.cu), 128.f));
+              o.v.p[n * o.v.s_n + yh * o.v.s_y + xh * o.v.s_x] =
+                  (uint8_t)__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[0], ym), o.cv), 128.f));
+            } else {
+              o.u.p[n * o.u.s_n + yh * o.u.s_y + xh * o.u.s_x] =
+                  (uint16_t)(__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[2], ym), o.cu), o.co)) << o.shift);
+              o.v.p[n * o.v.s_n + yh * o.v.s_y + xh * o.v.s_x] =
+                  (uint16_t)(__float2int_rn(__fadd_rn(__fmul_rn(__fsub_rn(m[0], ym), o.cv), o.co)) << o.shift);
+            }
           }
         }
       }
@@ -287,7 +329,7 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
   if (warp == 1) tmem_dealloc<ST_TMEM>(tmem_d);
 }
 
-// checks, tensor map and launch shared by the RGB and the 4:2:0 entry points
+// checks, tensor map and launch shared by the RGB and the 4:2:0 entry points of both sample sizes
 template <class Out>
 int sr_tail_launch(const char* who, const void* x, const int64_t x_strides[4], const void* packed_weight,
                    const void* bias, const float* lr, const int64_t lr_strides[4], const Out& out, int n, int c, int h,
@@ -387,4 +429,53 @@ extern "C" int eavsr_sr_tail_yuv420_forward(const void* x, const int64_t x_strid
   o.cu = 112.f / (1.f - kb); o.cv = 112.f / (1.f - kr);
   return sr_tail_launch("sr_tail_yuv420_forward", x, x_strides, packed_weight, bias, lr, lr_strides, o, n, c, h, w,
                         scale, out_h, out_w, dtype, stream);
+}
+
+static bool hbd_bits_ok(int bits) { return bits == 10 || bits == 12 || bits == 16; }
+
+extern "C" int eavsr_sr_tail_u16_forward(const void* x, const int64_t x_strides[4], const void* packed_weight,
+                                         const void* bias, const float* lr, const int64_t lr_strides[4], void* out,
+                                         const int64_t out_strides[4], int n, int c, int h, int w, int scale,
+                                         int out_h, int out_w, int bits, int dtype, void* stream) {
+  EAVSR_REQUIRE(x && x_strides && packed_weight && lr && lr_strides && out && out_strides,
+                "sr_tail_u16_forward: null pointer");
+  EAVSR_REQUIRE(hbd_bits_ok(bits), "sr_tail_u16_forward: bits must be 10, 12 or 16 (got %d)", bits);
+  EAVSR_REQUIRE((reinterpret_cast<uintptr_t>(out) & 1u) == 0, "sr_tail_u16_forward: out must be 2-byte aligned");
+  const Rgb16Out o = {(uint16_t*)out, out_strides[0], out_strides[1], out_strides[2], out_strides[3],
+                      (float)((1 << bits) - 1)};
+  return sr_tail_launch("sr_tail_u16_forward", x, x_strides, packed_weight, bias, lr, lr_strides, o, n, c, h, w,
+                        scale, out_h, out_w, dtype, stream);
+}
+
+extern "C" int eavsr_sr_tail_yuv420_u16_forward(const void* x, const int64_t x_strides[4], const void* packed_weight,
+                                                const void* bias, const float* lr, const int64_t lr_strides[4],
+                                                void* out_y, const int64_t y_strides[4], void* out_u,
+                                                const int64_t u_strides[4], void* out_v, const int64_t v_strides[4],
+                                                int n, int c, int h, int w, int scale, int out_h, int out_w, float kr,
+                                                float kb, int bits, int shift, int dtype, void* stream) {
+  EAVSR_REQUIRE(x && x_strides && packed_weight && lr && lr_strides && out_y && y_strides && out_u && u_strides &&
+                    out_v && v_strides,
+                "sr_tail_yuv420_u16_forward: null pointer");
+  EAVSR_REQUIRE(hbd_bits_ok(bits), "sr_tail_yuv420_u16_forward: bits must be 10, 12 or 16 (got %d)", bits);
+  EAVSR_REQUIRE(shift == 0 || shift == 16 - bits, "sr_tail_yuv420_u16_forward: shift must be 0 or %d (got %d)",
+                16 - bits, shift);
+  EAVSR_REQUIRE(((reinterpret_cast<uintptr_t>(out_y) | reinterpret_cast<uintptr_t>(out_u) |
+                  reinterpret_cast<uintptr_t>(out_v)) & 1u) == 0,
+                "sr_tail_yuv420_u16_forward: the planes must be 2-byte aligned");
+  EAVSR_REQUIRE(out_h % 2 == 0 && out_w % 2 == 0,
+                "sr_tail_yuv420_u16_forward: 4:2:0 needs an even crop (got %dx%d)", out_h, out_w);
+  EAVSR_REQUIRE(kr > 0.f && kb > 0.f && kr + kb < 1.f, "sr_tail_yuv420_u16_forward: bad matrix (kr %g, kb %g)", kr,
+                kb);
+  Yuv420Out16 o;
+  o.y = {(uint16_t*)out_y, y_strides[0], y_strides[2], y_strides[3]};
+  o.u = {(uint16_t*)out_u, u_strides[0], u_strides[2], u_strides[3]};
+  o.v = {(uint16_t*)out_v, v_strides[0], v_strides[2], v_strides[3]};
+  // the fp32 coefficients of eavsr_b200/yuv.py at k = 2^(bits - 8); k is a power of two, so k * cu is exact
+  const float k = (float)(1 << (bits - 8));
+  o.kr = kr; o.kb = kb; o.kg = (1.f - kr) - kb;
+  o.cu = k * (112.f / (1.f - kb)); o.cv = k * (112.f / (1.f - kr));
+  o.ys = 219.f * k; o.yo = 16.f * k; o.co = 128.f * k;
+  o.shift = shift;
+  return sr_tail_launch("sr_tail_yuv420_u16_forward", x, x_strides, packed_weight, bias, lr, lr_strides, o, n, c, h,
+                        w, scale, out_h, out_w, dtype, stream);
 }

@@ -30,8 +30,9 @@ from .ops import (ModulatedDeformConv2d, adapt_mix, grouped_conv3x3, grouped_con
                   conv3x3_64, conv3x3_64_ca, conv3x3_64_eligible, conv3x3_chain_eligible, rca_group_chain,
                   flow_warp, flow_warp2, flow_warp_nhw2, flow_warp_pyramid, flow_warp_pyramid_eligible, fused_inference_ok,
                   spynet_level_input, sr_tail_u8, sr_tail_u8_eligible, sr_tail_yuv420,
+                  sr_tail_u16, sr_tail_yuv420_u16,
                   modulated_deform_conv2d)
-from .yuv import MATRICES, rgb_to_yuv420, yuv420_to_rgb
+from .yuv import HBD_MATRICES, MATRICES, check_bits, rgb_to_yuv420, yuv420_to_rgb
 
 __all__ = ["EAVSRP", "MultiAdSTN", "SPyNet"]
 
@@ -597,8 +598,94 @@ class EAVSRP(nn.Module):
             self._sr_frames(yuv420_to_rgb(y, u, v, kr, kb), fused, composed)
         return tuple(out)
 
+    def forward_uint16(self, frames, bits=16):
+        """16-bit RGB frames in and out, for 10-, 12- or 16-bit codes: ``frames`` (n, t, h, w, 3) uint16 on the GPU,
+        codes 0 .. M = 2**bits - 1 in the low bits -> (n, t, s*h, s*w, 3) uint16, ``round(clamp(sr * M, 0, M))`` of
+        the forward on ``frames / M``.  As `forward_uint8` otherwise: padded to multiples of 4 and cropped back; with
+        bf16 features one kernel per frame (`ops.sr_tail_u16`) keeps the residual in fp32 and writes the codes,
+        otherwise PyTorch composes the tail.  Inference only (``no_grad``); no host synchronisation, so codes above M
+        are not rejected (they scale past 1 as they are) and it can be captured in a CUDA graph."""
+        if not isinstance(frames, torch.Tensor) or frames.dtype != torch.uint16:
+            raise TypeError(f"EAVSRP.forward_uint16 takes a uint16 tensor, got {getattr(frames, 'dtype', type(frames))}")
+        check_bits("EAVSRP.forward_uint16", bits, 0, allowed=(10, 12, 16))
+        if frames.dim() != 5 or frames.shape[-1] != 3:
+            raise ValueError(f"EAVSRP.forward_uint16 takes (n, t, h, w, 3) RGB frames, got {tuple(frames.shape)}")
+        n, t, h, w, _ = frames.shape
+        if h < 64 or w < 64:
+            raise ValueError(f"EAVSRP.forward_uint16 needs a height and width of at least 64, got {h}x{w}")
+        if not frames.is_cuda:
+            raise NotImplementedError("EAVSRP.forward_uint16: CUDA tensors only (the B200 library has no CPU fallback)")
+        s, m = self.scale, float(2 ** bits - 1)
+        with torch.no_grad():
+            lrs = frames.permute(0, 1, 4, 2, 3).float().div(m).contiguous()
+            out = torch.empty((n, t, s * h, s * w, 3), dtype=torch.uint16, device=frames.device)
+
+            def fused(i, x, lr):
+                sr_tail_u16(self.conv_last, x, lr, s, out[:, i], s * h, s * w, bits)
+
+            def composed(i, sr):
+                out[:, i] = torch.clamp(sr * m, 0, m).round().permute(0, 2, 3, 1).to(torch.uint16)
+            self._sr_frames(lrs, fused, composed)
+        return out
+
+    def forward_yuv420_u16(self, y, u, v, bits=10, shift=0, matrix="bt709", out=None):
+        """Limited-range Y'CbCr 4:2:0 frames of 10, 12 or 16 bits in and out, as HEVC Main10 / AV1 decoders and
+        encoders exchange them.
+
+        ``y`` (n, t, h, w) and ``u``, ``v`` (n, t, h/2, w/2) are uint16 planes on the GPU with any strides; h and w
+        are even and at least 64.  Each sample holds a ``bits``-bit code times ``2**shift``: ``shift=0`` is planar
+        ``yuv420p10le`` (codes in the low bits), ``shift = 16 - bits`` is P010 / P012 (codes in the high bits, chroma
+        interleaved: pass the views ``uv[..., 0::2]``, ``uv[..., 1::2]``).  Returns ``(Y, U, V)``: (n, t, s*h, s*w) and
+        (n, t, s*h/2, s*w/2) uint16 in the same packing, or writes into ``out = (Y, U, V)``, caller planes of those
+        shapes with any strides.  ``matrix`` is a key of `yuv.HBD_MATRICES` ("bt709", "bt601", "bt2020").
+
+        The result is ``rgb_to_yuv420(crop(forward(pad_clip(yuv420_to_rgb(y, u, v, bits=bits, shift=shift)))),
+        bits=bits, shift=shift)`` (`eavsr_b200.yuv`).  With bf16 features conv_last, the bilinear base and the
+        conversion run as one kernel per frame (`ops.sr_tail_yuv420_u16`), keeping the residual in fp32; otherwise
+        they are composed in PyTorch.  Inference only (``no_grad``); no host synchronisation, so the code range is not
+        checked (out-of-range codes are converted as they are) and it can be captured in a CUDA graph."""
+        planes = (y, u, v) + (tuple(out) if out is not None else ())
+        for p in planes:
+            if not isinstance(p, torch.Tensor) or p.dtype != torch.uint16:
+                raise TypeError(f"EAVSRP.forward_yuv420_u16 takes uint16 planes, got {getattr(p, 'dtype', type(p))}")
+        check_bits("EAVSRP.forward_yuv420_u16", bits, shift, allowed=(10, 12, 16))
+        if matrix not in HBD_MATRICES:
+            raise ValueError(f"EAVSRP.forward_yuv420_u16: matrix must be one of {sorted(HBD_MATRICES)}, got {matrix!r}")
+        if y.dim() != 4:
+            raise ValueError(f"EAVSRP.forward_yuv420_u16 takes an (n, t, h, w) Y plane, got {tuple(y.shape)}")
+        n, t, h, w = y.shape
+        if h % 2 or w % 2 or h < 64 or w < 64:
+            raise ValueError(f"EAVSRP.forward_yuv420_u16 needs an even height and width of at least 64, got {h}x{w}")
+        s = self.scale
+        shapes = [(n, t, h, w), (n, t, h // 2, w // 2), (n, t, h // 2, w // 2)]
+        if out is not None:
+            if len(out) != 3:
+                raise ValueError(f"EAVSRP.forward_yuv420_u16: out must be three planes (Y, U, V), got {len(out)}")
+            shapes += [(n, t, s * h, s * w), (n, t, s * h // 2, s * w // 2), (n, t, s * h // 2, s * w // 2)]
+        for name, p, shape in zip(("y", "u", "v", "out Y", "out U", "out V"), planes, shapes):
+            if tuple(p.shape) != shape:
+                raise ValueError(f"EAVSRP.forward_yuv420_u16: {name} must be {shape}, got {tuple(p.shape)}")
+        if not all(p.is_cuda for p in planes):
+            raise NotImplementedError("EAVSRP.forward_yuv420_u16: CUDA tensors only (the B200 library has no CPU "
+                                      "fallback)")
+        kr, kb = HBD_MATRICES[matrix]
+        with torch.no_grad():
+            if out is None:
+                out = (torch.empty((n, t, s * h, s * w), dtype=torch.uint16, device=y.device),) + tuple(
+                    torch.empty((n, t, s * h // 2, s * w // 2), dtype=torch.uint16, device=y.device) for _ in range(2))
+            Y, U, V = out
+
+            def fused(i, x, lr):
+                sr_tail_yuv420_u16(self.conv_last, x, lr, s, Y[:, i], U[:, i], V[:, i], s * h, s * w, kr, kb, bits,
+                                   shift)
+
+            def composed(i, sr):
+                Y[:, i], U[:, i], V[:, i] = rgb_to_yuv420(sr, kr, kb, bits, shift)
+            self._sr_frames(yuv420_to_rgb(y, u, v, kr, kb, bits, shift), fused, composed)
+        return tuple(out)
+
     def _sr_frames(self, lrs, fused, composed):
-        """The 8-bit forwards' common part, under ``no_grad``: pad the (n, t, 3, h, w) clip `lrs` (`pad_clip`), run
+        """The frame-in, frame-out forwards' common part, under ``no_grad``: pad the (n, t, 3, h, w) clip `lrs` (`pad_clip`), run
         `_trunk`, then per frame i `_hr_features` and the tail -- ``fused(i, x, lr_i)`` when the fused tail kernel can
         run on the HR features ``x`` (`ops.sr_tail_u8_eligible`), else ``composed(i, sr_i)`` with the SR frame of
         `_sr_frame` cropped to (s*h, s*w)."""

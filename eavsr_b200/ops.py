@@ -36,6 +36,7 @@ from torch.autograd.function import once_differentiable
 from torch.nn.modules.utils import _pair
 
 from . import _lib as L
+from .yuv import check_bits
 
 __all__ = [
     "modulated_deform_conv2d", "ModulatedDeformConv2d", "dcn_affine", "dcn_affine_eligible", "flow_warp", "flow_warp_nhw2",
@@ -45,6 +46,7 @@ __all__ = [
     "adapt_mix", "affine_offsets_mask", "ca_residual", "fused_inference_ok", "bias_act_", "conv2d_bias_act",
     "conv3x3_64", "conv3x3_64_ca", "conv3x3_64_eligible", "ca_scale", "conv2d_bias_act_shuffle",
     "conv3x3_chain_eligible", "rca_group_chain", "sr_tail_u8", "sr_tail_u8_eligible", "sr_tail_yuv420",
+    "sr_tail_u16", "sr_tail_yuv420_u16",
 ]
 
 _DTYPES = {torch.float32: L.F32, torch.bfloat16: L.BF16}
@@ -1104,4 +1106,48 @@ def sr_tail_yuv420(conv_last: nn.Conv2d, x, lr, scale: int, y_out, u_out, v_out,
     _launch("sr_tail_yuv420_forward", x, _strides(x), _packed_conv_weight(conv_last, x.device, "sr_tail"),
             _param(conv_last.bias, torch.bfloat16), lr, L.Strides(*lr.stride()), *planes,
             n, x.shape[1], x.shape[2], x.shape[3], int(scale), int(out_h), int(out_w), float(kr), float(kb), L.BF16)
+    return y_out, u_out, v_out
+
+
+def sr_tail_u16(conv_last: nn.Conv2d, x, lr, scale: int, out, out_h: int, out_w: int, bits: int):
+    """`sr_tail_u8` at 10, 12 or 16 bits: ``out[n, y, x, :] = round(clamp(M * (conv_last(x) + interpolate(lr, scale,
+    bilinear)), 0, M))`` with ``M = 2**bits - 1``, the code in the low bits.  ``out``: (n, out_h, out_w, 3) uint16,
+    any strides.  ``x`` and ``lr`` as for `sr_tail_u8`, with the same eligibility (`sr_tail_u8_eligible`).
+    Returns ``out``."""
+    check_bits("eavsr_b200.sr_tail_u16", bits, 0, allowed=(10, 12, 16))
+    n, c, h, w = x.shape
+    _check_tail_lr("sr_tail_u16", x, lr, scale)
+    if out.dtype != torch.uint16 or tuple(out.shape) != (n, out_h, out_w, 3):
+        raise ValueError(f"eavsr_b200.sr_tail_u16: out must be uint16 (n, out_h, out_w, 3), got {out.dtype} "
+                         f"{tuple(out.shape)}")
+    _require_cuda("sr_tail_u16", x, lr, out)
+    _launch("sr_tail_u16_forward", x, _strides(x), _packed_conv_weight(conv_last, x.device, "sr_tail"),
+            _param(conv_last.bias, torch.bfloat16), lr, L.Strides(*lr.stride()), out, L.Strides(*out.stride()),
+            n, c, h, w, int(scale), int(out_h), int(out_w), int(bits), L.BF16)
+    return out
+
+
+def sr_tail_yuv420_u16(conv_last: nn.Conv2d, x, lr, scale: int, y_out, u_out, v_out, out_h: int, out_w: int,
+                       kr: float, kb: float, bits: int, shift: int):
+    """`sr_tail_yuv420` at 10, 12 or 16 bits: ``rgb_to_yuv420(conv_last(x) + interpolate(lr, scale, bilinear), kr, kb,
+    bits, shift)`` (`eavsr_b200.yuv`) cropped to ``out_h`` x ``out_w``, in one kernel.  ``y_out``: (n, out_h, out_w)
+    uint16; ``u_out``, ``v_out``: (n, out_h/2, out_w/2) uint16; any strides, so planar ``yuv420p10le`` (``shift=0``)
+    or the interleaved chroma of P010 (``shift=6``, ``uv[..., 0::2]``, ``uv[..., 1::2]``) are written in place.
+    ``x`` and ``lr`` as for `sr_tail_u8`, with the same eligibility.  Returns ``(y_out, u_out, v_out)``."""
+    check_bits("eavsr_b200.sr_tail_yuv420_u16", bits, shift, allowed=(10, 12, 16))
+    if out_h % 2 or out_w % 2:
+        raise ValueError(f"eavsr_b200.sr_tail_yuv420_u16: 4:2:0 needs an even crop, got {out_h}x{out_w}")
+    n = x.shape[0]
+    _check_tail_lr("sr_tail_yuv420_u16", x, lr, scale)
+    for name, p, shape in (("y_out", y_out, (n, out_h, out_w)), ("u_out", u_out, (n, out_h // 2, out_w // 2)),
+                           ("v_out", v_out, (n, out_h // 2, out_w // 2))):
+        if p.dtype != torch.uint16 or tuple(p.shape) != shape:
+            raise ValueError(f"eavsr_b200.sr_tail_yuv420_u16: {name} must be uint16 {shape}, got {p.dtype} "
+                             f"{tuple(p.shape)}")
+    _require_cuda("sr_tail_yuv420_u16", x, lr, y_out, u_out, v_out)
+    planes = [a for p in (y_out, u_out, v_out) for a in (p, L.Strides(*p.unsqueeze(1).stride()))]
+    _launch("sr_tail_yuv420_u16_forward", x, _strides(x), _packed_conv_weight(conv_last, x.device, "sr_tail"),
+            _param(conv_last.bias, torch.bfloat16), lr, L.Strides(*lr.stride()), *planes,
+            n, x.shape[1], x.shape[2], x.shape[3], int(scale), int(out_h), int(out_w), float(kr), float(kb),
+            int(bits), int(shift), L.BF16)
     return y_out, u_out, v_out

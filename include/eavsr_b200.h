@@ -382,6 +382,40 @@ int eavsr_sr_tail_yuv420_forward(const void* x, const int64_t x_strides[4], cons
                                  int n, int c, int h, int w, int scale, int out_h, int out_w, float kr, float kb,
                                  int dtype, void* stream);
 
+/* ---- the same tail to 16-bit RGB frames (10-, 12- or 16-bit codes) ----------------------------------------------
+ * With M = 2^bits - 1, for y < out_h, x < out_w and c < 3:
+ *   out[n, y, x, c] = rint(clamp(M * (bias[c] + conv_last(x)[n, c, y, x] + up_s(lr)[n, c, y, x]), 0, M))
+ * i.e. eavsr_sr_tail_u8_forward with M in place of 255, the code in the low bits of a uint16 sample.
+ *   x, W, bias, lr: as eavsr_sr_tail_u8_forward, with the same packed weight.
+ *   out:  uint16, 2-byte aligned, by element strides out_strides in (n, y, x, c) order.
+ * bits must be 10, 12 or 16; that, a misaligned out, and everything eavsr_sr_tail_u8_forward rejects return
+ * EAVSR_ERR_INVALID; dtype other than EAVSR_BF16 returns EAVSR_ERR_UNSUPPORTED. */
+int eavsr_sr_tail_u16_forward(const void* x, const int64_t x_strides[4], const void* packed_weight, const void* bias,
+                              const float* lr, const int64_t lr_strides[4], void* out, const int64_t out_strides[4],
+                              int n, int c, int h, int w, int scale, int out_h, int out_w, int bits, int dtype,
+                              void* stream);
+
+/* ---- the same tail to limited-range Y'CbCr 4:2:0 planes of 10, 12 or 16 bits ------------------------------------
+ * eavsr_sr_tail_yuv420_forward at bits b with k = 2^(b - 8), each code stored times 2^shift in a uint16 sample:
+ *   Y[n, y, x]     = rint(16k + 219k * Yc(v[n, :, y, x]))                         for y < out_h, x < out_w
+ *   U[n, y/2, x/2] = rint(128k + 112k / (1 - kb) * (m_b - Yc(m))),  V likewise with m_r and kr,
+ * in the fp32 order of rgb_to_yuv420(..., bits=b, shift=shift) in eavsr_b200/yuv.py (112k / (1 - kb) is computed as
+ * k * (112 / (1 - kb)), the same fp32 value).  shift = 0 keeps the codes in the low bits (yuv420p10le), shift =
+ * 16 - b puts them in the high bits (P010, P012).  kr, kb as for eavsr_sr_tail_yuv420_forward; BT.2020 is 0.2627,
+ * 0.0593.
+ *   x, W, bias, lr: as eavsr_sr_tail_u8_forward, with the same packed weight.
+ *   out_y, out_u, out_v: uint16 planes, each 2-byte aligned, by element strides of the plane viewed as (n, 1, H, W)
+ *         (the second stride is not read); out_u and out_v are (out_h/2, out_w/2).  Arbitrary strides write planar
+ *         yuv420p10le or P010 (u = uv[..., 0::2], v = uv[..., 1::2] of a uint16 view with a row pitch).
+ * bits not in {10, 12, 16}, shift not in {0, 16 - bits}, a misaligned plane, an odd out_h or out_w, a bad matrix and
+ * everything eavsr_sr_tail_u8_forward rejects return EAVSR_ERR_INVALID; dtype other than EAVSR_BF16 returns
+ * EAVSR_ERR_UNSUPPORTED. */
+int eavsr_sr_tail_yuv420_u16_forward(const void* x, const int64_t x_strides[4], const void* packed_weight,
+                                     const void* bias, const float* lr, const int64_t lr_strides[4], void* out_y,
+                                     const int64_t y_strides[4], void* out_u, const int64_t u_strides[4], void* out_v,
+                                     const int64_t v_strides[4], int n, int c, int h, int w, int scale, int out_h,
+                                     int out_w, float kr, float kb, int bits, int shift, int dtype, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

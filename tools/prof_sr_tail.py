@@ -3,6 +3,7 @@
 
     python tools/prof_sr_tail.py --out DIR [--rounds 5]          -> DIR/sr_tail.json
     python tools/prof_sr_tail.py --out DIR --yuv [--rounds 5]    -> DIR/sr_tail_yuv.json
+    python tools/prof_sr_tail.py --out DIR --hbd [--rounds 5]    -> DIR/sr_tail_hbd.json
 
 (a) The tail of one frame at the benchmark's operating point: 8 images of 64 x 1088 x 1920 bf16 features (2.1 GB,
     far more than L2) -> 8 frames of 1080 x 1920 x 3 uint8.  The fused kernel (`ops.sr_tail_u8`) against the
@@ -23,6 +24,12 @@ With --yuv, the Y'CbCr 4:2:0 variant instead:
     ingest of one step (`pad_clip(yuv420_to_rgb(...))`, captured, CUDA events) next to forward_uint8's ingest, and the
     host CPU time of converting forward_uint8's output to I420 with torch on the CPU, timed on one clip of 30 frames
     and scaled to the 8 clips of a step.
+With --hbd, the high-bit-depth variants:
+(a) the tail at the same operating point: 16-bit RGB (`ops.sr_tail_u16`) and 10-bit BT.709 4:2:0 written as P010
+    (`ops.sr_tail_yuv420_u16`, shift 6, chroma interleaved) against the 8-bit RGB and I420 kernels, alternated.  The
+    HBM floors count 6 and 3 B/px written.
+(b) host to host, 8 clips of 30 x 270 x 480: `forward_yuv420_u16` on P010 (pinned Y and interleaved UV planes -> H2D
+    -> graph -> D2H) against `forward_yuv420` on I420, both graph-captured and alternated.
 The GPU name, power limit and maximum SM clock are read with nvidia-smi in the same run.
 """
 import argparse
@@ -301,6 +308,116 @@ def e2e_yuv(dev, rounds, steps):
     }
 
 
+def tail_hbd(dev, rounds, reps):
+    conv, x, lr, (n, h, w, s, oh, ow) = _tail_operands(dev)
+    kr, kb = MATRICES["bt709"]
+    u8 = lambda *shape: torch.empty(shape, dtype=torch.uint8, device=dev)      # noqa: E731
+    u16 = lambda *shape: torch.empty(shape, dtype=torch.uint16, device=dev)    # noqa: E731
+    rgb8, rgb16 = u8(n, oh, ow, 3), u16(n, oh, ow, 3)
+    i420 = (u8(n, oh, ow), u8(n, oh // 2, ow // 2), u8(n, oh // 2, ow // 2))
+    y10, uv10 = u16(n, oh, ow), u16(n, oh // 2, ow)
+    arms = {
+        "rgb16_kernel": lambda: ops.sr_tail_u16(conv, x, lr, s, rgb16, oh, ow, 16),
+        "p010_kernel": lambda: ops.sr_tail_yuv420_u16(conv, x, lr, s, y10, uv10[..., 0::2], uv10[..., 1::2], oh, ow,
+                                                      kr, kb, 10, 6),
+        "rgb_kernel": lambda: ops.sr_tail_u8(conv, x, lr, s, rgb8, oh, ow),
+        "yuv420_kernel": lambda: ops.sr_tail_yuv420(conv, x, lr, s, *i420, oh, ow, kr, kb),
+    }
+    with torch.no_grad():
+        assert ops.sr_tail_u8_eligible(conv, x)
+        graphs = {k: capture(fn) for k, fn in arms.items()}
+        t = {k: [] for k in arms}
+        for g, _ in graphs.values():
+            time_replays(g, 3)
+        for _ in range(rounds):
+            for k, (g, _) in graphs.items():
+                t[k].append(time_replays(g, reps))
+        # the 16-bit codes against the 8-bit kernels' outputs, rescaled: at most half an 8-bit level apart
+        d_rgb = (rgb16.int().double() * (255 / 65535) - rgb8.int().double()).abs().max().item()
+        d_y = ((y10.int() >> 6).double() / 4 - i420[0].int().double()).abs().max().item()
+    lr_bytes = (h // s) * (w // s) * 12
+    written = {"rgb16_kernel": 6, "p010_kernel": 3, "rgb_kernel": 3, "yuv420_kernel": 1.5}
+    nbytes = {k: n * (h * w * 128 + int(oh * ow * b) + lr_bytes) for k, b in written.items()}
+    med = {k: statistics.median(v) for k, v in t.items()}
+    floor = {k: v / HBM_BPS * 1e6 for k, v in nbytes.items()}
+    return {
+        "shape": {"images": n, "features": [64, h, w], "out": [oh, ow], "scale": s, "matrix": "bt709"},
+        "us_per_frame": med, "us_per_image": {k: v / n for k, v in med.items()},
+        "rounds_us_per_frame": t, "replays_per_round": reps, "bytes_written_per_px": written,
+        "hbm_bytes": nbytes, "hbm_floor_us_at_7.7TBps": floor,
+        "fraction_of_hbm_floor": {k: floor[k] / med[k] for k in med},
+        "rgb16_over_rgb8": med["rgb16_kernel"] / med["rgb_kernel"],
+        "p010_over_yuv420_8bit": med["p010_kernel"] / med["yuv420_kernel"],
+        "max_abs_diff_in_8bit_levels": {"rgb16_vs_rgb8": d_rgb, "y10_vs_y8": d_y},
+    }
+
+
+def e2e_hbd(dev, rounds, steps):
+    clips, t, h, w = 8, 30, 270, 480
+    kr, kb = MATRICES["bt709"]
+    net = EAVSRP(4).eval()
+    seeded_parameters(net)
+    net = net.to(dev).prepare(torch.bfloat16)
+    f32 = torch.cat([clip_inputs(1, t, h, w, seed=1234 + i) for i in range(clips)])
+    host_i420 = [p.contiguous().pin_memory() for p in rgb_to_yuv420(f32, kr, kb)]
+    y, u, v = rgb_to_yuv420(f32, kr, kb, bits=10, shift=6)
+    host_p010 = [y.contiguous().pin_memory(),
+                 torch.stack([u.int(), v.int()], -1).to(torch.uint16).view(clips, t, h // 2, w).pin_memory()]
+    out_i420 = [torch.empty((clips, t, 4 * h, 4 * w), dtype=torch.uint8).pin_memory()] + [
+        torch.empty((clips, t, 2 * h, 2 * w), dtype=torch.uint8).pin_memory() for _ in range(2)]
+    out_p010 = [torch.empty((clips, t, 4 * h, 4 * w), dtype=torch.uint16).pin_memory(),
+                torch.empty((clips, t, 2 * h, 4 * w), dtype=torch.uint16).pin_memory()]
+    static_i420 = [p.to(dev) for p in host_i420]
+    static_p010 = [p.to(dev) for p in host_p010]
+    dev_p010 = [torch.empty(p.shape, dtype=torch.uint16, device=dev) for p in out_p010]
+    out_views = (dev_p010[0], dev_p010[1][..., 0::2], dev_p010[1][..., 1::2])
+
+    with torch.no_grad():
+        ga, va = capture(lambda: net.forward_yuv420(*static_i420))
+        gb, _ = capture(lambda: net.forward_yuv420_u16(static_p010[0], static_p010[1][..., 0::2],
+                                                       static_p010[1][..., 1::2], bits=10, shift=6, out=out_views),
+                        pool=ga.pool())
+
+    def step_i420():
+        for d, hst in zip(static_i420, host_i420):
+            d.copy_(hst, non_blocking=True)
+        ga.replay()
+        for hst, d in zip(out_i420, va):
+            hst.copy_(d, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+
+    def step_p010():
+        for d, hst in zip(static_p010, host_p010):
+            d.copy_(hst, non_blocking=True)
+        gb.replay()
+        for hst, d in zip(out_p010, dev_p010):
+            hst.copy_(d, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+
+    res = {"forward_yuv420": [], "forward_yuv420_u16_p010": []}
+    step_i420()
+    step_p010()
+    for _ in range(rounds):
+        for name, fn in (("forward_yuv420", step_i420), ("forward_yuv420_u16_p010", step_p010)):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(steps):
+                fn()
+            res[name].append(clips * t * steps / (time.perf_counter() - t0))
+    # the P010 luma against the 8-bit luma of the same clips, rescaled (codes, in 8-bit levels), clip 0
+    d_y = ((out_p010[0][0].int() >> 6).double() / 4 - out_i420[0][0].int().double()).abs()
+    return {
+        "clips": clips, "frames_per_clip": t, "lr": [h, w], "out": [4 * h, 4 * w], "steps_per_round": steps,
+        "matrix": "bt709", "frames_per_s": {k: statistics.median(v) for k, v in res.items()},
+        "rounds_frames_per_s": res,
+        "h2d_bytes": {"forward_yuv420": sum(p.numel() for p in host_i420),
+                      "forward_yuv420_u16_p010": sum(p.numel() * 2 for p in host_p010)},
+        "d2h_bytes": {"forward_yuv420": sum(p.numel() for p in out_i420),
+                      "forward_yuv420_u16_p010": sum(p.numel() * 2 for p in out_p010)},
+        "luma_p010_vs_i420_clip0_8bit_levels": {"max": d_y.max().item(), "mean": d_y.mean().item()},
+    }
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
@@ -308,19 +425,21 @@ def main():
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--steps", type=int, default=2)
     ap.add_argument("--yuv", action="store_true", help="measure the Y'CbCr 4:2:0 tail instead (sr_tail_yuv.json)")
+    ap.add_argument("--hbd", action="store_true", help="measure the 16-bit RGB and P010 tails (sr_tail_hbd.json)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("prof_sr_tail.py needs a CUDA device")
     dev = torch.device("cuda:0")
     torch.backends.cudnn.benchmark = False
     result = {"gpu": gpu_info(), "torch": torch.__version__}
-    if args.yuv:
-        result["tail"] = tail_yuv(dev, args.rounds, args.reps)
+    if args.yuv or args.hbd:
+        name, tail_fn, e2e_fn = ("sr_tail_hbd", tail_hbd, e2e_hbd) if args.hbd else ("sr_tail_yuv", tail_yuv, e2e_yuv)
+        result["tail"] = tail_fn(dev, args.rounds, args.reps)
         print(json.dumps(result["tail"], indent=1), flush=True)
         torch.cuda.empty_cache()
-        result["e2e"] = e2e_yuv(dev, args.rounds, args.steps)
+        result["e2e"] = e2e_fn(dev, args.rounds, args.steps)
         os.makedirs(args.out, exist_ok=True)
-        with open(os.path.join(args.out, "sr_tail_yuv.json"), "w") as f:
+        with open(os.path.join(args.out, name + ".json"), "w") as f:
             json.dump(result, f, indent=1)
         print(json.dumps(result, indent=1))
         return
