@@ -1,6 +1,7 @@
 // Reconstruction tail of EAVSR+ as one tcgen05 kernel, writing 8-bit frames (models/eavsrp_model.py:350-364 followed
 // by the visuals of models/base_model.py:146-150), or 16-bit ones (M = 2^bits - 1 in place of 255), or Y'CbCr 4:2:0
-// planes of 8- or 16-bit samples (the store types below):
+// planes of 8- or 16-bit samples, or the 8-bit frame's squared error against a ground-truth frame (the store types
+// below):
 //
 //   out[n, y, x, c] = rint(clamp(255 * (b[c] + sum_{k,ci} W[c,ci,k] X[n,ci,y+ky-1,x+kx-1] + up_s(lr)[n,c,y,x]), 0, 255))
 //
@@ -22,7 +23,8 @@
 //   warp  1    TMEM owner; one lane loads the 18 KB of packed weights, issues 12 MMAs per tile, commits to mbarriers
 //   warps 2-9  two epilogue teams of four warps (one TMEM lane quadrant = one tile row each); team t drains accumulator
 //              buffer t: bilinear base from the LR frame (loads issued before the accumulator wait), tcgen05.ld,
-//              shifted sum, + bias, quantise, 3 byte stores per pixel
+//              shifted sum, + bias, quantise, 3 byte stores per pixel (RgbSse: and the squared error against a
+//              ground-truth frame, one 64-bit atomic per warp and image)
 #include <cuda.h>
 
 #include <type_traits>
@@ -87,6 +89,17 @@ struct Yuv420Out16 {
   float ys, yo, co;                // 219k, 16k, 128k
   int shift;                       // codes are stored times 2^shift
 };
+// The 8-bit RGB codes of RgbOut measured against a ground-truth frame: sse[n * sse_s] += sum over the valid pixels
+// of image n of (q - gt)^2, exact in integers.  The frame itself is stored only when p is set.
+struct RgbSse {
+  using T = uint8_t;
+  const uint8_t* gt;
+  long long g_n, g_y, g_x, g_c;
+  uint8_t* p;                      // null: no store
+  long long s_n, s_y, s_x, s_c;
+  unsigned long long* sse;         // added to, never overwritten
+  long long sse_s;
+};
 template <class Out>
 constexpr bool is_yuv420 = std::is_same<Out, Yuv420Out>::value || std::is_same<Out, Yuv420Out16>::value;
 
@@ -118,9 +131,17 @@ __global__ void sr_tail_pack_weight_kernel(const __nv_bfloat16* __restrict__ w, 
       o < 3 ? w[((size_t)o * ST_CH + ci) * 9 + t] : __float2bfloat16_rn(0.f);
 }
 
+// RgbSse: the warp's sum of its lanes' running sums, added to image n's total by one 64-bit atomic
+__device__ __forceinline__ void sse_flush(const RgbSse& o, int n, unsigned long long acc, int lane) {
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+  if (lane == 0 && acc != 0) atomicAdd(o.sse + n * o.sse_s, acc);
+}
+
 template <class Out>
 __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_constant__ TailParams<Out> P) {
   constexpr bool YUV = is_yuv420<Out>;
+  constexpr bool SSE = std::is_same<Out, RgbSse>::value;
   using T = typename Out::T;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -215,6 +236,10 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
     float bias[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c) bias[c] = P.bias ? __bfloat162float(P.bias[c]) : 0.f;
+    // RgbSse: this lane's running sum over the tiles of image sse_n.  The team's tiles come in increasing order, so n
+    // never decreases along them, and each image's sum leaves the warp once, when n changes and after the last tile
+    unsigned long long sse_acc = 0;
+    int sse_n = -1;
     for (int tl = team; tl < my_tiles; tl += 2) {
       int n, ty, tx;
       tile_at(tl, n, ty, tx);
@@ -222,7 +247,14 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
       const bool valid = lane < ST_TC && y < P.out_h && x < P.out_w;
       // bilinear base, ATen's upsample_bilinear2d (align_corners=False, scale_factor=s) in its order of operations
       float up[3] = {0.f, 0.f, 0.f};
+      uint32_t gt[3] = {0u, 0u, 0u};
       if (valid) {
+        if constexpr (SSE) {
+          // the ground truth, loaded with the LR samples: both arrive while the MMAs finish
+          const uint8_t* g = P.out.gt + n * P.out.g_n + (long long)y * P.out.g_y + (long long)x * P.out.g_x;
+#pragma unroll
+          for (int c = 0; c < 3; ++c) gt[c] = __ldg(g + c * P.out.g_c);
+        }
         const float sy = fmaxf(P.inv_scale * ((float)y + 0.5f) - 0.5f, 0.f);
         const float sx = fmaxf(P.inv_scale * ((float)x + 0.5f) - 0.5f, 0.f);
         const int h1 = (int)sy, w1 = (int)sx;
@@ -252,7 +284,28 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_acce + 8 * team);          // accumulator drained: tile tl + 2 may start
-      if constexpr (!YUV) {
+      if constexpr (SSE) {
+        if (n != sse_n) {                                       // n is the same for the whole warp
+          if (sse_n >= 0) sse_flush(P.out, sse_n, sse_acc, lane);
+          sse_n = n;
+          sse_acc = 0;
+        }
+        const long long off = n * P.out.s_n + (long long)y * P.out.s_y + (long long)x * P.out.s_x;
+        const bool store = valid && P.out.p != nullptr;
+        // at most 3 * 255^2 per lane and tile: 32 bits hold it, the running sum is 64-bit
+        uint32_t e = 0;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const float t = __uint_as_float(a0[c]) + __shfl_down_sync(0xffffffffu, __uint_as_float(a1[c]), 1) +
+                          __shfl_down_sync(0xffffffffu, __uint_as_float(a2[c]), 2);
+          // RgbOut's codes, expression for expression
+          const int code = __float2int_rn(fminf(fmaxf(255.f * ((t + bias[c]) + up[c]), 0.f), 255.f));
+          if (store) P.out.p[off + c * P.out.s_c] = (uint8_t)code;
+          const int d = code - (int)gt[c];
+          e += (uint32_t)(d * d);
+        }
+        if (valid) sse_acc += e;
+      } else if constexpr (!YUV) {
         T* op = P.out.p + n * P.out.s_n + (long long)y * P.out.s_y + (long long)x * P.out.s_x;
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
@@ -322,6 +375,9 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
         }
       }
     }
+    if constexpr (SSE) {
+      if (sse_n >= 0) sse_flush(P.out, sse_n, sse_acc, lane);
+    }
   }
 
   tc_fence_before();
@@ -329,7 +385,7 @@ __global__ void __launch_bounds__(ST_THREADS, 1) sr_tail_u8_kernel(const __grid_
   if (warp == 1) tmem_dealloc<ST_TMEM>(tmem_d);
 }
 
-// checks, tensor map and launch shared by the RGB and the 4:2:0 entry points of both sample sizes
+// checks, tensor map and launch shared by the RGB, the 4:2:0 and the squared-error entry points
 template <class Out>
 int sr_tail_launch(const char* who, const void* x, const int64_t x_strides[4], const void* packed_weight,
                    const void* bias, const float* lr, const int64_t lr_strides[4], const Out& out, int n, int c, int h,
@@ -478,4 +534,25 @@ extern "C" int eavsr_sr_tail_yuv420_u16_forward(const void* x, const int64_t x_s
   o.shift = shift;
   return sr_tail_launch("sr_tail_yuv420_u16_forward", x, x_strides, packed_weight, bias, lr, lr_strides, o, n, c, h,
                         w, scale, out_h, out_w, dtype, stream);
+}
+
+extern "C" int eavsr_sr_tail_u8_sse_forward(const void* x, const int64_t x_strides[4], const void* packed_weight,
+                                            const void* bias, const float* lr, const int64_t lr_strides[4],
+                                            const void* gt, const int64_t gt_strides[4], void* out,
+                                            const int64_t out_strides[4], unsigned long long* sse,
+                                            long long sse_stride, int n, int c, int h, int w, int scale, int out_h,
+                                            int out_w, int dtype, void* stream) {
+  EAVSR_REQUIRE(x && x_strides && packed_weight && lr && lr_strides && gt && gt_strides && sse && (!out || out_strides),
+                "sr_tail_u8_sse_forward: null pointer");
+  EAVSR_REQUIRE((reinterpret_cast<uintptr_t>(sse) & 7u) == 0, "sr_tail_u8_sse_forward: sse must be 8-byte aligned");
+  RgbSse o;
+  o.gt = (const uint8_t*)gt;
+  o.g_n = gt_strides[0]; o.g_y = gt_strides[1]; o.g_x = gt_strides[2]; o.g_c = gt_strides[3];
+  o.p = (uint8_t*)out;
+  o.s_n = out ? out_strides[0] : 0; o.s_y = out ? out_strides[1] : 0;
+  o.s_x = out ? out_strides[2] : 0; o.s_c = out ? out_strides[3] : 0;
+  o.sse = sse;
+  o.sse_s = sse_stride;
+  return sr_tail_launch("sr_tail_u8_sse_forward", x, x_strides, packed_weight, bias, lr, lr_strides, o, n, c, h, w,
+                        scale, out_h, out_w, dtype, stream);
 }

@@ -30,7 +30,7 @@ from .ops import (ModulatedDeformConv2d, adapt_mix, grouped_conv3x3, grouped_con
                   conv3x3_64, conv3x3_64_ca, conv3x3_64_eligible, conv3x3_chain_eligible, rca_group_chain,
                   flow_warp, flow_warp2, flow_warp_nhw2, flow_warp_pyramid, flow_warp_pyramid_eligible, fused_inference_ok,
                   spynet_level_input, sr_tail_u8, sr_tail_u8_eligible, sr_tail_yuv420,
-                  sr_tail_u16, sr_tail_yuv420_u16,
+                  sr_tail_u16, sr_tail_yuv420_u16, sr_tail_u8_sse,
                   modulated_deform_conv2d)
 from .yuv import HBD_MATRICES, MATRICES, check_bits, rgb_to_yuv420, yuv420_to_rgb
 
@@ -684,6 +684,55 @@ class EAVSRP(nn.Module):
             self._sr_frames(yuv420_to_rgb(y, u, v, kr, kb, bits, shift), fused, composed)
         return tuple(out)
 
+    def psnr_uint8(self, frames, hr, out=None):
+        """Per-frame PSNR of the 8-bit SR frames against ground-truth frames, the evaluation of the reference's
+        test_basic.py (``calc_psnr`` of util/util.py on the visuals), without materialising the SR clip.
+
+        ``frames`` (n, t, h, w, 3) and ``hr`` (n, t, s*h, s*w, 3) are uint8 RGB on the GPU, ``hr`` with any strides.
+        Returns ``(psnr, sse)``, both (n, t) on the device: ``sse`` (int64) is the sum over pixels and channels of
+        ``(q - hr)**2``, exact, where ``q`` is the frame `forward_uint8` returns, and ``psnr`` (float64) is
+        ``10 * log10(255**2 * 3 * s*h * s*w / sse)`` (`psnr_from_sse`), ``+inf`` where ``sse == 0``.  A per-clip PSNR
+        is then either the mean of ``psnr`` or `psnr_from_sse` of ``sse.sum(1)``, as the evaluation protocol asks.
+        With ``out``, a caller clip of `forward_uint8`'s shape with any strides, the frames are written there too.
+
+        With bf16 features, conv_last, the bilinear base, the quantisation and the squared-error sum run as one kernel
+        per frame (`ops.sr_tail_u8_sse`), which reads each ground-truth byte once and writes nothing else unless
+        ``out`` is given; otherwise the tail is composed in PyTorch as in `forward_uint8`, and ``sse`` equals the int64
+        error of the visuals of `forward` exactly.  Inference only (``no_grad``); no host synchronisation, so it can be
+        captured in a CUDA graph."""
+        named = (("frames", frames), ("hr", hr)) + ((("out", out),) if out is not None else ())
+        for name, p in named:
+            if not isinstance(p, torch.Tensor) or p.dtype != torch.uint8:
+                raise TypeError(f"EAVSRP.psnr_uint8: {name} must be a uint8 tensor, got "
+                                f"{getattr(p, 'dtype', type(p))}")
+        if frames.dim() != 5 or frames.shape[-1] != 3:
+            raise ValueError(f"EAVSRP.psnr_uint8 takes (n, t, h, w, 3) RGB frames, got {tuple(frames.shape)}")
+        n, t, h, w, _ = frames.shape
+        if h < 64 or w < 64:
+            raise ValueError(f"EAVSRP.psnr_uint8 needs a height and width of at least 64, got {h}x{w}")
+        s = self.scale
+        for name, p in named[1:]:
+            if tuple(p.shape) != (n, t, s * h, s * w, 3):
+                raise ValueError(f"EAVSRP.psnr_uint8: {name} must be {(n, t, s * h, s * w, 3)}, got {tuple(p.shape)}")
+        if not all(p.is_cuda for _, p in named):
+            raise NotImplementedError("EAVSRP.psnr_uint8: CUDA tensors only (the B200 library has no CPU fallback)")
+        with torch.no_grad():
+            lrs = frames.permute(0, 1, 4, 2, 3).float().div(255).contiguous()
+            sse = torch.zeros((n, t), dtype=torch.int64, device=frames.device)
+
+            def fused(i, x, lr):
+                sr_tail_u8_sse(self.conv_last, x, lr, s, hr[:, i], sse[:, i], s * h, s * w,
+                               None if out is None else out[:, i])
+
+            def composed(i, sr):
+                q = torch.clamp(sr * 255, 0, 255).round().permute(0, 2, 3, 1).to(torch.uint8)
+                if out is not None:
+                    out[:, i] = q
+                d = q.int() - hr[:, i].int()
+                sse[:, i] = (d * d).sum((1, 2, 3), dtype=torch.int64)
+            self._sr_frames(lrs, fused, composed)
+            return psnr_from_sse(sse, 3 * s * h * s * w), sse
+
     def _sr_frames(self, lrs, fused, composed):
         """The frame-in, frame-out forwards' common part, under ``no_grad``: pad the (n, t, 3, h, w) clip `lrs` (`pad_clip`), run
         `_trunk`, then per frame i `_hr_features` and the tail -- ``fused(i, x, lr_i)`` when the fused tail kernel can
@@ -733,3 +782,10 @@ def pad_clip(lrs, multiple=4):
     n, t, c = lrs.shape[:3]
     out = F.pad(lrs.reshape(n * t, c, h, w), (0, pw, 0, ph), mode="replicate")
     return out.view(n, t, c, h + ph, w + pw)
+
+
+def psnr_from_sse(sse, samples):
+    """PSNR of 8-bit frames from their integer squared-error sums over ``samples`` values each (pixels times
+    channels): ``10 * log10(255**2 * samples / sse)`` in float64, as ``calc_psnr`` of the reference's util/util.py on
+    the visuals; ``+inf`` where ``sse == 0``."""
+    return 10 * torch.log10((255.0 ** 2 * samples) / sse.double())

@@ -46,7 +46,7 @@ __all__ = [
     "adapt_mix", "affine_offsets_mask", "ca_residual", "fused_inference_ok", "bias_act_", "conv2d_bias_act",
     "conv3x3_64", "conv3x3_64_ca", "conv3x3_64_eligible", "ca_scale", "conv2d_bias_act_shuffle",
     "conv3x3_chain_eligible", "rca_group_chain", "sr_tail_u8", "sr_tail_u8_eligible", "sr_tail_yuv420",
-    "sr_tail_u16", "sr_tail_yuv420_u16",
+    "sr_tail_u16", "sr_tail_yuv420_u16", "sr_tail_u8_sse",
 ]
 
 _DTYPES = {torch.float32: L.F32, torch.bfloat16: L.BF16}
@@ -1151,3 +1151,28 @@ def sr_tail_yuv420_u16(conv_last: nn.Conv2d, x, lr, scale: int, y_out, u_out, v_
             n, x.shape[1], x.shape[2], x.shape[3], int(scale), int(out_h), int(out_w), float(kr), float(kb),
             int(bits), int(shift), L.BF16)
     return y_out, u_out, v_out
+
+
+def sr_tail_u8_sse(conv_last: nn.Conv2d, x, lr, scale: int, hr, sse, out_h: int, out_w: int, out=None):
+    """The squared error of `sr_tail_u8`'s frame against a ground-truth frame, in one kernel: ``sse[n] += sum over
+    y < out_h, x < out_w, c of (q[n, y, x, c] - hr[n, y, x, c])**2``, exact in int64, where ``q`` is the frame
+    `sr_tail_u8` writes; with ``out`` given, ``q`` is also written there, bit for bit as `sr_tail_u8` writes it.
+    ``hr``: (n, out_h, out_w, 3) uint8, any strides; ``sse``: (n,) int64, any stride (e.g. ``sums[:, i]`` of an
+    (n, t) tensor), added to and not overwritten; ``out``: as for `sr_tail_u8`, or None.  ``x`` and ``lr`` as for
+    `sr_tail_u8`, with the same eligibility (`sr_tail_u8_eligible`).  Returns ``sse``."""
+    n, c, h, w = x.shape
+    _check_tail_lr("sr_tail_u8_sse", x, lr, scale)
+    if hr.dtype != torch.uint8 or tuple(hr.shape) != (n, out_h, out_w, 3):
+        raise ValueError(f"eavsr_b200.sr_tail_u8_sse: hr must be uint8 (n, out_h, out_w, 3), got {hr.dtype} "
+                         f"{tuple(hr.shape)}")
+    if sse.dtype != torch.int64 or tuple(sse.shape) != (n,):
+        raise ValueError(f"eavsr_b200.sr_tail_u8_sse: sse must be int64 (n,), got {sse.dtype} {tuple(sse.shape)}")
+    if out is not None and (out.dtype != torch.uint8 or tuple(out.shape) != (n, out_h, out_w, 3)):
+        raise ValueError(f"eavsr_b200.sr_tail_u8_sse: out must be uint8 (n, out_h, out_w, 3), got {out.dtype} "
+                         f"{tuple(out.shape)}")
+    _require_cuda("sr_tail_u8_sse", x, lr, hr, sse, out)
+    _launch("sr_tail_u8_sse_forward", x, _strides(x), _packed_conv_weight(conv_last, x.device, "sr_tail"),
+            _param(conv_last.bias, torch.bfloat16), lr, L.Strides(*lr.stride()), hr, L.Strides(*hr.stride()),
+            out, None if out is None else L.Strides(*out.stride()), sse, sse.stride(0),
+            n, c, h, w, int(scale), int(out_h), int(out_w), L.BF16)
+    return sse

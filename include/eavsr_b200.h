@@ -416,6 +416,27 @@ int eavsr_sr_tail_yuv420_u16_forward(const void* x, const int64_t x_strides[4], 
                                      const int64_t v_strides[4], int n, int c, int h, int w, int scale, int out_h,
                                      int out_w, float kr, float kb, int bits, int shift, int dtype, void* stream);
 
+/* ---- the same tail's 8-bit frame measured against a ground-truth frame (the error sum of PSNR) --------------------
+ * With q[n, y, x, c] the code eavsr_sr_tail_u8_forward writes (the same expression, bit for bit), adds
+ *   sse[n * sse_stride] += sum_{y < out_h, x < out_w, c < 3} (q[n, y, x, c] - gt[n, y, x, c])^2
+ * exactly, in 64-bit integers, and, when out is not NULL, also stores q into out as eavsr_sr_tail_u8_forward does.
+ * sse is added to, not overwritten: the caller zeroes it (e.g. once per clip, then passes frame i's column of an
+ * (n, t) int64 tensor with sse_stride = t).  Each image's sum is exact and independent of the order of the additions,
+ * so two calls on the same operands give the same bits.
+ *   x, W, bias, lr: as eavsr_sr_tail_u8_forward, with the same packed weight.
+ *   gt:   uint8 by element strides gt_strides in (n, y, x, c) order, (n, out_h, out_w, 3).
+ *   out, out_strides: as eavsr_sr_tail_u8_forward, or both NULL for no store.
+ *   sse:  n unsigned 64-bit integers (an int64 tensor holds the same bits: a sum stays below 2^63 for any frame
+ *         under 4.7e13 pixels), 8-byte aligned, by element stride sse_stride.
+ * A null x, gt, sse or stride array (out_strides only when out is set), a misaligned sse and everything
+ * eavsr_sr_tail_u8_forward rejects return EAVSR_ERR_INVALID; dtype other than EAVSR_BF16 returns
+ * EAVSR_ERR_UNSUPPORTED. */
+int eavsr_sr_tail_u8_sse_forward(const void* x, const int64_t x_strides[4], const void* packed_weight, const void* bias,
+                                 const float* lr, const int64_t lr_strides[4], const void* gt,
+                                 const int64_t gt_strides[4], void* out, const int64_t out_strides[4],
+                                 unsigned long long* sse, long long sse_stride, int n, int c, int h, int w, int scale,
+                                 int out_h, int out_w, int dtype, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

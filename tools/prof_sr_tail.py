@@ -4,6 +4,7 @@
     python tools/prof_sr_tail.py --out DIR [--rounds 5]          -> DIR/sr_tail.json
     python tools/prof_sr_tail.py --out DIR --yuv [--rounds 5]    -> DIR/sr_tail_yuv.json
     python tools/prof_sr_tail.py --out DIR --hbd [--rounds 5]    -> DIR/sr_tail_hbd.json
+    python tools/prof_sr_tail.py --out DIR --psnr [--rounds 5]   -> DIR/sr_tail_psnr.json
 
 (a) The tail of one frame at the benchmark's operating point: 8 images of 64 x 1088 x 1920 bf16 features (2.1 GB,
     far more than L2) -> 8 frames of 1080 x 1920 x 3 uint8.  The fused kernel (`ops.sr_tail_u8`) against the
@@ -30,6 +31,15 @@ With --hbd, the high-bit-depth variants:
     HBM floors count 6 and 3 B/px written.
 (b) host to host, 8 clips of 30 x 270 x 480: `forward_yuv420_u16` on P010 (pinned Y and interleaved UV planes -> H2D
     -> graph -> D2H) against `forward_yuv420` on I420, both graph-captured and alternated.
+With --psnr, the squared error against ground-truth frames:
+(a) the tail at the same operating point with 8 ground-truth frames of 1080 x 1920 x 3 uint8: the RGB kernel
+    (`ops.sr_tail_u8`), the squared-error kernel without and with the store (`ops.sr_tail_u8_sse`), and the
+    composition it replaces (`ops.sr_tail_u8`, then the int64 SSE of that frame in PyTorch), alternated.  The HBM
+    floors count 3 B/px read for the ground truth, and 3 more written with the store.
+(b) host to host, 8 clips of 30 x 270 x 480 and their 8 x 30 ground-truth frames of 1080 x 1920 per step:
+    `psnr_uint8` (pinned LR and ground-truth frames -> H2D -> graph -> D2H of the (n, t) PSNR and SSE) against
+    `forward_uint8` + the int64 SSE in PyTorch on the device + D2H of the frames and the SSE, both graph-captured and
+    alternated.
 The GPU name, power limit and maximum SM clock are read with nvidia-smi in the same run.
 """
 import argparse
@@ -418,6 +428,123 @@ def e2e_hbd(dev, rounds, steps):
     }
 
 
+def tail_psnr(dev, rounds, reps):
+    conv, x, lr, (n, h, w, s, oh, ow) = _tail_operands(dev)
+    hr = torch.randint(0, 256, (n, oh, ow, 3), dtype=torch.uint8, device=dev)
+    rgb, rgb2 = (torch.empty((n, oh, ow, 3), dtype=torch.uint8, device=dev) for _ in range(2))
+    sums, sums2 = (torch.zeros(n, dtype=torch.int64, device=dev) for _ in range(2))
+
+    def composed():
+        ops.sr_tail_u8(conv, x, lr, s, rgb, oh, ow)
+        d = rgb.int() - hr.int()
+        return (d * d).sum((1, 2, 3), dtype=torch.int64)
+
+    arms = {
+        "rgb_kernel": lambda: ops.sr_tail_u8(conv, x, lr, s, rgb, oh, ow),
+        # the sums grow over the replays; the caller's zeroing (one memset per clip) is not part of the kernel
+        "sse_kernel": lambda: ops.sr_tail_u8_sse(conv, x, lr, s, hr, sums, oh, ow),
+        "sse_store_kernel": lambda: ops.sr_tail_u8_sse(conv, x, lr, s, hr, sums2, oh, ow, out=rgb2),
+        "composed_sse": composed,
+    }
+    with torch.no_grad():
+        assert ops.sr_tail_u8_eligible(conv, x)
+        graphs = {k: capture(fn) for k, fn in arms.items()}
+        t = {k: [] for k in arms}
+        for g, _ in graphs.values():
+            time_replays(g, 3)
+        for _ in range(rounds):
+            for k, (g, _) in graphs.items():
+                t[k].append(time_replays(g, reps))
+        # one more call of each on zeroed sums, against the composition's result
+        sums.zero_()
+        sums2.zero_()
+        ops.sr_tail_u8_sse(conv, x, lr, s, hr, sums, oh, ow)
+        ops.sr_tail_u8_sse(conv, x, lr, s, hr, sums2, oh, ow, out=rgb2)
+        want = composed()
+        exact = {"sse_kernel": torch.equal(sums, want), "sse_store_kernel": torch.equal(sums2, want),
+                 "stored_frames_equal_rgb_kernel": torch.equal(rgb2, rgb)}
+    lr_bytes = (h // s) * (w // s) * 12
+    # per output pixel: ground truth read + frame written (the composition adds its int64 reduction's traffic on top)
+    moved = {"rgb_kernel": 3, "sse_kernel": 3, "sse_store_kernel": 6, "composed_sse": 6}
+    nbytes = {k: n * (h * w * 128 + oh * ow * b + lr_bytes) for k, b in moved.items()}
+    med = {k: statistics.median(v) for k, v in t.items()}
+    floor = {k: v / HBM_BPS * 1e6 for k, v in nbytes.items()}
+    return {
+        "shape": {"images": n, "features": [64, h, w], "out": [oh, ow, 3], "scale": s},
+        "us_per_frame": med, "us_per_image": {k: v / n for k, v in med.items()},
+        "rounds_us_per_frame": t, "replays_per_round": reps, "frame_bytes_per_px": moved,
+        "hbm_bytes": nbytes, "hbm_floor_us_at_7.7TBps": floor,
+        "fraction_of_hbm_floor": {k: floor[k] / med[k] for k in med},
+        "over_rgb_kernel": {k: med[k] / med["rgb_kernel"] for k in med},
+        "sse_equal_to_composed": exact, "sse_per_image": want.tolist(),
+    }
+
+
+def e2e_psnr(dev, rounds, steps):
+    clips, t, h, w = 8, 30, 270, 480
+    net = EAVSRP(4).eval()
+    seeded_parameters(net)
+    net = net.to(dev).prepare(torch.bfloat16)
+    # the LR clips of the other arms; as ground truth, their bicubic x4 upsampling (the throughput does not depend on
+    # what the frames show)
+    f32 = torch.cat([clip_inputs(1, t, h, w, seed=1234 + i) for i in range(clips)])
+    host_u8 = (f32 * 255).round().to(torch.uint8).permute(0, 1, 3, 4, 2).contiguous().pin_memory()
+    host_hr = torch.empty((clips, t, 4 * h, 4 * w, 3), dtype=torch.uint8).pin_memory()
+    for i in range(clips):
+        up = F.interpolate(f32[i].to(dev), scale_factor=4, mode="bicubic", align_corners=False)
+        host_hr[i] = (up.clamp(0, 1) * 255).round().to(torch.uint8).permute(0, 2, 3, 1).cpu()
+    out_u8 = torch.empty((clips, t, 4 * h, 4 * w, 3), dtype=torch.uint8).pin_memory()
+    out_sse = [torch.empty((clips, t), dtype=torch.int64).pin_memory() for _ in range(2)]
+    out_psnr = torch.empty((clips, t), dtype=torch.float64).pin_memory()
+    static_u8, static_hr = host_u8.to(dev), host_hr.to(dev)
+
+    def forward_and_sse():
+        sr = net.forward_uint8(static_u8)
+        return sr, (sr.int() - static_hr.int()).pow(2).sum((2, 3, 4), dtype=torch.int64)
+
+    with torch.no_grad():
+        ga, (pa, sa) = capture(lambda: net.psnr_uint8(static_u8, static_hr))
+        gb, (vb, sb) = capture(forward_and_sse, pool=ga.pool())
+
+    def step_psnr():
+        static_u8.copy_(host_u8, non_blocking=True)
+        static_hr.copy_(host_hr, non_blocking=True)
+        ga.replay()
+        out_psnr.copy_(pa, non_blocking=True)
+        out_sse[0].copy_(sa, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+
+    def step_forward():
+        static_u8.copy_(host_u8, non_blocking=True)
+        static_hr.copy_(host_hr, non_blocking=True)
+        gb.replay()
+        out_u8.copy_(vb, non_blocking=True)
+        out_sse[1].copy_(sb, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+
+    res = {"psnr_uint8": [], "forward_uint8_torch_sse": []}
+    step_psnr()
+    step_forward()
+    for _ in range(rounds):
+        for name, fn in (("psnr_uint8", step_psnr), ("forward_uint8_torch_sse", step_forward)):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(steps):
+                fn()
+            res[name].append(clips * t * steps / (time.perf_counter() - t0))
+    # two runs of the trunk agree to rounding only (float atomics, DESIGN.md 4): the sums of the two arms differ by
+    # the few codes that moved by one level
+    rel = ((out_sse[0] - out_sse[1]).abs().double() / out_sse[1].double()).max().item()
+    return {
+        "clips": clips, "frames_per_clip": t, "lr": [h, w], "out": [4 * h, 4 * w, 3], "steps_per_round": steps,
+        "frames_per_s": {k: statistics.median(v) for k, v in res.items()}, "rounds_frames_per_s": res,
+        "h2d_bytes": {k: host_u8.numel() + host_hr.numel() for k in res},
+        "d2h_bytes": {"psnr_uint8": out_psnr.numel() * 8 + out_sse[0].numel() * 8,
+                      "forward_uint8_torch_sse": out_u8.numel() + out_sse[1].numel() * 8},
+        "mean_psnr_db": out_psnr.mean().item(), "max_relative_sse_difference_between_arms": rel,
+    }
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
@@ -426,14 +553,16 @@ def main():
     ap.add_argument("--steps", type=int, default=2)
     ap.add_argument("--yuv", action="store_true", help="measure the Y'CbCr 4:2:0 tail instead (sr_tail_yuv.json)")
     ap.add_argument("--hbd", action="store_true", help="measure the 16-bit RGB and P010 tails (sr_tail_hbd.json)")
+    ap.add_argument("--psnr", action="store_true", help="measure the squared-error tail and psnr_uint8 (sr_tail_psnr.json)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("prof_sr_tail.py needs a CUDA device")
     dev = torch.device("cuda:0")
     torch.backends.cudnn.benchmark = False
     result = {"gpu": gpu_info(), "torch": torch.__version__}
-    if args.yuv or args.hbd:
-        name, tail_fn, e2e_fn = ("sr_tail_hbd", tail_hbd, e2e_hbd) if args.hbd else ("sr_tail_yuv", tail_yuv, e2e_yuv)
+    if args.yuv or args.hbd or args.psnr:
+        name, tail_fn, e2e_fn = (("sr_tail_psnr", tail_psnr, e2e_psnr) if args.psnr else
+                                 ("sr_tail_hbd", tail_hbd, e2e_hbd) if args.hbd else ("sr_tail_yuv", tail_yuv, e2e_yuv))
         result["tail"] = tail_fn(dev, args.rounds, args.reps)
         print(json.dumps(result["tail"], indent=1), flush=True)
         torch.cuda.empty_cache()
